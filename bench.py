@@ -1,13 +1,20 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric on synthetic clouds of BASELINE.json's configurations.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on rank 0.  metric = ICP hypotheses/s (whole job) on configs[3] — 1024 initial
 poses x 50k-pt model vs ~500k-pt scene, 30 point-to-point iterations, hypotheses sharded over
 the ranks — and, at N = 1, the single-align latency of configs[1] (200k scene / 50k model,
 30 iterations) beside it as `align_ms`.  A "step" is one pass of the hot path over the whole
 batch of hypotheses.  See DESIGN.md ("Measurement") for every key.
+
+--dump-outputs DIR writes the result records of the last timed step, one DIR/<field>.npy per field of
+peb_icp_result in hypothesis order (float32 / float64), so that two builds can be compared output for
+output: the inputs are seeded and identical from run to run.
+
+The benchmark writes nothing into the repository tree (which may be read-only): it expects the
+native libraries that build() compiled and writes no bytecode cache.
 """
 from __future__ import annotations
 
@@ -26,11 +33,14 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # no __pycache__ of the project's modules in the tree
 
 ITERATIONS = 30
 MAX_CORR_DIST = 0.02
 N_HYP = 1024
 ALG_BYTES_PER_QUERY = 40  # SURVEY.md 8d: 16 read source + 16 gather matched target + 8 write correspondence
+DUMP_BYTES_MAX = 64 << 20
+HBM_PEAK_GBS = 6544.7  # measured HBM bandwidth of one B200 (power limit not recorded): the roofline denominator of BASELINE.md
 
 
 def log(*a):
@@ -191,9 +201,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    from oracle import Oracle, build
+    from oracle import Oracle
 
-    build()
     orc = Oracle(fast=True)
     slow = Oracle()
     cores = host_threads()
@@ -370,6 +379,7 @@ def run_ours(args):
         barrier()
         clocks = sampler.stop() if rank == 0 else None
         launches = ctx.launch_count - launches0
+        last_step_records = (d_all if world > 1 else d_res).cpu().numpy().tobytes() if args.dump_outputs else None
         # per-iteration detail from one extra, untimed step (events between the launches serialise them)
         ctx.set_int("profile", 2)
         _, kernel_ms = timed(step_device, 1, profile=2)
@@ -408,11 +418,7 @@ def run_ours(args):
     results_bytes = (d_all if world > 1 else d_res).cpu().numpy().tobytes()
 
     # ---- roofline of the dominant kernel (icp_iteration_kernel) -------------------------------
-    peaks_file = ROOT / "MEASURED_PEAKS.json"
-    if peaks_file.exists():
-        peak, peak_src = float(json.loads(peaks_file.read_text())["hbm_gbs"]), "MEASURED_PEAKS.json hbm_gbs (of measured)"
-    else:
-        peak, peak_src = 6650.0, "B200_PROFILING.md fallback (of fallback)"
+    peak, peak_src = HBM_PEAK_GBS, "measured HBM bandwidth of one B200, BASELINE.md (of measured)"
     kernel_name = "icp_iteration_kernel (batched, one launch = one ICP iteration of this rank's hypotheses)"
     alg_bytes = h_local * len(c4.source) * ALG_BYTES_PER_QUERY
     avg_kernel_ms = sum(span_ms) / max(len(span_ms) * ITERATIONS, 1)
@@ -471,9 +477,28 @@ def run_ours(args):
         line["check"] = {"iterations_all": bool((recs["iterations"] == ITERATIONS).all()),
                          "fitness_median": float(np.median(recs["fitness"])),
                          "best_hypothesis": multi.best_hypothesis(recs)}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, multi.unpack_results(last_step_records, H, world))
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, records: np.ndarray) -> None:
+    """One <out_dir>/<field>.npy per field of the peb_icp_result records: T as (H, 16) float32, column-major as in the
+    struct, fitness and last_mse float64, the integer fields widened to float64 (exact), and hypothesis.npy, the index of
+    every row.  Above DUMP_BYTES_MAX in all, the rows are a fixed, seeded sample of the hypotheses, in hypothesis order."""
+    cols = {f: records[f] if records[f].dtype.kind == "f" else records[f].astype(np.float64) for f in records.dtype.names}
+    cols["hypothesis"] = np.arange(len(records), dtype=np.float64)
+    total = sum(a.nbytes for a in cols.values())
+    budget = DUMP_BYTES_MAX - 4096 * len(cols)  # room for the .npy headers
+    if total > budget:
+        keep = np.sort(np.random.default_rng(0).choice(len(records), len(records) * budget // total, replace=False))
+        cols = {f: a[keep] for f, a in cols.items()}
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for f, a in cols.items():
+        np.save(out / f"{f}.npy", a)
 
 
 def inproc_leg(args, torch, pcl, lib, c4, guesses_cm, params, n_dev, H, rec, ranks_records):
@@ -667,10 +692,9 @@ def cpu_stage_baselines(c2):
     """The CPU port (oracle timing build, the PCL 1.10 restatement: single kd-tree, leaf 15, exact search) on this box's
     host cores for every stage bench.py times on the GPU.  PCL 1.10's ICP loop, VoxelGrid and NormalEstimation are serial
     (1 thread); NormalEstimationOMP is the all-cores figure."""
-    from oracle import Oracle, build, default_params
+    from oracle import Oracle, default_params
     from pose_estimation_b200.testing import synth
 
-    build()
     orc = Oracle(fast=True)
     cores = host_threads()
 
@@ -984,9 +1008,8 @@ def preprocessing_stages(ctx, c2, torch, stream, flush, pcl, lib):
 
 def cpu_baseline(c4):
     """The oracle's timing build on this box's host cores, bounded sample of the same workload."""
-    from oracle import Oracle, build
+    from oracle import Oracle
 
-    build()
     orc = Oracle(fast=True)
     cores = host_threads()
     icp = orc.icp(c4.target)
@@ -1013,7 +1036,12 @@ def main():
     ap.add_argument("--no-single", action="store_true", help="skip the configs[1] single-align leg")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-inproc", action="store_true", help="skip the single-process peb_multi_* leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA arm (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         log("[bench] note: the timing rules ask for >= 3 warm-up steps")
     if args.impl == "reference":
