@@ -124,6 +124,12 @@ PEB_API uint64_t peb_ctx_launch_count(const peb_ctx* ctx);
  * 32-point patch, how far a point may be from its anchor in cells x 10, and up to how many grid rows a patch
  * verifies its candidates warp-cooperatively; 0 = per lane), "batch_streams" (independent chains of launches
  * of a batched align, 0 = auto), "blocks_factor" / "blocks_factor_cold" (blocks per SM and launch, 0 = auto),
+ * "split_moments" (default 1: every iteration of a batch runs as a search launch — nearest neighbours only, more
+ * resident warps — and a moment launch that recomputes the correspondences' distances, sums the moments in the order of
+ * the fused kernel and solves — icp.cu : icp_search_kernel; byte-identical records; 0 = one fused launch per
+ * iteration) in batches of at least "split_min_hyp" (default 256; smaller batches measured no faster split) hypotheses,
+ * "blocks_factor_search" (blocks per SM of those search launches, 0 = like the iteration's moment launch; results do
+ * not depend on it),
  * "flag_deps" (warm launches of a batch wait per hypothesis instead of for the whole previous grid),
  * "pdl" (programmatic dependent launch), "cert_margin_x1000" (search-skipping certificates, off),
  * "profile" (0 / 1 / 2, see peb_profile_read), "debug_timers" (development),

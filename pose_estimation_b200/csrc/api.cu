@@ -269,6 +269,21 @@ PEB_API int peb_ctx_set_int(peb_ctx* ctx, const char* key, int value) {
     ctx->blocks_factor_cold = value;
     return PEB_OK;
   }
+  if (!strcmp(key, "blocks_factor_search")) {
+    if (value < 0 || value > 4096) return fail(ctx, PEB_E_INVALID_ARG, "blocks_factor_search out of [0, 4096]");
+    ctx->blocks_factor_search = value;
+    return PEB_OK;
+  }
+  if (!strcmp(key, "split_moments")) {
+    if (value < 0 || value > 1) return fail(ctx, PEB_E_INVALID_ARG, "split_moments must be 0 or 1");
+    ctx->split_moments = value;
+    return PEB_OK;
+  }
+  if (!strcmp(key, "split_min_hyp")) {
+    if (value < 2) return fail(ctx, PEB_E_INVALID_ARG, "split_min_hyp must be >= 2 (batches only)");
+    ctx->split_min_hyp = value;
+    return PEB_OK;
+  }
   if (!strcmp(key, "flag_deps")) {
     ctx->flag_deps = value != 0;
     return PEB_OK;

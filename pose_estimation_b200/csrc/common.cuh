@@ -127,6 +127,10 @@ struct peb_ctx {
   cudaEvent_t fork_event = nullptr;
   int blocks_factor = 0;        // batched aligns: ~this many blocks per SM and launch in total; 0 = auto
   int blocks_factor_cold = 0;   // the same for launch 0 of a batched align; 0 = like blocks_factor
+  int blocks_factor_search = 0; // the same for the search launches of split iterations; 0 = like the launch's moment launch
+  int split_moments = 1;        // batched iterations run as a search launch and a moment launch (icp.cu : icp_search_kernel)
+  int split_min_hyp = 256;      // ... in batches of at least this many hypotheses (a 128-hypothesis shard: 8.27 / 8.58 ms fused,
+                                // 8.27 / 8.66 split at PEB_HYP_OFFSET 0 / 512, B200)
   bool flag_deps = true;        // warm launches wait per hypothesis (epoch flags) instead of for the whole previous grid
   peb::DevBuf epochs;           // H solved-iteration counters + 1 error flag
   int* last_err_flag = nullptr; // device address of that flag for the last batched align (nullptr: whole-grid dependencies)

@@ -736,7 +736,8 @@ struct IcpState {
   int iterations, state, converged, similar;
   int ncorr, active, fit_n, pad0;
   unsigned ticket, ticket_fit;
-  int pad1[2];
+  unsigned ticket_search;  // split iterations of a batch (icp.cu : icp_search_kernel): search blocks of the launch done
+  int searched;            // ... and search launches of this hypothesis completed
 };
 
 struct IcpCriteria {

@@ -43,6 +43,12 @@ constexpr int kMinBlocksSingle = 5;
 #define PEB_MIN_BLOCKS_BATCH 8
 #endif
 constexpr int kMinBlocksBatch = PEB_MIN_BLOCKS_BATCH;  // (development: -DPEB_MIN_BLOCKS_BATCH=n builds a variant library, PEB_LIB_VARIANT)
+// The search launch of a split iteration (icp_search_kernel) holds no moments and no solve: without a cap it needs 82
+// registers, so its cap is chosen on its own (measured, profiles/README.md).
+#ifndef PEB_MIN_BLOCKS_SEARCH
+#define PEB_MIN_BLOCKS_SEARCH 10
+#endif
+constexpr int kMinBlocksSearch = PEB_MIN_BLOCKS_SEARCH;
 
 struct IcpLaunch {
   GridView grid;
@@ -115,7 +121,8 @@ __global__ void icp_init_kernel(IcpState* __restrict__ states, const float* __re
   st.pad0 = 0;
   st.ticket = 0;
   st.ticket_fit = 0;
-  st.pad1[0] = st.pad1[1] = 0;
+  st.ticket_search = 0;
+  st.searched = 0;
   states[h] = st;
 }
 
@@ -253,6 +260,25 @@ __device__ __forceinline__ void wait_for_hypothesis(const int* __restrict__ solv
     const unsigned long long t0 = global_ns();
     unsigned spins = 0;
     while (ld_acquire_gpu(solved) < need) {
+      __nanosleep(40);
+      if ((++spins & 0xFFFu) == 0u && global_ns() - t0 > kFlagWaitLimitNs) {
+        atomicExch(err_flag, 1);
+        break;
+      }
+    }
+  }
+  __syncthreads();
+}
+
+// Waits (thread 0, then the block) until `need` search launches of the hypothesis have completed (a split iteration's
+// moment launch, icp_moment_kernel) or the hypothesis has stopped (its epoch carries kEpochStopped; its later search launches
+// count nothing).  Bounded like wait_for_hypothesis.
+__device__ __forceinline__ void wait_for_search(const int* __restrict__ searched, int need, const int* __restrict__ solved,
+                                                int* err_flag) {
+  if (threadIdx.x == 0 && ld_acquire_gpu(searched) < need && ld_acquire_gpu(solved) < kEpochStopped) {
+    const unsigned long long t0 = global_ns();
+    unsigned spins = 0;
+    while (ld_acquire_gpu(searched) < need && ld_acquire_gpu(solved) < kEpochStopped) {
       __nanosleep(40);
       if ((++spins & 0xFFFu) == 0u && global_ns() - t0 > kFlagWaitLimitNs) {
         atomicExch(err_flag, 1);
@@ -499,6 +525,82 @@ __device__ __forceinline__ void icp_query(const IcpLaunch& L, const int h, float
   if (keep && lane_in_group == 0) accumulate_pair<EST>(L.grid, p, best, acc);
 }
 
+// The search half of icp_query (move, search, store the working point) for one lane per query and no certificate: the
+// whole of a split iteration's search launch (icp_search_kernel).  A copy rather than a helper shared with icp_query, so
+// that the fused kernels keep their code generation.  p: the moved point; valid: the query's point was finite before.
+template <int UPF>
+__device__ __forceinline__ NnBest icp_search_query(const IcpLaunch& L, const int h, float4* __restrict__ work, const int i,
+                                                   const bool first, const bool apply, const bool graph, const float* T,
+                                                   CoopTile* tile, float4& p, bool& valid) {
+  const bool in = i < L.n_src;
+  p = make_float4(0.f, 0.f, 0.f, 1.f);
+  if (in) p = first ? L.src[i] : work[i];
+  const int j_prev = first ? -1 : __float_as_int(p.w);  // last iteration's match (sorted position)
+  valid = in && finite3(p.x, p.y, p.z);
+  if (valid && apply) {
+    float ox, oy, oz;
+    transform_icp(T, p.x, p.y, p.z, ox, oy, oz);
+    p.x = ox;
+    p.y = oy;
+    p.z = oz;
+  }
+  NnBest best;
+  best.d2 = pos_inf();
+  best.idx = -1;
+  best.j = -1;
+  if (first && L.anchors) {
+    // (uniform branch: every lane of the warp takes part, valid or not)
+    best = first_iteration_search(L, h, i, valid, p, T, apply, tile);
+  } else if (valid) {
+    if (L.warm && j_prev >= 0 && j_prev < L.grid.n) {
+      if (UPF == 4 || UPF == 6) best = graph ? grid_nn_warm_graph(L.grid, L.knn, p.x, p.y, p.z, j_prev, L.stop_d2, kGraphSkipHopeless, L.launch_idx <= L.knn_peek_until, UPF == 6 ? L.knn_aux : nullptr)
+                                 : grid_nn_warm(L.grid, p.x, p.y, p.z, j_prev, L.stop_d2);
+      else best = grid_nn_warm(L.grid, p.x, p.y, p.z, j_prev, L.stop_d2);
+    } else {
+      best = grid_nn<1>(L.grid, p.x, p.y, p.z, L.stop_d2);
+    }
+  }
+  if (in && (first || valid)) {
+    p.w = __int_as_float(best.j);
+    work[i] = p;
+  }
+  return best;
+}
+
+// [PCL] determineCorrespondences (d2 > max_dist^2 rejected) and the distance rejector (kept iff d2 < max)
+__device__ __forceinline__ bool keep_pair(const IcpLaunch& L, const bool valid, const NnBest& best) {
+  bool keep = valid && best.idx >= 0;
+  if (keep && static_cast<double>(best.d2) > L.max_dist_sqr) keep = false;
+  if (keep && L.use_rejector && !(best.d2 < L.rej_max2)) keep = false;
+  return keep;
+}
+
+// s_inc <- the transform every query of this launch is moved by; s_flags <- active, first iteration, apply transform,
+// warm searches over the k-NN graph.  (Followed by a barrier in the caller.)
+template <bool FIRST, int UPF>
+__device__ __forceinline__ void load_launch_flags(const IcpLaunch& L, const IcpState* st, float* s_inc, int* s_flags) {
+  // the guess in launch 0, else the last increment
+  if (threadIdx.x < 16) s_inc[threadIdx.x] = FIRST ? __ldcg(&st->final_t.m[threadIdx.x]) : __ldcg(&st->inc.m[threadIdx.x]);
+  if (threadIdx.x == 32) {
+    const int active = __ldcg(&st->active);
+    const int first = FIRST ? 1 : 0;
+    int apply = 1;
+    if (first) {
+      // [PCL] icp.hpp: the guess is applied only if it differs from the identity
+      apply = 0;
+      for (int i = 0; i < 16; ++i) {
+        const float g = __ldcg(&st->final_t.m[i]);
+        if (g != ((i % 5 == 0) ? 1.0f : 0.0f)) apply = 1;
+      }
+    }
+    s_flags[0] = active;
+    s_flags[1] = first;
+    s_flags[2] = apply;
+    const int graph = ((UPF == 4 || UPF == 6) && graph_pays(L, st)) ? 1 : 0;
+    s_flags[3] = graph;
+  }
+}
+
 // One block's share of one ICP iteration of hypothesis h: chunk `blk` of L.blocks_per_hyp.  Shared by
 // the per-iteration kernel (blk = blockIdx.x, h = blockIdx.y) and the work-queue kernel below.
 template <int G, int EST, int MB, bool CERT, bool FIRST, int UPF>
@@ -605,6 +707,136 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_iteration_kernel(const Ic
     wait_for_hypothesis(L.epochs + blockIdx.y, L.launch_idx, L.err_flag);
   }
   icp_iteration_body<G, EST, MB, CERT, FIRST, UPF>(L, blockIdx.y, blockIdx.x);
+}
+
+// ---- one iteration of a batch as two launches: the searches, then the moments and the solve ----------------------
+// In icp_iteration_kernel the double moment sums (17 for SVD, 28 for LLS), the block reduction and the out-of-line
+// solve share the allocation of the search loop: the batched kernels spill at their 64-register cap, and their late
+// launches, bound by the L2 latency of the searches, run with about 25 resident warps per SM.  Split:
+//   icp_search_kernel  grid = (search blocks per hypothesis, H): the fused kernel's search half (icp_search_query)
+//                      and nothing else — no double state, no reduction, no solve — under its own register cap (kMinBlocksSearch): more
+//                      resident warps to hide the search's latency.  Its block count is free: it writes no records.
+//   icp_moment_kernel  grid = (blocks_per_hyp, H): per query the working point and its match are read back and d2 is
+//                      recomputed as every search path computes it (l2_simple of the query and the match); threshold,
+//                      moments, block record, ticket, reduction and solve follow as in icp_iteration_body.  Its blocks
+//                      and its query-to-thread mapping (G = 1) are the fused kernel's, so every double is added in the
+//                      same order: byte-identical records.  It reads the working clouds once more.
+// A point that this launch's transform makes non-finite (a non-finite guess or increment) is still a valid query of the
+// fused kernel, which searches it; its match is stored as -2 - j in .w so that the moment launch can tell, and the next
+// search launch, for which the point is invalid, resets it to -1 (the fitness search is exact whether it starts warm or
+// cold, so nothing else reads the difference).
+// Dependencies with flags: a search block of (h, k) waits for epochs[h] >= k as a fused block does; if h is active, every
+// search block then takes a ticket of the state (ticket_search), and the last one resets it and publishes searched = k + 1
+// (fence + atomic); a moment block of (h, k) waits for searched >= k + 1 or for h to have stopped (wait_for_search).  The
+// split launches of an align are a prefix of its launches (the host keeps it so), hence the count.  The launches of an
+// active hypothesis never overlap (search k + 1 waits for the solve of k), so the ticket's reset races with nothing; those
+// of a stopped one do (its epoch releases them all), and they take no ticket.  Every block still waits only for blocks of
+// earlier launches (see icp_iteration_kernel).  Without flags both launches wait for the whole previous grid.
+// The search stride is gridDim.x: its blocks per hypothesis are free (it writes no records).
+template <int MB, bool FIRST, int UPF>
+__global__ void __launch_bounds__(kIcpThreads, MB) icp_search_kernel(const IcpLaunch L) {
+  if (FIRST || L.epochs == nullptr) {
+    pdl_trigger_and_wait();
+  } else {
+    asm volatile("griddepcontrol.launch_dependents;");
+    wait_for_hypothesis(L.epochs + blockIdx.y, L.launch_idx, L.err_flag);
+  }
+  const int h = blockIdx.y, blk = blockIdx.x;
+  __shared__ float s_inc[16];
+  __shared__ int s_flags[4];
+  __shared__ CoopTile s_tile[kIcpThreads / 32];
+  IcpState* st = L.states + h;
+  load_launch_flags<FIRST, UPF>(L, st, s_inc, s_flags);
+  __syncthreads();
+  if (s_flags[0]) {
+    const bool apply = s_flags[2] != 0;
+    const bool graph = (UPF == 4 || UPF == 6) && s_flags[3] != 0;
+    float4* work = L.work + static_cast<size_t>(h) * L.n_src;
+    for (int base = blk * kIcpThreads; base < L.n_src; base += gridDim.x * kIcpThreads) {
+      const int i = base + threadIdx.x;
+      float4 p;
+      bool valid;
+      const NnBest best = icp_search_query<UPF>(L, h, work, i, FIRST, apply, graph, s_inc, &s_tile[threadIdx.x >> 5], p, valid);
+      int* w = reinterpret_cast<int*>(work + i) + 3;
+      if (valid && best.j >= 0 && !finite3(p.x, p.y, p.z)) *w = -2 - best.j;
+      else if (!FIRST && !valid && i < L.n_src && __float_as_int(p.w) <= -2) *w = -1;
+    }
+  }
+  if (L.epochs && s_flags[0]) {
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      __threadfence();
+      if (atomicAdd(&st->ticket_search, 1u) == gridDim.x - 1u) {
+        st->ticket_search = 0u;
+        __threadfence();
+        atomicAdd(&st->searched, 1);
+      }
+    }
+  }
+}
+
+template <int EST, int MB>
+__global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLaunch L) {
+  if (L.epochs == nullptr) {
+    pdl_trigger_and_wait();
+  } else {
+    asm volatile("griddepcontrol.launch_dependents;");
+    wait_for_search(&L.states[blockIdx.y].searched, L.launch_idx + 1, L.epochs + blockIdx.y, L.err_flag);
+  }
+  const int h = blockIdx.y, blk = blockIdx.x;
+  constexpr int NACC = (EST == PEB_ESTIMATOR_SVD) ? kAccSvd : kAccLls;
+  __shared__ double sm[kIcpThreads / 32][kAccMax];
+  __shared__ double sm_tot[kAccMax];
+  __shared__ int s_active;
+  IcpState* st = L.states + h;
+  if (threadIdx.x == 0) s_active = __ldcg(&st->active);
+  __syncthreads();
+  if (!s_active) return;
+
+  double acc[NACC];
+#pragma unroll
+  for (int i = 0; i < NACC; ++i) acc[i] = 0.0;
+  const float4* work = L.work + static_cast<size_t>(h) * L.n_src;
+  for (int i = blk * kIcpThreads + threadIdx.x; i < L.n_src; i += L.blocks_per_hyp * kIcpThreads) {
+    const float4 p = __ldcg(work + i);
+    bool valid = finite3(p.x, p.y, p.z);
+    int j = __float_as_int(p.w);
+    if (j <= -2) {  // made non-finite by this launch's transform: searched all the same (see above)
+      valid = true;
+      j = -2 - j;
+    }
+    if (!valid || j < 0) continue;
+    const float4 t = L.grid.pts[j];
+    NnBest best;
+    best.d2 = l2_simple(p.x, p.y, p.z, t.x, t.y, t.z);
+    best.idx = point_index(t);
+    best.j = j;
+    if (keep_pair(L, valid, best)) accumulate_pair<EST>(L.grid, p, best, acc);
+  }
+
+  // ---- the block's record, the last block's solve: as in icp_iteration_body ----
+  const double r = block_reduce_acc<NACC>(acc, sm);
+  double* part = L.partials + (static_cast<size_t>(h) * L.part_stride) * kAccMax;
+  if (threadIdx.x < NACC) __stcg(part + static_cast<size_t>(blk) * kAccMax + threadIdx.x, r);
+  __threadfence();
+  __syncthreads();
+  __shared__ int s_last;
+  if (threadIdx.x == 0) {
+    const unsigned t = atomicAdd(&st->ticket, 1u);
+    s_last = (t == static_cast<unsigned>(L.blocks_per_hyp) - 1u);
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  reduce_partials<NACC>(part, L.blocks_per_hyp, sm, sm_tot);
+  if (threadIdx.x == 0) {
+    finish_iteration<MB>(st, &L.crit, sm_tot, L.trace, L.trace_cap, nullptr);
+    if (L.epochs) {
+      const int still_active = st->active;
+      __threadfence();
+      atomicAdd(L.epochs + h, still_active ? 1 : kEpochStopped);
+    }
+  }
 }
 
 // ---- warm iterations with the queries of a block binned by the size of their search ------------------------------
@@ -1299,8 +1531,43 @@ int prof_mark(peb_ctx* ctx, int slot) {
   return PEB_OK;
 }
 
+// Does this iteration launch run as a search launch and a moment launch?  Batched aligns with one lane per query on
+// their default paths: launch 0, the warm launches over the k-NN graph (with or without the flatness certificate) and
+// the plain warm launches.  The single align (latency-bound per launch: one more launch per iteration would cost it),
+// the certificates, the debug timers and the experimental variants keep the fused kernel.
+bool split_iteration(const peb_ctx* ctx, const IcpLaunch& L, size_t H, int G, bool first) {
+  if (!ctx->split_moments || H < static_cast<size_t>(ctx->split_min_hyp) || H <= 1 || G != 1 || L.margin > 0.0f || L.dbg ||
+      L.corr_idx)
+    return false;
+  if (first) return true;
+  if (L.cache || (ctx->warm_upfront && L.warm && L.launch_idx >= ctx->warm_upfront_from)) return false;
+  if (L.warm && L.knn) return ctx->warm_graph_queue == 0;
+  return !(L.warm && ctx->warm_bin);
+}
+
+template <bool FIRST>
+int launch_split_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
+  const dim3 sgrid(search_bph, static_cast<unsigned>(H)), mgrid(L.blocks_per_hyp, static_cast<unsigned>(H));
+  // (launch 0 keeps the batched cap: its cooperative verification holds more state than a warm search)
+  if (FIRST)
+    PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksBatch, true, 0>), sgrid, dim3(kIcpThreads), L);
+  else if (L.warm && L.knn && L.knn_aux && L.launch_idx >= ctx->warm_graph_flat_from && L.launch_idx <= ctx->warm_graph_flat_until)
+    PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksSearch, false, 6>), sgrid, dim3(kIcpThreads), L);
+  else if (L.warm && L.knn)
+    PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksSearch, false, 4>), sgrid, dim3(kIcpThreads), L);
+  else
+    PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksSearch, false, 0>), sgrid, dim3(kIcpThreads), L);
+  if (estimator == PEB_ESTIMATOR_SVD)
+    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_SVD, kMinBlocksBatch>), mgrid, dim3(kIcpThreads), L);
+  else
+    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_POINT_TO_PLANE_LLS, kMinBlocksBatch>), mgrid, dim3(kIcpThreads), L);
+  return PEB_OK;
+}
+
+// search_bph > 0: the iteration runs split, with this many search blocks per hypothesis
 template <int G, bool FIRST>
-int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator) {
+int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
+  if (G == 1 && search_bph > 0) return launch_split_iteration<FIRST>(ctx, L, H, estimator, search_bph);
   dim3 grid(L.blocks_per_hyp, static_cast<unsigned>(H));
   constexpr int S = PEB_ESTIMATOR_SVD, P = PEB_ESTIMATOR_POINT_TO_PLANE_LLS;
   const bool cert = G == 1 && L.margin > 0.0f;
@@ -1371,8 +1638,8 @@ int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimat
 }
 
 // first: launch 0 of the align
-int launch_one_iteration_g(peb_ctx* ctx, int G, bool first, const IcpLaunch& L, size_t H, int estimator) {
-#define PEB_ICP_G(GG) return first ? launch_one_iteration<GG, true>(ctx, L, H, estimator) : launch_one_iteration<GG, false>(ctx, L, H, estimator)
+int launch_one_iteration_g(peb_ctx* ctx, int G, bool first, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
+#define PEB_ICP_G(GG) return first ? launch_one_iteration<GG, true>(ctx, L, H, estimator, search_bph) : launch_one_iteration<GG, false>(ctx, L, H, estimator, search_bph)
   switch (G) {
     case 1: PEB_ICP_G(1);
     case 2: PEB_ICP_G(2);
@@ -1545,6 +1812,10 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   }
   Lw.blocks_per_hyp = blocks_for(n, H, g_warm, ctx->blocks_factor);
   Lw.warm = ctx->warm_start ? 1 : 0;
+  // the search launches of split iterations (icp_search_kernel; one lane per query)
+  const int fs = ctx->blocks_factor_search;
+  const int search_bph_cold = blocks_for(n, H, 1, fs > 0 ? fs : cold_blocks_factor(ctx));
+  const int search_bph_warm = blocks_for(n, H, 1, fs > 0 ? fs : ctx->blocks_factor);
   // the warm searches of a large enough batch run over the target's k-NN graph (built once per target)
   if (ctx->warm_graph && ctx->warm_start && g_warm == 1 && !single_mode && !(L.margin > 0.0f) && !ctx->warm_upfront &&
       !ctx->warm_bin && ctx->nn_cache_from == 0 && H >= static_cast<size_t>(ctx->warm_graph_min_hyp) && launches > 1) {
@@ -1571,6 +1842,13 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   auto set_cache = [&](int it) {
     Lw.cache = (cache_buf && it >= cache_from && it < launches) ? cache_buf : nullptr;
     Lw.cache_init = it == cache_from ? 1 : 0;
+  };
+  // (per launch, after set_cache: the search blocks per hypothesis if iteration `it` runs split, else 0.  The split
+  //  launches of an align stay a prefix of its launches: a moment launch waits for the count of search launches before it.)
+  bool split_prefix = true;
+  auto split_bph = [&](int it) {
+    split_prefix = split_prefix && split_iteration(ctx, it == 0 ? Lc : Lw, H, it == 0 ? g_cold : g_warm, it == 0);
+    return split_prefix ? (it == 0 ? search_bph_cold : search_bph_warm) : 0;
   };
   ctx->prof_launches = 0;
   ctx->prof_chain_ends = 0;
@@ -1623,16 +1901,17 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
     // the anchor launch above ran on the main stream for all hypotheses: the fork event orders it
     for (int c = 0; c < S; ++c) PEB_CUDA(ctx, cudaStreamWaitEvent(ctx->sub_streams[c], ctx->fork_event, 0));
     for (int it = 0; it <= launches; ++it) {
+      Lc.launch_idx = Lw.launch_idx = it;
+      set_cache(it);
+      const int sb = it < launches ? split_bph(it) : 0;
       for (int c = 0; c < S; ++c) {
         const size_t h0 = c * per, h1 = std::min(H, h0 + per);
         if (h0 >= h1) continue;
         StreamSwap swap(ctx, ctx->sub_streams[c]);
-        Lc.launch_idx = Lw.launch_idx = it;
-        set_cache(it);
         if (it == 0) {
-          PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, chunk_of(Lc, h0), h1 - h0, prm->estimator));
+          PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, chunk_of(Lc, h0), h1 - h0, prm->estimator, sb));
         } else if (it < launches) {
-          PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, chunk_of(Lw, h0), h1 - h0, prm->estimator));
+          PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, chunk_of(Lw, h0), h1 - h0, prm->estimator, sb));
         } else {
           // profile 1: the span ends with the last ITERATION launch of the slowest chain, as in the single-chain path
           // (peb_profile_read takes the maximum over the chains)
@@ -1653,13 +1932,14 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
 
   if (!per_launch) PEB_TRY(prof_mark(ctx, 0));
   for (int it = 0; it < launches; ++it) {
-    if (per_launch) PEB_TRY(prof_mark(ctx, 2 * it));
+    if (per_launch) PEB_TRY(prof_mark(ctx, 2 * it));  // (a split iteration: both of its launches between the marks)
     Lc.launch_idx = Lw.launch_idx = it;
     set_cache(it);
+    const int sb = split_bph(it);
     if (it == 0)
-      PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, Lc, H, prm->estimator));
+      PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, Lc, H, prm->estimator, sb));
     else
-      PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, Lw, H, prm->estimator));
+      PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, Lw, H, prm->estimator, sb));
     if (per_launch) PEB_TRY(prof_mark(ctx, 2 * it + 1));
   }
   Lw.launch_idx = launches;  // the fitness launch needs all iteration launches of its hypothesis

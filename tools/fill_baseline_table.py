@@ -32,7 +32,9 @@ def main():
     cores = cb["cores"]
     rl = d["roofline"]
     c4_bytes = rl["algorithmic_bytes_per_launch"] * d["config"]["iterations"]
-    traffic = json.loads((ROOT / "profiles" / "roofline_traffic.json").read_text())["icp_iteration_kernel_batch_bytes_per_launch"]
+    traffic = rl.get("traffic")  # ncu DRAM bytes per launch (profiles/roofline_traffic.json), null when none is recorded
+    traffic_note = (f"DRAM traffic per launch measured by ncu: {traffic / 1e9:.2f} GB, `profiles/roofline_traffic.json`"
+                    if traffic else "DRAM traffic per launch: not measured for this launch structure")
     rows = [
         "| config | stage | GPU ms (median, cold L2) | algorithmic bytes | achieved GB/s | % of measured HBM (6 544.7 GB/s) | CPU oracle ms (threads) | parity (test) |",
         "|---|---|---|---|---|---|---|---|",
@@ -73,8 +75,7 @@ def main():
         "",
         f"C4 roofline of the dominant kernel: {rl['achieved']:.0f} GB/s = {rl['frac']:.3f} of {rl['peak']} GB/s "
         f"(algorithmic {rl['algorithmic_bytes_per_launch'] / 1e9:.3f} GB per launch = 40 B per query; average launch "
-        f"{rl['avg_launch_ms']:.2f} ms; DRAM traffic per launch measured by ncu: {traffic / 1e9:.2f} GB, "
-        f"`profiles/roofline_traffic.json`).  End to end from host buffers: {d['e2e']['value']:.0f} hypotheses/s.",
+        f"{rl['avg_launch_ms']:.2f} ms; {traffic_note}).  End to end from host buffers: {d['e2e']['value']:.0f} hypotheses/s.",
         "",
         f"Source: `{src.name}` (B200, SM clock {d['clocks']['sm_mhz']} MHz, throttle reasons {d['clocks']['reasons']}); CPU = "
         f"{cb['what']}; the GPU box had {cores} host cores.",
