@@ -151,7 +151,10 @@ PEB_API uint64_t peb_ctx_launch_count(const peb_ctx* ctx);
  * along the local surface normal is proven far beyond the triangle inequality), "warm_graph_peek" (default 1: in graph launches 1 .. this, a query whose row cannot certify
  * looks at the four nearest neighbours of its previous match before it walks the grid), "warm_graph_queue" (default 0;
  * 8 / 16: every warp queues the unproven queries of a tile of that many passes and walks the grid for them 32 at a
- * time — icp.cu : icp_iteration_graphq_kernel; byte-identical, measured -7 %, profiles/r2_ai_graph_queue.txt) */
+ * time — icp.cu : icp_iteration_graphq_kernel; byte-identical, measured -7 %, profiles/r2_ai_graph_queue.txt).
+ * An align with a rejector chain (peb_icp_align_ex) always runs split with whole-grid launch dependencies: there
+ * "split_moments", "split_min_hyp", "cert_margin_x1000", "warm_bin", "warm_graph_queue", "nn_cache_from",
+ * "warm_upfront", "nn_group" and "flag_deps" have no effect. */
 PEB_API int peb_ctx_set_int(peb_ctx* ctx, const char* key, int value);
 
 /* ---- pcl::VoxelGrid<PointXYZ>::filter  [PCL] filters/.../impl/voxel_grid.hpp -------- */
@@ -358,6 +361,37 @@ PEB_API int peb_icp_align(peb_ctx* ctx, const float guess[16], const peb_icp_par
 PEB_API int peb_icp_align_batch(peb_ctx* ctx, const float* guesses, size_t n_guesses,
                                 const peb_icp_params* params, peb_icp_result* results);
 
+/* ---- correspondence rejectors: pcl::Registration::addCorrespondenceRejector ---------------------------------
+ * A chain of rejectors runs in every ICP iteration after the correspondence search, in the order given; each one
+ * sees what the one before kept, and the pairs left at the end feed min_correspondences, the estimator, last_mse and
+ * n_correspondences (getFitnessScore is not affected).  params->rejector_max_dist > 0 stays a DISTANCE rejector in
+ * front of the chain.  [PCL] registration/src/correspondence_rejection_{distance,median_distance,one_to_one,trimmed}.cpp
+ * (restated from recollection, DESIGN.md section 12):
+ *   DISTANCE         keep iff d2 < value^2 (the limit stored as a float)
+ *   MEDIAN_DISTANCE  score = the squared norm of (moved source - target) as a float Vector4f, ((dx dx + dz dz) + dy dy);
+ *                    median = the (m / 2)-th smallest score (m pairs in); keep iff score <= median * value (value =
+ *                    setMedianFactor, 1.0 in PCL: a factor on SQUARED distances)
+ *   ONE_TO_ONE       per target point the pair of smallest d2; a tie goes to the smaller source index (value unused)
+ *   TRIMMED          r = value clamped to [0, 1] (setOverlapRatio, 0.5 in PCL), n_keep = max(floor(r * m) in float,
+ *                    min_correspondences); the n_keep pairs of smallest (d2, source index), all if n_keep >= m
+ * An align with a chain runs every iteration as a search launch, one rejector launch and a moment launch (icp.cu :
+ * icp_reject_kernel).  ONE_TO_ONE keeps a table of H x (finite target points) x 8 bytes on the device (4.1 GB for 1024
+ * hypotheses and a 500 000-point scene); PEB_E_OOM if it cannot be allocated.  At most PEB_MAX_REJECTORS entries;
+ * an unknown kind, a non-finite value, a negative min_correspondences or chain == NULL with n_chain > 0 is
+ * PEB_E_INVALID_ARG.  n_chain == 0 is exactly the entry point without _ex. */
+enum { PEB_REJECTOR_DISTANCE = 0, PEB_REJECTOR_MEDIAN_DISTANCE = 1, PEB_REJECTOR_ONE_TO_ONE = 2, PEB_REJECTOR_TRIMMED = 3 };
+enum { PEB_MAX_REJECTORS = 8 };
+typedef struct peb_rejector {
+  int32_t kind;                 /* PEB_REJECTOR_*                                                       */
+  int32_t min_correspondences;  /* TRIMMED: setMinCorrespondences (0); otherwise 0                      */
+  double value;                 /* DISTANCE: max distance (m); MEDIAN: factor; TRIMMED: overlap ratio   */
+} peb_rejector;
+PEB_API int peb_icp_align_ex(peb_ctx* ctx, const float guess[16], const peb_icp_params* params, const peb_rejector* chain,
+                             size_t n_chain, peb_icp_result* result, float* out_aligned_xyz4, int32_t* out_corr_idx,
+                             float* out_corr_d2);
+PEB_API int peb_icp_align_batch_ex(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_icp_params* params,
+                                   const peb_rejector* chain, size_t n_chain, peb_icp_result* results);
+
 /* pcl::Registration::getFitnessScore(max_range) for an arbitrary transform */
 PEB_API int peb_fitness_score(peb_ctx* ctx, const float T[16], double max_range, double* out_fitness,
                               int32_t* out_n_inliers);
@@ -398,6 +432,9 @@ PEB_API int peb_multi_source_set(peb_multi* m, const void* pts, size_t n, size_t
 /* peb_icp_align_batch, sharded: guesses H x 16 floats, results H records, hypothesis order */
 PEB_API int peb_multi_icp_align_batch(peb_multi* m, const float* guesses, size_t n_guesses,
                                       const peb_icp_params* params, peb_icp_result* results);
+/* peb_icp_align_batch_ex, sharded the same way */
+PEB_API int peb_multi_icp_align_batch_ex(peb_multi* m, const float* guesses, size_t n_guesses, const peb_icp_params* params,
+                                         const peb_rejector* chain, size_t n_chain, peb_icp_result* results);
 /* kernel launches of all contexts so far */
 PEB_API uint64_t peb_multi_launch_count(const peb_multi* m);
 

@@ -265,22 +265,36 @@ class IterativeClosestPoint {
   void setRANSACIterations(int n) {
     if (n) throw Error(PEB_E_UNSUPPORTED, "the RANSAC rejector has no CUDA path (no CPU fallback)");
   }
-  // addCorrespondenceRejector(CorrespondenceRejectorDistance with setMaximumDistance(d))
-  void addCorrespondenceRejectorDistance(double max_distance) { params_.rejector_max_dist = max_distance; }
+  // addCorrespondenceRejector(CorrespondenceRejectorDistance with setMaximumDistance(d)): before any other rejector it
+  // sets params().rejector_max_dist, the head of the chain; after one it joins the chain, so PCL's order is kept
+  void addCorrespondenceRejectorDistance(double max_distance) {
+    if (chain_.empty()) params_.rejector_max_dist = max_distance;
+    else add_rejector(PEB_REJECTOR_DISTANCE, max_distance, 0);
+  }
+  // addCorrespondenceRejector(CorrespondenceRejectorMedianDistance with setMedianFactor(factor))
+  void addCorrespondenceRejectorMedianDistance(double factor = 1.0) { add_rejector(PEB_REJECTOR_MEDIAN_DISTANCE, factor, 0); }
+  // addCorrespondenceRejector(CorrespondenceRejectorOneToOne)
+  void addCorrespondenceRejectorOneToOne() { add_rejector(PEB_REJECTOR_ONE_TO_ONE, 0.0, 0); }
+  // addCorrespondenceRejector(CorrespondenceRejectorTrimmed with setOverlapRatio(ratio), setMinCorrespondences(min_corr))
+  void addCorrespondenceRejectorTrimmed(double ratio = 0.5, int min_corr = 0) { add_rejector(PEB_REJECTOR_TRIMMED, ratio, min_corr); }
+  // the rejectors after params().rejector_max_dist, in the order they were added (peb_icp_align_ex)
+  const std::vector<peb_rejector>& correspondenceRejectors() const { return chain_; }
   ConvergenceCriteria* getConvergeCriteria() { return &criteria_; }
 
   // align(output, guess): out_xyz4 (nullable) receives final * input as x y z 1 records
   void align(std::vector<float>* out_xyz4 = nullptr, const float* guess16 = nullptr) {
     if (out_xyz4) out_xyz4->resize(4 * n_src_);
-    c_.check(peb_icp_align(c_.get(), guess16, &params_, &result_, out_xyz4 && n_src_ ? out_xyz4->data() : nullptr, nullptr,
-                           nullptr));
+    float* out = out_xyz4 && n_src_ ? out_xyz4->data() : nullptr;
+    if (chain_.empty()) c_.check(peb_icp_align(c_.get(), guess16, &params_, &result_, out, nullptr, nullptr));
+    else c_.check(peb_icp_align_ex(c_.get(), guess16, &params_, chain_.data(), chain_.size(), &result_, out, nullptr, nullptr));
     criteria_.state_ = result_.state;
   }
   // H initial poses against one source / one target: the call shape of
   // cv::ppf_match_3d::ICP::registerModelToScene(model, scene, poses), opencv_surface_match.cpp:94
   void alignBatch(const float* guesses16, size_t n_guesses, std::vector<peb_icp_result>& results) {
     results.resize(n_guesses);
-    c_.check(peb_icp_align_batch(c_.get(), guesses16, n_guesses, &params_, results.data()));
+    if (chain_.empty()) c_.check(peb_icp_align_batch(c_.get(), guesses16, n_guesses, &params_, results.data()));
+    else c_.check(peb_icp_align_batch_ex(c_.get(), guesses16, n_guesses, &params_, chain_.data(), chain_.size(), results.data()));
   }
   bool hasConverged() const { return result_.converged != 0; }
   const float* getFinalTransformation() const { return result_.T; }  // column-major 4x4
@@ -293,6 +307,18 @@ class IterativeClosestPoint {
   int nr_iterations() const { return result_.iterations; }
   const peb_icp_result& result() const { return result_; }
   const peb_icp_params& params() const { return params_; }
+
+ private:
+  void add_rejector(int kind, double value, int min_corr) {
+    if (chain_.size() >= PEB_MAX_REJECTORS)
+      throw Error(PEB_E_INVALID_ARG, "at most " + std::to_string(PEB_MAX_REJECTORS) + " correspondence rejectors after the distance one");
+    peb_rejector r;
+    r.kind = kind;
+    r.min_correspondences = min_corr;
+    r.value = value;
+    chain_.push_back(r);
+  }
+  std::vector<peb_rejector> chain_;
 
  protected:
   Context& c_;
@@ -531,19 +557,22 @@ class MultiContext {
 // Configure a pe_b200::IterativeClosestPoint(+WithNormals) with PCL's setters as usual and hand it over as `like`.
 class MultiDeviceICP {
  public:
-  MultiDeviceICP(MultiContext& m, const IterativeClosestPoint& like) : m_(m), params_(like.params()) {}
+  MultiDeviceICP(MultiContext& m, const IterativeClosestPoint& like)
+      : m_(m), params_(like.params()), chain_(like.correspondenceRejectors()) {}
   void setInputSource(const void* pts, size_t n, size_t stride = 16) { m_.check(peb_multi_source_set(m_.get(), pts, n, stride)); }
   void setInputTarget(const void* pts, size_t n, size_t stride = 16, const void* normals = nullptr, size_t nstride = 32) {
     m_.check(peb_multi_target_set(m_.get(), pts, n, stride, normals, nstride));
   }
   void alignBatch(const float* guesses16, size_t n_guesses, std::vector<peb_icp_result>& results) {
     results.resize(n_guesses);
-    m_.check(peb_multi_icp_align_batch(m_.get(), guesses16, n_guesses, &params_, results.data()));
+    if (chain_.empty()) m_.check(peb_multi_icp_align_batch(m_.get(), guesses16, n_guesses, &params_, results.data()));
+    else m_.check(peb_multi_icp_align_batch_ex(m_.get(), guesses16, n_guesses, &params_, chain_.data(), chain_.size(), results.data()));
   }
 
  private:
   MultiContext& m_;
   peb_icp_params params_;
+  std::vector<peb_rejector> chain_;
 };
 
 }  // namespace pe_b200

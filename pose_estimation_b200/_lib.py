@@ -57,6 +57,32 @@ class IcpParams(C.Structure):
     ]
 
 
+REJECTOR_DISTANCE = 0
+REJECTOR_MEDIAN_DISTANCE = 1
+REJECTOR_ONE_TO_ONE = 2
+REJECTOR_TRIMMED = 3
+MAX_REJECTORS = 8
+
+
+class Rejector(C.Structure):
+    """peb_rejector: one entry of a correspondence rejector chain."""
+
+    _fields_ = [("kind", C.c_int32), ("min_correspondences", C.c_int32), ("value", C.c_double)]
+
+
+def rejector_array(chain):
+    """chain: Rejector records (or (kind, value[, min_correspondences]) tuples) -> (ctypes array, count)."""
+    arr = (Rejector * max(len(chain), 1))()
+    for k, r in enumerate(chain):
+        if isinstance(r, Rejector):
+            arr[k] = r
+        else:
+            arr[k].kind = int(r[0])
+            arr[k].value = float(r[1]) if len(r) > 1 else 0.0
+            arr[k].min_correspondences = int(r[2]) if len(r) > 2 else 0
+    return arr, len(chain)
+
+
 class IcpResult(C.Structure):
     """peb_icp_result (96 bytes)."""
 
@@ -175,6 +201,8 @@ SYMBOLS = {
     "peb_ctx_enable_peer": (_i, [_vp, _vp]),
     "peb_icp_align": (_i, [_vp, _vp, _pp(IcpParams), _pp(IcpResult), _vp, _vp, _vp]),
     "peb_icp_align_batch": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp]),
+    "peb_icp_align_ex": (_i, [_vp, _vp, _pp(IcpParams), _vp, _sz, _pp(IcpResult), _vp, _vp, _vp]),
+    "peb_icp_align_batch_ex": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp, _sz, _vp]),
     "peb_fitness_score": (_i, [_vp, _vp, _d, _pp(_d), _pp(C.c_int32)]),
     "peb_target_set_dev": (_i, [_vp, _vp, _sz, _vp]),
     "peb_source_set_dev": (_i, [_vp, _vp, _sz]),
@@ -196,6 +224,7 @@ SYMBOLS = {
     "peb_multi_target_set": (_i, [_vp, _vp, _sz, _sz, _vp, _sz]),
     "peb_multi_source_set": (_i, [_vp, _vp, _sz, _sz]),
     "peb_multi_icp_align_batch": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp]),
+    "peb_multi_icp_align_batch_ex": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp, _sz, _vp]),
     "peb_multi_launch_count": (C.c_uint64, [_vp]),
 }
 

@@ -3,7 +3,9 @@
 // file and there is no CPU implementation behind any entry point: if the device path cannot run,
 // the call fails with a peb_status and a message.
 #include <algorithm>
+#include <cmath>
 #include <cstring>
+#include <string>
 #include <new>
 
 #include "core_math.cuh"
@@ -783,6 +785,28 @@ PEB_API int peb_nn_search_bruteforce(peb_ctx* ctx, const void* queries, size_t n
 }
 
 // ---- ICP ---------------------------------------------------------------------------------------------
+// a rejector chain from the caller (include/pe_b200.h : peb_rejector): "" if it is valid, else why not
+static std::string chain_error(const peb_rejector* chain, size_t n_chain) {
+  if (n_chain == 0) return "";
+  if (!chain) return "null rejector chain with n_chain > 0";
+  if (n_chain > PEB_MAX_REJECTORS)
+    return "rejector chain of " + std::to_string(n_chain) + " entries (at most " + std::to_string(PEB_MAX_REJECTORS) + ")";
+  for (size_t s = 0; s < n_chain; ++s) {
+    const peb_rejector& r = chain[s];
+    const std::string at = "rejector " + std::to_string(s) + ": ";
+    if (r.kind != PEB_REJECTOR_DISTANCE && r.kind != PEB_REJECTOR_MEDIAN_DISTANCE && r.kind != PEB_REJECTOR_ONE_TO_ONE &&
+        r.kind != PEB_REJECTOR_TRIMMED)
+      return at + "unknown kind " + std::to_string(r.kind);
+    if (!std::isfinite(r.value)) return at + "non-finite value";
+    if (r.min_correspondences < 0) return at + "negative min_correspondences";
+  }
+  return "";
+}
+
+static int check_chain(peb_ctx* ctx, const char* what, const peb_rejector* chain, size_t n_chain) {
+  const std::string e = chain_error(chain, n_chain);
+  return e.empty() ? PEB_OK : fail(ctx, PEB_E_INVALID_ARG, "%s: %s", what, e.c_str());
+}
 static int icp_align_batch_dev_impl(peb_ctx* ctx, const float* d_guesses, size_t n_guesses, const peb_icp_params* params,
                                     peb_icp_result* d_results) {
   if (!ctx || !params) return PEB_E_INVALID_ARG;
@@ -800,13 +824,15 @@ static int icp_align_dev_impl(peb_ctx* ctx, const float guess[16], const peb_icp
 }
 
 static int icp_align_impl(peb_ctx* ctx, const float guess[16], const peb_icp_params* params, peb_icp_result* result,
-                          float* out_aligned_xyz4, int32_t* out_corr_idx, float* out_corr_d2) {
+                          float* out_aligned_xyz4, int32_t* out_corr_idx, float* out_corr_d2,
+                          const peb_rejector* chain = nullptr, size_t n_chain = 0) {
   if (!ctx || !params || !result) return PEB_E_INVALID_ARG;
+  PEB_TRY(check_chain(ctx, "peb_icp_align_ex", chain, n_chain));
   DeviceGuard guard(ctx->device);
   const float* d_g = nullptr;
   PEB_TRY(upload_guesses(ctx, guess, 1, &d_g));
   PEB_CUDA(ctx, ctx->d_results.ensure(sizeof(peb_icp_result)));
-  PEB_TRY(icp_align_device(ctx, d_g, 1, params, ctx->d_results.as<peb_icp_result>(), true));
+  PEB_TRY(icp_align_device(ctx, d_g, 1, params, ctx->d_results.as<peb_icp_result>(), true, chain, static_cast<int>(n_chain)));
   const size_t n = ctx->n_src;
   PEB_CUDA(ctx, cudaMemcpyAsync(result, ctx->d_results.p, sizeof(peb_icp_result), cudaMemcpyDeviceToHost, ctx->stream));
   if (out_aligned_xyz4 && n) {
@@ -824,15 +850,17 @@ static int icp_align_impl(peb_ctx* ctx, const float guess[16], const peb_icp_par
 }
 
 static int icp_align_batch_impl(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_icp_params* params,
-                                peb_icp_result* results) {
+                                peb_icp_result* results, const peb_rejector* chain = nullptr, size_t n_chain = 0) {
   if (!ctx || !params) return PEB_E_INVALID_ARG;
+  PEB_TRY(check_chain(ctx, "peb_icp_align_batch_ex", chain, n_chain));
   DeviceGuard guard(ctx->device);
   if (n_guesses == 0) return PEB_OK;
   if (!guesses || !results) return fail(ctx, PEB_E_INVALID_ARG, "align_batch: null guesses / results");
   const float* d_g = nullptr;
   PEB_TRY(upload_guesses(ctx, guesses, n_guesses, &d_g));
   PEB_CUDA(ctx, ctx->d_results.ensure(n_guesses * sizeof(peb_icp_result)));
-  PEB_TRY(icp_align_device(ctx, d_g, n_guesses, params, ctx->d_results.as<peb_icp_result>(), false));
+  PEB_TRY(icp_align_device(ctx, d_g, n_guesses, params, ctx->d_results.as<peb_icp_result>(), false, chain,
+                           static_cast<int>(n_chain)));
   PEB_CUDA(ctx, cudaMemcpyAsync(results, ctx->d_results.p, n_guesses * sizeof(peb_icp_result), cudaMemcpyDeviceToHost,
                                 ctx->stream));
   // the error flag of the dependency waits is read AFTER every launch of the align has finished: a record written
@@ -1002,6 +1030,45 @@ PEB_API int peb_icp_align(peb_ctx* ctx, const float guess[16], const peb_icp_par
 
 PEB_API int peb_icp_align_batch(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_icp_params* params, peb_icp_result* results) {
   return guarded(ctx, "peb_icp_align_batch", [&]() { return icp_align_batch_impl(ctx, guesses, n_guesses, params, results); });
+}
+
+PEB_API int peb_icp_align_ex(peb_ctx* ctx, const float guess[16], const peb_icp_params* params, const peb_rejector* chain,
+                             size_t n_chain, peb_icp_result* result, float* out_aligned_xyz4, int32_t* out_corr_idx,
+                             float* out_corr_d2) {
+  return guarded(ctx, "peb_icp_align_ex", [&]() {
+    return icp_align_impl(ctx, guess, params, result, out_aligned_xyz4, out_corr_idx, out_corr_d2, chain, n_chain);
+  });
+}
+
+PEB_API int peb_icp_align_batch_ex(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_icp_params* params,
+                                   const peb_rejector* chain, size_t n_chain, peb_icp_result* results) {
+  return guarded(ctx, "peb_icp_align_batch_ex",
+                 [&]() { return icp_align_batch_impl(ctx, guesses, n_guesses, params, results, chain, n_chain); });
+}
+
+// (here rather than in multi.cu, which is also compiled against fake single-device entry points that have no _ex)
+PEB_API int peb_multi_icp_align_batch_ex(peb_multi* m, const float* guesses, size_t n_guesses, const peb_icp_params* params,
+                                         const peb_rejector* chain, size_t n_chain, peb_icp_result* results) {
+  if (!m || !params) return PEB_E_INVALID_ARG;
+  if (n_guesses == 0) return PEB_OK;
+  if (!guesses || !results) return multi_set_error(m, PEB_E_INVALID_ARG, "peb_multi_icp_align_batch_ex: null guesses / results");
+  try {
+    const std::string e = chain_error(chain, n_chain);
+    if (!e.empty()) return multi_set_error(m, PEB_E_INVALID_ARG, ("peb_multi_icp_align_batch_ex: " + e).c_str());
+  } catch (...) {
+    return multi_set_error(m, PEB_E_OOM, "peb_multi_icp_align_batch_ex: out of host memory");
+  }
+  struct Job {
+    const float* guesses;
+    const peb_icp_params* params;
+    const peb_rejector* chain;
+    size_t n_chain;
+    peb_icp_result* results;
+  } job{guesses, params, chain, n_chain, results};
+  return multi_run_sharded(m, "peb_multi_icp_align_batch_ex", n_guesses, [](peb_ctx* c, size_t lo, size_t hi, void* user) {
+    const Job* j = static_cast<const Job*>(user);
+    return peb_icp_align_batch_ex(c, j->guesses + 16 * lo, hi - lo, j->params, j->chain, j->n_chain, j->results + lo);
+  }, &job);
 }
 
 }  // extern "C"

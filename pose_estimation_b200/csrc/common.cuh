@@ -188,6 +188,9 @@ struct peb_ctx {
   peb::DevBuf slack;         // float per working point: remaining certificate of its match
   peb::DevBuf corr_idx, corr_d2;
   peb::DevBuf partials;      // per-block double partial sums
+  peb::DevBuf rej_kept;      // rejector chains: one kept byte per working point (icp.cu : icp_reject_kernel)
+  peb::DevBuf rej_o2o;       // ... the one-to-one rejector's H x target-point keys, all ones between aligns
+  bool rej_o2o_clean = false;  // rej_o2o holds all ones (an align that stopped queueing half-way may have left keys)
   peb::DevBuf state;         // IcpState per hypothesis
   peb::DevBuf trace;         // per-iteration increments of the last single align
   peb::DevBuf d_guesses, d_results, d_aligned;
@@ -271,8 +274,15 @@ int exclusive_scan_u32(peb_ctx* ctx, const uint32_t* in, uint32_t* out, int n, u
 int grid_build(peb_ctx* ctx, Grid* g, const float4* d_pts, const float4* d_normals, int n, float occupancy);
 int bbox_finite(peb_ctx* ctx, const float4* d_pts, int n, float mn[3], float mx[3], int* n_finite);
 // icp.cu
+// chain / n_chain: a rejector chain, checked by the caller (n_chain 0: none)
 int icp_align_device(peb_ctx* ctx, const float* d_guesses /*nullable: identity*/, size_t H, const peb_icp_params* prm,
-                     peb_icp_result* d_results, bool single_mode);
+                     peb_icp_result* d_results, bool single_mode, const peb_rejector* chain = nullptr, int n_chain = 0);
+// multi.cu: fn(ctx i, lo, hi) on every context of m with its shard [lo, hi) of n_items (skipped when empty), device 0's
+// on the calling thread; the first failing context is reported in m's error text
+int multi_run_sharded(peb_multi* m, const char* what, size_t n_items, int (*fn)(peb_ctx*, size_t lo, size_t hi, void* user),
+                      void* user);
+// m's error text
+int multi_set_error(peb_multi* m, int code, const char* msg);
 int icp_output_device(peb_ctx* ctx, float4* d_out);
 int nn_search_device(peb_ctx* ctx, const float4* d_q, int nq, int32_t* d_idx, float* d_d2);
 // fitness of one transform (device, 16 floats); the record's n_correspondences carries the inlier count

@@ -25,6 +25,7 @@
 // incremental float update is reproduced exactly for every hypothesis.
 #include <algorithm>
 
+#include "block_select.cuh"
 #include "nn_cache.cuh"
 #include "nn_graph.cuh"
 #include "nn_search.cuh"
@@ -775,8 +776,10 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_search_kernel(const IcpLa
   }
 }
 
-template <int EST, int MB>
-__global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLaunch L) {
+// CHAIN: the align has a rejector chain (icp_reject_kernel ran between the two launches): a pair is summed iff
+// kept[i] of its hypothesis is set, and the single align's correspondence outputs are written here.
+template <int EST, int MB, bool CHAIN>
+__global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLaunch L, const unsigned char* __restrict__ kept) {
   if (L.epochs == nullptr) {
     pdl_trigger_and_wait();
   } else {
@@ -804,6 +807,23 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLa
     if (j <= -2) {  // made non-finite by this launch's transform: searched all the same (see above)
       valid = true;
       j = -2 - j;
+    }
+    if (CHAIN) {
+      NnBest best;
+      const bool keep = valid && j >= 0 && kept[static_cast<size_t>(h) * L.n_src + i];
+      if (keep) {
+        const float4 t = L.grid.pts[j];
+        best.d2 = l2_simple(p.x, p.y, p.z, t.x, t.y, t.z);
+        best.idx = point_index(t);
+        best.j = j;
+        accumulate_pair<EST>(L.grid, p, best, acc);
+      }
+      if (L.corr_idx) {
+        const int orig = __float_as_int(L.src[i].w);
+        L.corr_idx[orig] = keep ? best.idx : -1;
+        L.corr_d2[orig] = keep ? best.d2 : 0.0f;
+      }
+      continue;
     }
     if (!valid || j < 0) continue;
     const float4 t = L.grid.pts[j];
@@ -836,6 +856,199 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLa
       __threadfence();
       atomicAdd(L.epochs + h, still_active ? 1 : kEpochStopped);
     }
+  }
+}
+
+// ---- correspondence rejectors (peb_icp_align_ex) --------------------------------------------------------------------
+// An align with a rejector chain runs every iteration as three launches: icp_search_kernel, icp_reject_kernel and
+// icp_moment_kernel<CHAIN = true>.  Between the search and the moments every pair of the iteration is known and no moment
+// has been summed: the reject launch gives every hypothesis one block of kRejThreads threads, which applies the threshold,
+// rejector_max_dist and then the chain in order to all pairs of its hypothesis (a __syncthreads between stages) and leaves
+// one kept byte per working point.  One block sees the whole pair set, so the order statistics and the one-to-one table
+// need no cross-block protocol; the launches wait for the whole previous grid (griddepcontrol.wait, no epoch flags).
+//   MEDIAN_DISTANCE  score (rej_score), exact (m / 2)-th order statistic over the kept pairs (block_select_nth), keep iff
+//                    (double) score <= median * factor.
+//   TRIMMED          the (n_keep - 1)-th smallest d2 v over the kept pairs; all pairs below v stay, and of the pairs AT v the
+//                    ones of the smallest original source indices (a second select over those indices) fill n_keep.
+//   ONE_TO_ONE       atomicMin of (d2 bits << 32 | original source index) into the hypothesis's row of the table (indexed by
+//                    the match's sorted position), then every pair reads its entry back: the one that finds its own key
+//                    wins and resets the entry to all ones.  A loser reads the winner's key or all ones, never its own, so
+//                    the table is all ones again after every stage without a pass over it (it is set once, when allocated).
+// Sign bits are cleared before a select (a NaN distance from a non-finite working point sorts last instead of being lost).
+constexpr int kRejThreads = 1024;
+
+struct RejChain {
+  int kind[PEB_MAX_REJECTORS];
+  int min_corr[PEB_MAX_REJECTORS];
+  double value[PEB_MAX_REJECTORS];
+  int n;
+  unsigned char* kept;         // H x n_src: the pair of working point i survives the chain
+  unsigned long long* o2o;     // H x grid.n one-to-one keys, all ones between stages (nullptr without ONE_TO_ONE)
+};
+
+// the pair of working point i as the moment launch reads it (best.idx = -1: no pair)
+__device__ __forceinline__ NnBest rej_pair(const IcpLaunch& L, const float4* __restrict__ work, int i, float4& p, bool& valid) {
+  p = __ldcg(work + i);
+  valid = finite3(p.x, p.y, p.z);
+  int j = __float_as_int(p.w);
+  if (j <= -2) {
+    valid = true;
+    j = -2 - j;
+  }
+  NnBest best;
+  best.d2 = pos_inf();
+  best.idx = -1;
+  best.j = -1;
+  if (valid && j >= 0) {
+    const float4 t = L.grid.pts[j];
+    best.d2 = l2_simple(p.x, p.y, p.z, t.x, t.y, t.z);
+    best.idx = point_index(t);
+    best.j = j;
+  }
+  return best;
+}
+
+__device__ __forceinline__ unsigned abs_bits(float v) { return __float_as_uint(v) & 0x7FFFFFFFu; }
+
+// [PCL] CorrespondenceRejectorMedianDistance's score: DataContainer::getCorrespondenceScore, (src.getVector4fMap() -
+// tgt.getVector4fMap()).squaredNorm() in float, w = 1 on both sides; Eigen's 4-lane reduction (v0 + v2) + (v1 + v3),
+// the last term 0.  Written without contraction (the library is built with -fmad=false).
+__device__ __forceinline__ float rej_score(const IcpLaunch& L, const float4& p, int j) {
+  const float4 t = L.grid.pts[j];
+  const float dx = p.x - t.x, dy = p.y - t.y, dz = p.z - t.z;
+  return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dz, dz)), __fmul_rn(dy, dy));
+}
+
+// number of kept pairs of the block's hypothesis (every thread gets it)
+__device__ __forceinline__ int rej_count(const unsigned char* kept, int n) {
+  int m = 0;
+  for (int base = 0; base < n; base += kRejThreads) {
+    const int i = base + threadIdx.x;
+    m += __syncthreads_count(i < n && kept[i]);
+  }
+  return m;
+}
+
+__global__ void __launch_bounds__(kRejThreads, 1) icp_reject_kernel(const IcpLaunch L, const RejChain R) {
+  pdl_trigger_and_wait();
+  __shared__ unsigned hist[2048];
+  __shared__ unsigned s_state[2];
+  __shared__ unsigned s_wsum[32];
+  __shared__ int s_active;
+  const int h = blockIdx.x;
+  if (threadIdx.x == 0) s_active = __ldcg(&L.states[h].active);
+  __syncthreads();
+  if (!s_active) return;
+  const int n = L.n_src;
+  const float4* work = L.work + static_cast<size_t>(h) * n;
+  unsigned char* kept = R.kept + static_cast<size_t>(h) * n;
+  unsigned long long* tab = R.o2o ? R.o2o + static_cast<size_t>(h) * L.grid.n : nullptr;
+  for (int i = threadIdx.x; i < n; i += kRejThreads) {
+    float4 p;
+    bool valid;
+    const NnBest b = rej_pair(L, work, i, p, valid);
+    kept[i] = keep_pair(L, valid, b) ? 1 : 0;
+  }
+  __syncthreads();
+  for (int s = 0; s < R.n; ++s) {
+    const int kind = R.kind[s];
+    if (kind == PEB_REJECTOR_DISTANCE) {
+      const float lim = static_cast<float>(R.value[s] * R.value[s]);
+      for (int i = threadIdx.x; i < n; i += kRejThreads) {
+        if (!kept[i]) continue;
+        float4 p;
+        bool valid;
+        const NnBest b = rej_pair(L, work, i, p, valid);
+        if (!(b.d2 < lim)) kept[i] = 0;
+      }
+    } else if (kind == PEB_REJECTOR_MEDIAN_DISTANCE) {
+      const int m = rej_count(kept, n);
+      if (m == 0) continue;
+      auto score = [&](int i) {
+        if (!kept[i]) return -1.0f;
+        float4 p;
+        bool valid;
+        const NnBest b = rej_pair(L, work, i, p, valid);
+        return __uint_as_float(abs_bits(rej_score(L, p, b.j)));
+      };
+      const float med = block_select_nth<decltype(score), true>(score, n, m / 2, hist, s_state, s_wsum);
+      const double lim = static_cast<double>(med) * R.value[s];
+      for (int i = threadIdx.x; i < n; i += kRejThreads) {
+        if (!kept[i]) continue;
+        float4 p;
+        bool valid;
+        const NnBest b = rej_pair(L, work, i, p, valid);
+        if (!(static_cast<double>(rej_score(L, p, b.j)) <= lim)) kept[i] = 0;
+      }
+    } else if (kind == PEB_REJECTOR_ONE_TO_ONE) {
+      for (int i = threadIdx.x; i < n; i += kRejThreads) {
+        if (!kept[i]) continue;
+        float4 p;
+        bool valid;
+        const NnBest b = rej_pair(L, work, i, p, valid);
+        const unsigned long long key = (static_cast<unsigned long long>(abs_bits(b.d2)) << 32) |
+                                       static_cast<unsigned>(__float_as_int(L.src[i].w));
+        atomicMin(tab + b.j, key);
+      }
+      __syncthreads();
+      for (int i = threadIdx.x; i < n; i += kRejThreads) {
+        if (!kept[i]) continue;
+        float4 p;
+        bool valid;
+        const NnBest b = rej_pair(L, work, i, p, valid);
+        const unsigned long long key = (static_cast<unsigned long long>(abs_bits(b.d2)) << 32) |
+                                       static_cast<unsigned>(__float_as_int(L.src[i].w));
+        if (__ldcg(tab + b.j) == key) __stcg(tab + b.j, ~0ull);
+        else kept[i] = 0;
+      }
+    } else {  // PEB_REJECTOR_TRIMMED
+      const int m = rej_count(kept, n);
+      const float ratio = fminf(1.0f, fmaxf(0.0f, static_cast<float>(R.value[s])));
+      const int n_keep = max(static_cast<int>(floorf(ratio * static_cast<float>(m))), R.min_corr[s]);
+      if (n_keep >= m) continue;
+      unsigned vb = 0u;  // the d2 bits of the cut
+      int o_cut = -1;    // pairs at the cut with source index <= o_cut stay
+      if (n_keep > 0) {
+        auto d2_of = [&](int i) {
+          if (!kept[i]) return -1.0f;
+          float4 p;
+          bool valid;
+          return __uint_as_float(abs_bits(rej_pair(L, work, i, p, valid).d2));
+        };
+        vb = __float_as_uint(block_select_nth<decltype(d2_of), true>(d2_of, n, n_keep - 1, hist, s_state, s_wsum));
+        int below = 0;
+        for (int base = 0; base < n; base += kRejThreads) {
+          const int i = base + threadIdx.x;
+          bool lt = false;
+          if (i < n && kept[i]) {
+            float4 p;
+            bool valid;
+            lt = abs_bits(rej_pair(L, work, i, p, valid).d2) < vb;
+          }
+          below += __syncthreads_count(lt);
+        }
+        auto src_at_cut = [&](int i) {
+          if (!kept[i]) return -1.0f;
+          float4 p;
+          bool valid;
+          if (abs_bits(rej_pair(L, work, i, p, valid).d2) != vb) return -1.0f;
+          return __int_as_float(__float_as_int(L.src[i].w));
+        };
+        o_cut = __float_as_int(block_select_nth<decltype(src_at_cut), true>(src_at_cut, n, n_keep - below - 1, hist, s_state, s_wsum));
+      }
+      for (int i = threadIdx.x; i < n; i += kRejThreads) {
+        if (!kept[i]) continue;
+        bool stay = false;
+        if (n_keep > 0) {
+          float4 p;
+          bool valid;
+          const unsigned db = abs_bits(rej_pair(L, work, i, p, valid).d2);
+          stay = db < vb || (db == vb && __float_as_int(L.src[i].w) <= o_cut);
+        }
+        if (!stay) kept[i] = 0;
+      }
+    }
+    __syncthreads();
   }
 }
 
@@ -1545,8 +1758,9 @@ bool split_iteration(const peb_ctx* ctx, const IcpLaunch& L, size_t H, int G, bo
   return !(L.warm && ctx->warm_bin);
 }
 
+// R: the align's rejector chain (nullable): a reject launch between the two, and the moments of the kept pairs
 template <bool FIRST>
-int launch_split_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
+int launch_split_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph, const RejChain* R) {
   const dim3 sgrid(search_bph, static_cast<unsigned>(H)), mgrid(L.blocks_per_hyp, static_cast<unsigned>(H));
   // (launch 0 keeps the batched cap: its cooperative verification holds more state than a warm search)
   if (FIRST)
@@ -1557,17 +1771,27 @@ int launch_split_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estim
     PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksSearch, false, 4>), sgrid, dim3(kIcpThreads), L);
   else
     PEB_LAUNCH_PDL(ctx, (icp_search_kernel<kMinBlocksSearch, false, 0>), sgrid, dim3(kIcpThreads), L);
+  if (R) {
+    PEB_LAUNCH_PDL(ctx, icp_reject_kernel, dim3(static_cast<unsigned>(H)), dim3(kRejThreads), L, *R);
+    const unsigned char* kept = R->kept;
+    if (estimator == PEB_ESTIMATOR_SVD)
+      PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_SVD, kMinBlocksBatch, true>), mgrid, dim3(kIcpThreads), L, kept);
+    else
+      PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_POINT_TO_PLANE_LLS, kMinBlocksBatch, true>), mgrid, dim3(kIcpThreads), L, kept);
+    return PEB_OK;
+  }
+  const unsigned char* none = nullptr;
   if (estimator == PEB_ESTIMATOR_SVD)
-    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_SVD, kMinBlocksBatch>), mgrid, dim3(kIcpThreads), L);
+    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_SVD, kMinBlocksBatch, false>), mgrid, dim3(kIcpThreads), L, none);
   else
-    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_POINT_TO_PLANE_LLS, kMinBlocksBatch>), mgrid, dim3(kIcpThreads), L);
+    PEB_LAUNCH_PDL(ctx, (icp_moment_kernel<PEB_ESTIMATOR_POINT_TO_PLANE_LLS, kMinBlocksBatch, false>), mgrid, dim3(kIcpThreads), L, none);
   return PEB_OK;
 }
 
 // search_bph > 0: the iteration runs split, with this many search blocks per hypothesis
 template <int G, bool FIRST>
-int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
-  if (G == 1 && search_bph > 0) return launch_split_iteration<FIRST>(ctx, L, H, estimator, search_bph);
+int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimator, int search_bph, const RejChain* R) {
+  if (G == 1 && search_bph > 0) return launch_split_iteration<FIRST>(ctx, L, H, estimator, search_bph, R);
   dim3 grid(L.blocks_per_hyp, static_cast<unsigned>(H));
   constexpr int S = PEB_ESTIMATOR_SVD, P = PEB_ESTIMATOR_POINT_TO_PLANE_LLS;
   const bool cert = G == 1 && L.margin > 0.0f;
@@ -1638,8 +1862,10 @@ int launch_one_iteration(peb_ctx* ctx, const IcpLaunch& L, size_t H, int estimat
 }
 
 // first: launch 0 of the align
-int launch_one_iteration_g(peb_ctx* ctx, int G, bool first, const IcpLaunch& L, size_t H, int estimator, int search_bph) {
-#define PEB_ICP_G(GG) return first ? launch_one_iteration<GG, true>(ctx, L, H, estimator, search_bph) : launch_one_iteration<GG, false>(ctx, L, H, estimator, search_bph)
+// R (nullable): the rejector chain; it comes with G = 1 and search_bph > 0
+int launch_one_iteration_g(peb_ctx* ctx, int G, bool first, const IcpLaunch& L, size_t H, int estimator, int search_bph,
+                           const RejChain* R = nullptr) {
+#define PEB_ICP_G(GG) return first ? launch_one_iteration<GG, true>(ctx, L, H, estimator, search_bph, R) : launch_one_iteration<GG, false>(ctx, L, H, estimator, search_bph, R)
   switch (G) {
     case 1: PEB_ICP_G(1);
     case 2: PEB_ICP_G(2);
@@ -1747,7 +1973,7 @@ int ensure_sub_streams(peb_ctx* ctx, int S) {
 }  // namespace
 
 int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_icp_params* prm,
-                     peb_icp_result* d_results, bool single_mode) {
+                     peb_icp_result* d_results, bool single_mode, const peb_rejector* chain, int n_chain) {
   if (!ctx->tgt_grid.valid) return fail(ctx, PEB_E_NO_TARGET, "align: no target set (peb_target_set)");
   if (!ctx->src_set) return fail(ctx, PEB_E_NO_SOURCE, "align: no source set (peb_source_set)");
   if (H == 0) return PEB_OK;
@@ -1761,6 +1987,37 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   IcpLaunch L{};
   PEB_TRY(prepare_launch(ctx, H, prm, L));
   L.results = d_results;
+  // a rejector chain (icp_reject_kernel): every iteration split, one lane per query, no certificate, no cache
+  const bool with_chain = n_chain > 0;
+  RejChain R{};
+  if (with_chain) {
+    L.margin = 0.0f;
+    R.n = n_chain;
+    bool o2o = false;
+    for (int s = 0; s < n_chain; ++s) {
+      R.kind[s] = chain[s].kind;
+      R.min_corr[s] = chain[s].min_correspondences;
+      R.value[s] = chain[s].value;
+      o2o = o2o || chain[s].kind == PEB_REJECTOR_ONE_TO_ONE;
+    }
+    PEB_CUDA(ctx, ctx->rej_kept.ensure(std::max<size_t>(H * static_cast<size_t>(n), 1)));
+    R.kept = ctx->rej_kept.as<unsigned char>();
+    if (o2o) {
+      const size_t bytes = std::max<size_t>(H * static_cast<size_t>(L.grid.n), 1) * sizeof(unsigned long long);
+      const size_t cap0 = ctx->rej_o2o.cap;
+      const cudaError_t e = ctx->rej_o2o.ensure(bytes);
+      if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, PEB_E_OOM, "align: the one-to-one rejector's table of %zu hypotheses x %d target points (%.2f GB) "
+                    "could not be allocated: %s", H, L.grid.n, static_cast<double>(bytes) / 1e9, cudaGetErrorString(e));
+      }
+      // all ones when allocated; every stage leaves it so (icp_reject_kernel)
+      if (ctx->rej_o2o.cap != cap0 || !ctx->rej_o2o_clean)
+        PEB_CUDA(ctx, cudaMemsetAsync(ctx->rej_o2o.p, 0xFF, ctx->rej_o2o.cap, ctx->stream));
+      ctx->rej_o2o_clean = false;  // (set again once every launch of this align is queued)
+      R.o2o = ctx->rej_o2o.as<unsigned long long>();
+    }
+  }
   if (single_mode) {
     PEB_CUDA(ctx, ctx->corr_idx.ensure(std::max(n_all, 1) * sizeof(int32_t)));
     PEB_CUDA(ctx, ctx->corr_d2.ensure(std::max(n_all, 1) * sizeof(float)));
@@ -1775,7 +2032,7 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
     L.trace_cap = cap;
     ctx->last_trace_cap = cap;
   }
-  const int g_cold = ctx->nn_group;
+  const int g_cold = with_chain ? 1 : ctx->nn_group;
   const int g_warm = ctx->warm_start ? 1 : g_cold;
   const bool per_launch = ctx->profile_level >= 2;
   const int launches = std::max(prm->max_iterations, 1);  // PCL runs the loop body at least once (do ... while)
@@ -1783,7 +2040,7 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   // nothing between the launches (profile level 2 and the debug timers put events there)
   // (not for a single align or a handful of hypotheses: hundreds of blocks polling one flag slow down the
   //  one thread everybody waits for — measured 0.74 -> 0.78 ms on C2)
-  const bool flag_deps = ctx->flag_deps && ctx->use_pdl && !per_launch && !ctx->debug_timers && !single_mode && H >= 16 &&
+  const bool flag_deps = !with_chain && ctx->flag_deps && ctx->use_pdl && !per_launch && !ctx->debug_timers && !single_mode && H >= 16 &&
                          launches < kEpochStopped;
   ctx->last_err_flag = nullptr;
   if (flag_deps) {
@@ -1817,8 +2074,9 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   const int search_bph_cold = blocks_for(n, H, 1, fs > 0 ? fs : cold_blocks_factor(ctx));
   const int search_bph_warm = blocks_for(n, H, 1, fs > 0 ? fs : ctx->blocks_factor);
   // the warm searches of a large enough batch run over the target's k-NN graph (built once per target)
-  if (ctx->warm_graph && ctx->warm_start && g_warm == 1 && !single_mode && !(L.margin > 0.0f) && !ctx->warm_upfront &&
-      !ctx->warm_bin && ctx->nn_cache_from == 0 && H >= static_cast<size_t>(ctx->warm_graph_min_hyp) && launches > 1) {
+  if (ctx->warm_graph && ctx->warm_start && g_warm == 1 && !single_mode &&
+      (with_chain || (!(L.margin > 0.0f) && !ctx->warm_upfront && !ctx->warm_bin && ctx->nn_cache_from == 0)) &&
+      H >= static_cast<size_t>(ctx->warm_graph_min_hyp) && launches > 1) {
     PEB_TRY(target_graph_ensure(ctx));
     Lw.knn = ctx->tgt_knn.as<KnnRow>();
     Lw.knn_stat = ctx->tgt_knn_stat.as<double>();
@@ -1831,7 +2089,7 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
     }
   }
   // the candidate cache of the warm launches from launch nn_cache_from on (0: never)
-  const int cache_from = (ctx->nn_cache_from > 0 && ctx->warm_start && g_warm == 1 && !(L.margin > 0.0f)) ? ctx->nn_cache_from : 0;
+  const int cache_from = (!with_chain && ctx->nn_cache_from > 0 && ctx->warm_start && g_warm == 1 && !(L.margin > 0.0f)) ? ctx->nn_cache_from : 0;
   NnCache* cache_buf = nullptr;
   if (cache_from > 0 && cache_from < launches) {
     PEB_CUDA(ctx, ctx->nn_cache.ensure(H * static_cast<size_t>(std::max(n, 1)) * sizeof(NnCache)));
@@ -1847,6 +2105,7 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
   //  launches of an align stay a prefix of its launches: a moment launch waits for the count of search launches before it.)
   bool split_prefix = true;
   auto split_bph = [&](int it) {
+    if (with_chain) return it == 0 ? search_bph_cold : search_bph_warm;
     split_prefix = split_prefix && split_iteration(ctx, it == 0 ? Lc : Lw, H, it == 0 ? g_cold : g_warm, it == 0);
     return split_prefix ? (it == 0 ? search_bph_cold : search_bph_warm) : 0;
   };
@@ -1898,6 +2157,12 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
       if (C.cache) C.cache += h0 * static_cast<size_t>(n);
       return C;
     };
+    auto rchunk_of = [&](size_t h0) {
+      RejChain C = R;
+      C.kept += h0 * static_cast<size_t>(n);
+      if (C.o2o) C.o2o += h0 * static_cast<size_t>(L.grid.n);
+      return C;
+    };
     // the anchor launch above ran on the main stream for all hypotheses: the fork event orders it
     for (int c = 0; c < S; ++c) PEB_CUDA(ctx, cudaStreamWaitEvent(ctx->sub_streams[c], ctx->fork_event, 0));
     for (int it = 0; it <= launches; ++it) {
@@ -1908,10 +2173,12 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
         const size_t h0 = c * per, h1 = std::min(H, h0 + per);
         if (h0 >= h1) continue;
         StreamSwap swap(ctx, ctx->sub_streams[c]);
+        const RejChain Rc = rchunk_of(h0);
+        const RejChain* rc = with_chain ? &Rc : nullptr;
         if (it == 0) {
-          PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, chunk_of(Lc, h0), h1 - h0, prm->estimator, sb));
+          PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, chunk_of(Lc, h0), h1 - h0, prm->estimator, sb, rc));
         } else if (it < launches) {
-          PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, chunk_of(Lw, h0), h1 - h0, prm->estimator, sb));
+          PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, chunk_of(Lw, h0), h1 - h0, prm->estimator, sb, rc));
         } else {
           // profile 1: the span ends with the last ITERATION launch of the slowest chain, as in the single-chain path
           // (peb_profile_read takes the maximum over the chains)
@@ -1922,6 +2189,7 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
       }
     }
     for (int c = 0; c < S; ++c) PEB_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->join_events[c], 0));
+    if (R.o2o) ctx->rej_o2o_clean = true;
     if (ctx->profile) {
       ctx->prof_launches = 1;  // one record: from the fork to the end of the last iteration launch of the slowest chain
       ctx->prof_span_launches = launches;
@@ -1936,14 +2204,16 @@ int icp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_i
     Lc.launch_idx = Lw.launch_idx = it;
     set_cache(it);
     const int sb = split_bph(it);
+    const RejChain* rc = with_chain ? &R : nullptr;
     if (it == 0)
-      PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, Lc, H, prm->estimator, sb));
+      PEB_TRY(launch_one_iteration_g(ctx, g_cold, true, Lc, H, prm->estimator, sb, rc));
     else
-      PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, Lw, H, prm->estimator, sb));
+      PEB_TRY(launch_one_iteration_g(ctx, g_warm, false, Lw, H, prm->estimator, sb, rc));
     if (per_launch) PEB_TRY(prof_mark(ctx, 2 * it + 1));
   }
   Lw.launch_idx = launches;  // the fitness launch needs all iteration launches of its hypothesis
   set_cache(launches);
+  if (R.o2o) ctx->rej_o2o_clean = true;
   if (per_launch) {
     PEB_TRY(prof_mark(ctx, 2 * launches));
     PEB_TRY(launch_fitness_g(ctx, g_warm, Lw, H));

@@ -257,6 +257,27 @@ PEB_API int peb_multi_icp_align_batch(peb_multi* m, const float* guesses, size_t
   });
 }
 
+}  // extern "C"
+
+namespace peb {
+
+int multi_run_sharded(peb_multi* m, const char* what, size_t n_items, int (*fn)(peb_ctx*, size_t lo, size_t hi, void* user),
+                      void* user) {
+  const int ndev = static_cast<int>(m->ctx.size());
+  return on_all_devices(m, what, [&](size_t i) {
+    size_t lo = 0, hi = 0;
+    peb_multi_shard_range(n_items, ndev, static_cast<int>(i), &lo, &hi);
+    if (hi == lo) return static_cast<int>(PEB_OK);  // more devices than items
+    return fn(m->ctx[i], lo, hi, user);
+  });
+}
+
+int multi_set_error(peb_multi* m, int code, const char* msg) { return multi_fail(m, code, msg); }
+
+}  // namespace peb
+
+extern "C" {
+
 PEB_API uint64_t peb_multi_launch_count(const peb_multi* m) {
   uint64_t total = 0;
   if (m)

@@ -219,8 +219,13 @@ class MultiContext:
         p = _cloud(pts)
         self.check(lib.peb_multi_source_set(self._h, p.ctypes.data, p.shape[0], _stride(p)))
 
-    def icp_align_batch(self, g16: np.ndarray, params: IcpParams, res):
-        self.check(lib.peb_multi_icp_align_batch(self._h, g16.ctypes.data, g16.shape[0], C.byref(params), res))
+    def icp_align_batch(self, g16: np.ndarray, params: IcpParams, res, chain=()):
+        """chain: correspondence rejectors (_lib.rejector_array), applied in order after rejector_max_dist."""
+        if chain:
+            arr, n = _lib.rejector_array(chain)
+            self.check(lib.peb_multi_icp_align_batch_ex(self._h, g16.ctypes.data, g16.shape[0], C.byref(params), arr, n, res))
+        else:
+            self.check(lib.peb_multi_icp_align_batch(self._h, g16.ctypes.data, g16.shape[0], C.byref(params), res))
 
 
 def default_context() -> Context:
@@ -573,6 +578,7 @@ class IterativeClosestPoint:
         self._have_target = False
         self._n_src = 0
         self.correspondences = None
+        self._chain: list[tuple] = []  # rejectors added after the first non-distance one, in PCL's order
 
     @property
     def _sctx(self) -> Context:
@@ -628,8 +634,35 @@ class IterativeClosestPoint:
             raise PebError(-6, "the RANSAC rejector has no CUDA path (no CPU fallback)")
 
     def addCorrespondenceRejectorDistance(self, max_distance: float):
-        """addCorrespondenceRejector(CorrespondenceRejectorDistance with setMaximumDistance(d))."""
-        self.params.rejector_max_dist = float(max_distance)
+        """addCorrespondenceRejector(CorrespondenceRejectorDistance with setMaximumDistance(d)).  Before any other
+        rejector it sets params.rejector_max_dist (the head of the chain); after one, it joins the chain in order."""
+        if self._chain:
+            self._add_rejector((_lib.REJECTOR_DISTANCE, float(max_distance)))
+        else:
+            self.params.rejector_max_dist = float(max_distance)
+
+    def addCorrespondenceRejectorMedianDistance(self, factor: float = 1.0):
+        """addCorrespondenceRejector(CorrespondenceRejectorMedianDistance with setMedianFactor(factor)): keeps the
+        pairs whose squared distance is at most factor x the median squared distance."""
+        self._add_rejector((_lib.REJECTOR_MEDIAN_DISTANCE, float(factor)))
+
+    def addCorrespondenceRejectorOneToOne(self):
+        """addCorrespondenceRejector(CorrespondenceRejectorOneToOne): the closest source per target point."""
+        self._add_rejector((_lib.REJECTOR_ONE_TO_ONE, 0.0))
+
+    def addCorrespondenceRejectorTrimmed(self, ratio: float = 0.5, min_correspondences: int = 0):
+        """addCorrespondenceRejector(CorrespondenceRejectorTrimmed with setOverlapRatio(ratio) and
+        setMinCorrespondences(min_correspondences)): the closest max(floor(ratio * m), min) pairs."""
+        self._add_rejector((_lib.REJECTOR_TRIMMED, float(ratio), int(min_correspondences)))
+
+    def getCorrespondenceRejectors(self) -> list[tuple]:
+        """The chain after params.rejector_max_dist: (kind, value[, min_correspondences]) in the order added."""
+        return list(self._chain)
+
+    def _add_rejector(self, r: tuple):
+        if len(self._chain) >= _lib.MAX_REJECTORS:
+            raise PebError(-1, f"at most {_lib.MAX_REJECTORS} correspondence rejectors after the distance one")
+        self._chain.append(r)
 
     def getConvergeCriteria(self) -> ConvergenceCriteria:
         return self._criteria
@@ -646,10 +679,15 @@ class IterativeClosestPoint:
         out = np.empty((n, 4), np.float32) if (want_output and n) else None
         idx = np.empty(n, np.int32) if (want_correspondences and n) else None
         d2 = np.empty(n, np.float32) if (want_correspondences and n) else None
-        self._sctx.check(lib.peb_icp_align(self._sctx.handle, g.ctypes.data if g is not None else None, C.byref(self.params),
-                                         C.byref(res), out.ctypes.data if out is not None else None,
-                                         idx.ctypes.data if idx is not None else None,
-                                         d2.ctypes.data if d2 is not None else None))
+        outs = (out.ctypes.data if out is not None else None, idx.ctypes.data if idx is not None else None,
+                d2.ctypes.data if d2 is not None else None)
+        if self._chain:
+            arr, nc = _lib.rejector_array(self._chain)
+            self._sctx.check(lib.peb_icp_align_ex(self._sctx.handle, g.ctypes.data if g is not None else None,
+                                                  C.byref(self.params), arr, nc, C.byref(res), *outs))
+        else:
+            self._sctx.check(lib.peb_icp_align(self._sctx.handle, g.ctypes.data if g is not None else None,
+                                               C.byref(self.params), C.byref(res), *outs))
         self._result = res
         self._criteria._state = res.state
         self.correspondences = (idx, d2) if want_correspondences else None
@@ -663,7 +701,10 @@ class IterativeClosestPoint:
         H = g.shape[0]
         res = (IcpResult * max(H, 1))()
         if getattr(self.ctx, "is_multi", False):
-            self.ctx.icp_align_batch(g, self.params, res)  # contiguous blocks of hypotheses per device
+            self.ctx.icp_align_batch(g, self.params, res, self._chain)  # contiguous blocks of hypotheses per device
+        elif self._chain:
+            arr, nc = _lib.rejector_array(self._chain)
+            self.ctx.check(lib.peb_icp_align_batch_ex(self.ctx.handle, g.ctypes.data, H, C.byref(self.params), arr, nc, res))
         else:
             self.ctx.check(lib.peb_icp_align_batch(self.ctx.handle, g.ctypes.data, H, C.byref(self.params), res))
         return list(res)[:H]
