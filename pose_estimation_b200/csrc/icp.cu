@@ -526,13 +526,13 @@ __device__ __forceinline__ void icp_query(const IcpLaunch& L, const int h, float
   if (keep && lane_in_group == 0) accumulate_pair<EST>(L.grid, p, best, acc);
 }
 
-// The search half of icp_query (move, search, store the working point) for one lane per query and no certificate: the
-// whole of a split iteration's search launch (icp_search_kernel).  A copy rather than a helper shared with icp_query, so
-// that the fused kernels keep their code generation.  p: the moved point; valid: the query's point was finite before.
-template <int UPF>
+// The search half of icp_query (move, search, store the working point) for one lane per query, no certificate and no
+// graph: a split iteration's search launch (icp_search_kernel) except where it searches over the graph.  A copy rather
+// than a helper shared with icp_query, so that the fused kernels keep their code generation.  p: the moved point; valid:
+// the query's point was finite before.
 __device__ __forceinline__ NnBest icp_search_query(const IcpLaunch& L, const int h, float4* __restrict__ work, const int i,
-                                                   const bool first, const bool apply, const bool graph, const float* T,
-                                                   CoopTile* tile, float4& p, bool& valid) {
+                                                   const bool first, const bool apply, const float* T, CoopTile* tile,
+                                                   float4& p, bool& valid) {
   const bool in = i < L.n_src;
   p = make_float4(0.f, 0.f, 0.f, 1.f);
   if (in) p = first ? L.src[i] : work[i];
@@ -553,13 +553,8 @@ __device__ __forceinline__ NnBest icp_search_query(const IcpLaunch& L, const int
     // (uniform branch: every lane of the warp takes part, valid or not)
     best = first_iteration_search(L, h, i, valid, p, T, apply, tile);
   } else if (valid) {
-    if (L.warm && j_prev >= 0 && j_prev < L.grid.n) {
-      if (UPF == 4 || UPF == 6) best = graph ? grid_nn_warm_graph(L.grid, L.knn, p.x, p.y, p.z, j_prev, L.stop_d2, kGraphSkipHopeless, L.launch_idx <= L.knn_peek_until, UPF == 6 ? L.knn_aux : nullptr)
-                                 : grid_nn_warm(L.grid, p.x, p.y, p.z, j_prev, L.stop_d2);
-      else best = grid_nn_warm(L.grid, p.x, p.y, p.z, j_prev, L.stop_d2);
-    } else {
-      best = grid_nn<1>(L.grid, p.x, p.y, p.z, L.stop_d2);
-    }
+    if (L.warm && j_prev >= 0 && j_prev < L.grid.n) best = grid_nn_warm(L.grid, p.x, p.y, p.z, j_prev, L.stop_d2);
+    else best = grid_nn<1>(L.grid, p.x, p.y, p.z, L.stop_d2);
   }
   if (in && (first || valid)) {
     p.w = __int_as_float(best.j);
@@ -714,8 +709,9 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_iteration_kernel(const Ic
 // In icp_iteration_kernel the double moment sums (17 for SVD, 28 for LLS), the block reduction and the out-of-line
 // solve share the allocation of the search loop: the batched kernels spill at their 64-register cap, and their late
 // launches, bound by the L2 latency of the searches, run with about 25 resident warps per SM.  Split:
-//   icp_search_kernel  grid = (search blocks per hypothesis, H): the fused kernel's search half (icp_search_query)
-//                      and nothing else — no double state, no reduction, no solve — under its own register cap (kMinBlocksSearch): more
+//   icp_search_kernel  grid = (search blocks per hypothesis, H): the fused kernel's search half (icp_search_query;
+//                      over the k-NN graph icp_search_graph_queued, which walks the grid in dense warps) and nothing
+//                      else — no double state, no reduction, no solve — under its own register cap (kMinBlocksSearch): more
 //                      resident warps to hide the search's latency.  Its block count is free: it writes no records.
 //   icp_moment_kernel  grid = (blocks_per_hyp, H): per query the working point and its match are read back and d2 is
 //                      recomputed as every search path computes it (l2_simple of the query and the match); threshold,
@@ -734,6 +730,95 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_iteration_kernel(const Ic
 // of a stopped one do (its epoch releases them all), and they take no ticket.  Every block still waits only for blocks of
 // earlier launches (see icp_iteration_kernel).  Without flags both launches wait for the whole previous grid.
 // The search stride is gridDim.x: its blocks per hypothesis are free (it writes no records).
+
+// .w of a searched valid query: its match, or -2 - match for a point this launch's transform made non-finite
+__device__ __forceinline__ int search_slot(float x, float y, float z, int j) {
+  return (j >= 0 && !finite3(x, y, z)) ? -2 - j : j;
+}
+
+// A query the graph could not prove, waiting in its warp's queue: the moved point, the sorted position of the best point
+// the graph met (-1: no previous match, a cold search) and the query's index.  20 bytes: lanes reading consecutive
+// entries hit 32 different banks.
+struct SearchQueued {
+  float x, y, z;
+  int cand;
+  int i;
+};
+constexpr int kSearchQueue = 64;  // per warp: at most 31 waiting + one pass of 32
+
+// The search launch of a hypothesis that searches over the graph (graph_pays).  In a late launch the row of the previous
+// match proves nearly every query, but the ~6 % it cannot prove walk the grid (grid_ball_search: per-lane loops, 8
+// dependent load levels) while the rest of their warp idles.  Here every lane moves its query and tries the graph
+// (grid_nn_graph_try); a proven query stores its working point at once, an unproven one goes to the warp's queue with
+// everything its walk needs, and whenever 32 are waiting (and once at the end) the warp walks them one per lane.  No block
+// barrier: the warps of a block queue and drain on their own.  The walk is exact for any candidate, and the candidate is
+// rebuilt from its position with the expression the graph computed it with, so every match is the per-lane search's and
+// every working point is written once, with the same bytes.
+template <int UPF>
+__device__ __forceinline__ void icp_search_graph_queued(const IcpLaunch& L, float4* __restrict__ work, const bool apply,
+                                                        const float* T) {
+  __shared__ SearchQueued s_queue[kIcpThreads / 32][kSearchQueue];
+  SearchQueued* queue = s_queue[threadIdx.x >> 5];
+  const int lane = threadIdx.x & 31;
+  const bool peek = L.launch_idx <= L.knn_peek_until;
+  int n_queue = 0;  // (warp-uniform)
+  // lanes [0, count) walk the grid for the LAST count entries of the queue
+  auto drain = [&](int count) {
+    if (lane < count) {
+      const SearchQueued e = queue[n_queue - count + lane];
+      NnBest best;
+      if (e.cand >= 0) {
+        const float4 t = L.grid.pts[e.cand];
+        best.d2 = l2_simple(e.x, e.y, e.z, t.x, t.y, t.z);
+        best.idx = point_index(t);
+        best.j = e.cand;
+        grid_ball_search(L.grid, e.x, e.y, e.z, L.stop_d2, best);
+      } else {
+        best = grid_nn<1>(L.grid, e.x, e.y, e.z, L.stop_d2);
+      }
+      work[e.i] = make_float4(e.x, e.y, e.z, __int_as_float(search_slot(e.x, e.y, e.z, best.j)));
+    }
+    n_queue -= count;
+    __syncwarp();
+  };
+  for (int base = blockIdx.x * kIcpThreads; base < L.n_src; base += gridDim.x * kIcpThreads) {
+    const int i = base + threadIdx.x;
+    const bool in = i < L.n_src;
+    float4 p = make_float4(0.f, 0.f, 0.f, 1.f);
+    if (in) p = work[i];
+    const int j_prev = __float_as_int(p.w);  // last iteration's match (sorted position)
+    bool need = false;
+    int cand = -1;
+    if (in && finite3(p.x, p.y, p.z)) {
+      if (apply) {
+        float ox, oy, oz;
+        transform_icp(T, p.x, p.y, p.z, ox, oy, oz);
+        p.x = ox;
+        p.y = oy;
+        p.z = oz;
+      }
+      need = true;
+      if (L.warm && j_prev >= 0 && j_prev < L.grid.n) {
+        NnBest best;
+        need = !grid_nn_graph_try(L.grid, L.knn, p.x, p.y, p.z, j_prev, best, kGraphSkipHopeless, peek,
+                                  UPF == 6 ? L.knn_aux : nullptr);
+        if (need) cand = best.j;
+        else work[i] = make_float4(p.x, p.y, p.z, __int_as_float(search_slot(p.x, p.y, p.z, best.j)));
+      }
+    } else if (in && j_prev <= -2) {
+      reinterpret_cast<int*>(work + i)[3] = -1;  // invalid before this launch: no match to carry (see above)
+    }
+    const unsigned m = __ballot_sync(0xFFFFFFFFu, need);
+    if (m) {
+      if (need) queue[n_queue + __popc(m & ((1u << lane) - 1u))] = SearchQueued{p.x, p.y, p.z, cand, i};
+      n_queue += __popc(m);
+      __syncwarp();
+      if (n_queue >= 32) drain(32);
+    }
+  }
+  if (n_queue) drain(n_queue);
+}
+
 template <int MB, bool FIRST, int UPF>
 __global__ void __launch_bounds__(kIcpThreads, MB) icp_search_kernel(const IcpLaunch L) {
   if (FIRST || L.epochs == nullptr) {
@@ -753,11 +838,12 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_search_kernel(const IcpLa
     const bool apply = s_flags[2] != 0;
     const bool graph = (UPF == 4 || UPF == 6) && s_flags[3] != 0;
     float4* work = L.work + static_cast<size_t>(h) * L.n_src;
-    for (int base = blk * kIcpThreads; base < L.n_src; base += gridDim.x * kIcpThreads) {
+    if (!FIRST && graph) icp_search_graph_queued<UPF>(L, work, apply, s_inc);
+    else for (int base = blk * kIcpThreads; base < L.n_src; base += gridDim.x * kIcpThreads) {
       const int i = base + threadIdx.x;
       float4 p;
       bool valid;
-      const NnBest best = icp_search_query<UPF>(L, h, work, i, FIRST, apply, graph, s_inc, &s_tile[threadIdx.x >> 5], p, valid);
+      const NnBest best = icp_search_query(L, h, work, i, FIRST, apply, s_inc, &s_tile[threadIdx.x >> 5], p, valid);
       int* w = reinterpret_cast<int*>(work + i) + 3;
       if (valid && best.j >= 0 && !finite3(p.x, p.y, p.z)) *w = -2 - best.j;
       else if (!FIRST && !valid && i < L.n_src && __float_as_int(p.w) <= -2) *w = -1;
