@@ -314,6 +314,28 @@ PEB_API int peb_normals_knn(peb_ctx* ctx, const void* pts, size_t n, size_t stri
 PEB_API int peb_normals_knn_ex(peb_ctx* ctx, const void* pts, size_t n, size_t stride, int k,
                                const float viewpoint[3], float* out_normal8, int32_t* out_nn_idx);
 
+/* ---- cv::ppf_match_3d::computeNormalsPC3d(pc, out, k, flip, viewpoint) ------------------------------------------
+ * What the reference runs in the normals slot (pose_estimation/src/opencv_surface_match.cpp:57-59:
+ * computeNormalsPC3d(pc_scene, pc_scene_normals, 20, true, (0, 0, 0))).  [CV] opencv_contrib/modules/surface_matching/
+ * src/ppf_helpers.cpp (restated from recollection, DESIGN.md section 13); the eigen solver is pinned bit for bit
+ * against cv2.eigen of an OpenCV built without Eigen.
+ *   neighbours  the k nearest points (the point itself included), ascending squared float distance: the exact
+ *               search of KDTreeSingleIndexParams(8); equidistant neighbours may come in another order than FLANN's
+ *   covariance  in list order: C(j,l) += (double)(float)(p_j * p_l), mu_j += p_j; then mu *= 1.0 / k, C *= 1.0 / k,
+ *               C(j,l) -= mu_j mu_l, all double (meanCovLocalPCInd)
+ *   normal      cv::eigen(C) = JacobiImpl_<double> (eigenvalues descending, eigenvectors as rows); row 2 rounded to float
+ *   flip        flip_viewpoint != 0: d = viewpoint - p (float), cos = d0 n0 + d1 n1 + d2 n2 (float, left to right);
+ *               cos < 0 negates n (flipNormalViewpoint)
+ * out_xyzn6: n rows of 6 floats x y z nx ny nz (a CV_32F PCNormals Mat, e.g. pc_scene_normals.ptr<float>(0)); x y z
+ * are copied from the input.  out_nn_idx (nullable): n x k original indices, -1 on rows of non-finite points.
+ * Where the reference is undefined, this library defines:
+ *   - a non-finite point is neither a query nor a neighbour; its row gets its x y z and a NaN normal;
+ *   - k < 1, or k greater than the number of finite points (FLANN would leave indices unfilled and OpenCV would read
+ *     row -1), is PEB_E_INVALID_ARG; k > 192 is PEB_E_UNSUPPORTED (the bound of peb_normals_knn); n == 0 is PEB_OK
+ *     for any valid k and writes nothing. */
+PEB_API int peb_cv_normals(peb_ctx* ctx, const void* pts, size_t n, size_t stride, int k, int flip_viewpoint,
+                           const float viewpoint[3], float* out_xyzn6, int32_t* out_nn_idx);
+
 /* ---- pcl::KdTreeFLANN::nearestKSearch over the resident target (k = 1) ------------ */
 /* out_idx: original target index (-1 if the target is empty), out_d2: squared distance. */
 PEB_API int peb_nn_search(peb_ctx* ctx, const void* queries, size_t nq, size_t stride,
@@ -451,6 +473,9 @@ PEB_API int peb_voxel_grid_dev(peb_ctx* ctx, const void* d_xyz4, size_t n, float
                                float leaf_z, unsigned min_pts, void* d_out_xyz4, size_t* out_n);
 PEB_API int peb_normals_knn_dev(peb_ctx* ctx, const void* d_xyz4, size_t n, int k,
                                 const float viewpoint[3], void* d_out_normal8);
+/* peb_cv_normals on the device: d_out_xyzn6 holds n x 6 floats (4-byte alignment suffices) */
+PEB_API int peb_cv_normals_dev(peb_ctx* ctx, const void* d_xyz4, size_t n, int k, int flip_viewpoint,
+                               const float viewpoint[3], void* d_out_xyzn6);
 /* waits for everything queued on the context.  PEB_E_CUDA if the last batched align raised its internal-error flag
  * (PEB_STATE_INTERNAL_ERROR): the asynchronous peb_icp_align_batch_dev cannot report it when it returns, and a
  * record written before another hypothesis hit the bound does not carry it. */

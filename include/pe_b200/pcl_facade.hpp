@@ -209,6 +209,15 @@ class NormalEstimation {
   float vp_[3] = {0, 0, 0};
 };
 
+// cv::ppf_match_3d::computeNormalsPC3d(pc, pc_normals, num_neighbors, flip_viewpoint, viewpoint) — the reference's
+// normals slot (pose_estimation/src/opencv_surface_match.cpp:57-59) with OpenCV's arithmetic (peb_cv_normals).
+// pc: rows of `stride` bytes whose first three floats are x y z (a CV_32F N x 3 or N x 6 Mat: ptr<float>(0), step);
+// out6: rows x 6 floats x y z nx ny nz, e.g. pc_normals.ptr<float>(0) of a continuous CV_32F rows x 6 Mat.
+inline void computeNormalsPC3d(Context& c, const float* pc, size_t rows, size_t stride, int num_neighbors, bool flip_viewpoint,
+                               const float viewpoint[3], float* out6) {
+  c.check(peb_cv_normals(c.get(), pc, rows, stride, num_neighbors, flip_viewpoint ? 1 : 0, viewpoint, out6, nullptr));
+}
+
 // pcl::registration::DefaultConvergenceCriteria<float>, the part reachable through getConvergeCriteria()
 class ConvergenceCriteria {
  public:

@@ -188,6 +188,7 @@ SYMBOLS = {
     "peb_ppf_match": (_i, [_vp, _vp, _vp, _sz, _d, _d, _vp, _sz, _pp(_sz), _vp, _sz, _pp(_sz)]),
     "peb_normals_knn": (_i, [_vp, _vp, _sz, _sz, _i, _vp, _vp]),
     "peb_normals_knn_ex": (_i, [_vp, _vp, _sz, _sz, _i, _vp, _vp, _vp]),
+    "peb_cv_normals": (_i, [_vp, _vp, _sz, _sz, _i, _i, _vp, _vp, _vp]),
     "peb_nn_search": (_i, [_vp, _vp, _sz, _sz, _vp, _vp]),
     "peb_nn_search_bruteforce": (_i, [_vp, _vp, _sz, _sz, _vp, _vp]),
     "peb_target_set": (_i, [_vp, _vp, _sz, _sz, _vp, _sz]),
@@ -210,6 +211,7 @@ SYMBOLS = {
     "peb_icp_align_batch_dev": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp]),
     "peb_voxel_grid_dev": (_i, [_vp, _vp, _sz, _f, _f, _f, C.c_uint, _vp, _pp(_sz)]),
     "peb_normals_knn_dev": (_i, [_vp, _vp, _sz, _i, _vp, _vp]),
+    "peb_cv_normals_dev": (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp]),
     "peb_sync": (_i, [_vp]),
     "peb_target_grid_info": (_i, [_vp, _pp(GridInfo)]),
     "peb_icp_trace": (_i, [_vp, _vp, _sz, _pp(_sz)]),

@@ -603,6 +603,45 @@ PEB_API int peb_normals_knn(peb_ctx* ctx, const void* pts, size_t n, size_t stri
   return peb_normals_knn_ex(ctx, pts, n, stride, k, viewpoint, out_normal8, nullptr);
 }
 
+// ---- cv::ppf_match_3d::computeNormalsPC3d -------------------------------------------------------
+PEB_API int peb_cv_normals_dev(peb_ctx* ctx, const void* d_xyz4, size_t n, int k, int flip_viewpoint, const float viewpoint[3],
+                               void* d_out_xyzn6) {
+  if (!ctx) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  if (n > 0 && (!d_xyz4 || !d_out_xyzn6)) return fail(ctx, PEB_E_INVALID_ARG, "cv_normals_dev: null device pointer");
+  if (n > static_cast<size_t>(INT32_MAX) / 2) return fail(ctx, PEB_E_INVALID_ARG, "cv_normals: too many points");
+  const float zero[3] = {0.f, 0.f, 0.f};
+  return cv_normals_device(ctx, static_cast<const float4*>(d_xyz4), static_cast<int>(n), k, flip_viewpoint != 0,
+                           viewpoint ? viewpoint : zero, static_cast<float*>(d_out_xyzn6), nullptr);
+}
+
+PEB_API int peb_cv_normals(peb_ctx* ctx, const void* pts, size_t n, size_t stride, int k, int flip_viewpoint,
+                           const float viewpoint[3], float* out_xyzn6, int32_t* out_nn_idx) {
+  if (!ctx) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  PEB_TRY(check_cloud(ctx, "cv_normals", pts, n, stride));
+  if (n > 0 && !out_xyzn6) return fail(ctx, PEB_E_INVALID_ARG, "cv_normals: null output");
+  if (k < 1) return fail(ctx, PEB_E_INVALID_ARG, "cv_normals: k must be >= 1 (got %d)", k);
+  if (k > 192) return fail(ctx, PEB_E_UNSUPPORTED, "cv_normals: k = %d > 192 has no CUDA path (no CPU fallback)", k);
+  if (n == 0) return PEB_OK;
+  const float zero[3] = {0.f, 0.f, 0.f};
+  PEB_CUDA(ctx, ctx->nrm_in.ensure(n * sizeof(float4)));
+  PEB_CUDA(ctx, ctx->nrm_out.ensure(n * 6 * sizeof(float)));
+  int32_t* d_nn = nullptr;
+  if (out_nn_idx) {
+    PEB_CUDA(ctx, ctx->nn_idx.ensure(n * static_cast<size_t>(k) * sizeof(int32_t)));
+    d_nn = ctx->nn_idx.as<int32_t>();
+  }
+  PEB_TRY(upload_cloud(ctx, pts, n, stride, 1.0f, ctx->nrm_in.as<float4>()));
+  PEB_TRY(cv_normals_device(ctx, ctx->nrm_in.as<float4>(), static_cast<int>(n), k, flip_viewpoint != 0,
+                            viewpoint ? viewpoint : zero, ctx->nrm_out.as<float>(), d_nn));
+  PEB_CUDA(ctx, cudaMemcpyAsync(out_xyzn6, ctx->nrm_out.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  if (out_nn_idx)
+    PEB_CUDA(ctx, cudaMemcpyAsync(out_nn_idx, d_nn, n * static_cast<size_t>(k) * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                  ctx->stream));
+  return sync(ctx);
+}
+
 // ---- target / source -----------------------------------------------------------------------------
 PEB_API int peb_target_stage(peb_ctx* ctx, const void* pts, size_t n, size_t stride, const void* normals, size_t nstride) {
   if (!ctx) return PEB_E_INVALID_ARG;

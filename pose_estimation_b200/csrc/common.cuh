@@ -305,5 +305,8 @@ int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, co
 int target_graph_ensure(peb_ctx* ctx);  // builds ctx->tgt_knn for the current target grid if it is not there yet
 int normals_knn_device(peb_ctx* ctx, const float4* d_in, int n, int k, const float vp[3], float* d_out8,
                        int32_t* d_out_nn /*nullable, n x k original indices*/);
+// cv::ppf_match_3d::computeNormalsPC3d: d_out6 = n rows of x y z nx ny nz (DESIGN.md §13)
+int cv_normals_device(peb_ctx* ctx, const float4* d_in, int n, int k, bool flip, const float vp[3], float* d_out6,
+                      int32_t* d_out_nn /*nullable, n x k original indices*/);
 
 }  // namespace peb

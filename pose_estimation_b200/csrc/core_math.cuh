@@ -950,4 +950,178 @@ PEB_HD void normal_from_accu(float* accu, int cnt, float px, float py, float pz,
   out8[5] = out8[6] = out8[7] = 0.0f;
 }
 
+// ---- cv::ppf_match_3d::computeNormalsPC3d (DESIGN.md §13) -----------------------------------
+// [CV] core/src/lapack.cpp : hypot<double> — mul, div and sqrt only, so -fmad=false / -ffp-contract=off make the
+// device and the host round every step alike
+PEB_HD double cv_hypot(double a, double b) {
+  a = fabs(a);
+  b = fabs(b);
+  if (a > b) {
+    b /= a;
+    return a * sqrt(1 + b * b);
+  }
+  if (b > 0) {
+    a /= b;
+    return b * sqrt(1 + a * a);
+  }
+  return 0;
+}
+
+// JacobiImpl_'s rotate(v0, v1)
+PEB_HD void cv_rotate(double& v0, double& v1, double c, double s) {
+  const double a0 = v0, b0 = v1;
+  v0 = a0 * c - b0 * s;
+  v1 = a0 * s + b0 * c;
+}
+
+template <int K, int L>
+PEB_HD void cv_rotate_rows(double (&V)[9], double c, double s) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) cv_rotate(V[K * 3 + i], V[L * 3 + i], c, s);
+}
+
+template <int K, int M>
+PEB_HD void cv_swap_rows(double (&W)[3], double (&V)[9]) {
+  const double tw = W[K];
+  W[K] = W[M];
+  W[M] = tw;
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const double tv = V[K * 3 + i];
+    V[K * 3 + i] = V[M * 3 + i];
+    V[M * 3 + i] = tv;
+  }
+}
+
+// cv::eigen(A, W, V) for a symmetric 3 x 3 double matrix in an OpenCV built without Eigen: [CV] core/src/lapack.cpp :
+// JacobiImpl_<double> with n = 3 (cyclic-by-largest Jacobi, at most n * n * 30 rotations, eps = DBL_EPSILON).
+// A is row-major; only its upper triangle is read.  W: eigenvalues, descending; V: eigenvectors as ROWS.
+// The three off-diagonal entries and the two pivot indices that vary for n = 3 (indR[0], indC[2]; indR[1] = 2 and
+// indC[1] = 0 always) are scalars, so the solver lives in registers.  Like upstream, a pivot index is recomputed only
+// for the row / column a rotation touches: a stale indR[0] after a (1, 2) rotation is part of the pivot sequence.
+PEB_HD void cv_eigen_sym3(const double (&A)[9], double (&W)[3], double (&V)[9]) {
+  const double eps = DBL_EPSILON;
+  double a01 = A[1], a02 = A[2], a12 = A[5];
+  W[0] = A[0];
+  W[1] = A[4];
+  W[2] = A[8];
+#pragma unroll
+  for (int i = 0; i < 9; ++i) V[i] = (i % 4 == 0) ? 1.0 : 0.0;
+  int r0 = fabs(a01) < fabs(a02) ? 2 : 1;  // indR[0]: argmax over m > 0 of |A[0][m]|, first maximum wins
+  int c2 = fabs(a02) < fabs(a12) ? 1 : 0;  // indC[2]: argmax over m < 2 of |A[m][2]|
+  for (int iters = 0; iters < 3 * 3 * 30; ++iters) {
+    // pivot (k, l): rows by indR first, then columns by indC, strict < so the first maximum wins
+    int k = 0, l;
+    double mv = fabs(r0 == 1 ? a01 : a02);
+    if (mv < fabs(a12)) {
+      mv = fabs(a12);
+      k = 1;
+    }
+    l = k == 0 ? r0 : 2;
+    if (mv < fabs(a01)) {
+      mv = fabs(a01);
+      k = 0;
+      l = 1;
+    }
+    const double a_c2 = c2 == 0 ? a02 : a12;
+    if (mv < fabs(a_c2)) {
+      k = c2;
+      l = 2;
+    }
+    const double p = k == 1 ? a12 : (l == 1 ? a01 : a02);
+    if (fabs(p) <= eps) break;
+    const double wk = k == 0 ? W[0] : W[1];
+    const double wl = l == 1 ? W[1] : W[2];
+    const double y = (wl - wk) * 0.5;
+    double t = fabs(y) + cv_hypot(p, y);
+    double s = cv_hypot(p, t);
+    const double c = t / s;
+    s = p / s;
+    t = (p / t) * p;
+    if (y < 0) {
+      s = -s;
+      t = -t;
+    }
+    if (k == 0 && l == 1) {
+      a01 = 0;
+      W[0] -= t;
+      W[1] += t;
+      cv_rotate(a02, a12, c, s);  // i > l: (A[k][i], A[l][i])
+      cv_rotate_rows<0, 1>(V, c, s);
+      r0 = fabs(a01) < fabs(a02) ? 2 : 1;
+    } else if (k == 0) {  // (0, 2)
+      a02 = 0;
+      W[0] -= t;
+      W[2] += t;
+      cv_rotate(a01, a12, c, s);  // k < i < l: (A[k][i], A[i][l])
+      cv_rotate_rows<0, 2>(V, c, s);
+      r0 = fabs(a01) < fabs(a02) ? 2 : 1;
+      c2 = fabs(a02) < fabs(a12) ? 1 : 0;
+    } else {  // (1, 2)
+      a12 = 0;
+      W[1] -= t;
+      W[2] += t;
+      cv_rotate(a01, a02, c, s);  // i < k: (A[i][k], A[i][l])
+      cv_rotate_rows<1, 2>(V, c, s);
+      c2 = fabs(a02) < fabs(a12) ? 1 : 0;
+    }
+  }
+  // selection sort, descending (first maximum wins), rows of V move with W
+  {
+    int m = 0;
+    if (W[0] < W[1]) m = 1;
+    if (W[m] < W[2]) m = 2;
+    if (m == 1) cv_swap_rows<0, 1>(W, V);
+    else if (m == 2) cv_swap_rows<0, 2>(W, V);
+    if (W[1] < W[2]) cv_swap_rows<1, 2>(W, V);
+  }
+}
+
+// [CV] surface_matching/src/ppf_helpers.cpp : meanCovLocalPCInd, one neighbour.  acc = the six distinct products
+// (xx xy xz yy yz zz) and the three coordinates, double; every product is formed in float, then widened.  The matrix is
+// symmetric bit for bit (a float product commutes), so the six sums stand for upstream's nine.
+PEB_HD void cv_moments_add(double (&acc)[9], float x, float y, float z) {
+  acc[0] += static_cast<double>(x * x);
+  acc[1] += static_cast<double>(x * y);
+  acc[2] += static_cast<double>(x * z);
+  acc[3] += static_cast<double>(y * y);
+  acc[4] += static_cast<double>(y * z);
+  acc[5] += static_cast<double>(z * z);
+  acc[6] += static_cast<double>(x);
+  acc[7] += static_cast<double>(y);
+  acc[8] += static_cast<double>(z);
+}
+
+// meanCovLocalPCInd's tail (mean and covariance scaled by the reciprocal 1.0 / k, then C -= mu mu^T), cv::eigen, row 2
+// of the eigenvectors rounded to float and — flip — flipNormalViewpoint: d = vp - p and d . n in float, left to right.
+PEB_HD void cv_normal_from_moments(const double (&acc)[9], int k, float px, float py, float pz, bool flip, float vx, float vy,
+                                   float vz, float (&n)[3]) {
+  const double inv = 1.0 / k;
+  const double mu[3] = {acc[6] * inv, acc[7] * inv, acc[8] * inv};
+  double C[9];
+  C[0] = acc[0] * inv - mu[0] * mu[0];
+  C[1] = acc[1] * inv - mu[0] * mu[1];
+  C[2] = acc[2] * inv - mu[0] * mu[2];
+  C[4] = acc[3] * inv - mu[1] * mu[1];
+  C[5] = acc[4] * inv - mu[1] * mu[2];
+  C[8] = acc[5] * inv - mu[2] * mu[2];
+  C[3] = C[1];
+  C[6] = C[2];
+  C[7] = C[5];
+  double W[3], V[9];
+  cv_eigen_sym3(C, W, V);
+  n[0] = static_cast<float>(V[6]);
+  n[1] = static_cast<float>(V[7]);
+  n[2] = static_cast<float>(V[8]);
+  if (flip) {
+    const float dx = vx - px, dy = vy - py, dz = vz - pz;
+    const float cos_theta = dx * n[0] + dy * n[1] + dz * n[2];
+    if (cos_theta < 0) {
+      n[0] *= -1;
+      n[1] *= -1;
+      n[2] *= -1;
+    }
+  }
+}
+
 }  // namespace peb

@@ -18,6 +18,10 @@
 // k > 32, or leftovers (normals_knn_kernel): one thread per query; its candidate list lives in shared memory, column
 // per thread, kept sorted by insertion, rings until the bound proves the list.
 // Algorithmic HBM bytes: N * (16 read + 16 k gather + 32 write).
+//
+// cv::ppf_match_3d::computeNormalsPC3d (cv_normals_*; DESIGN.md §13) runs the same grid and the same two searches and
+// only swaps the tail: float products summed in double in list order, OpenCV's Jacobi eigen solver in double
+// (core_math.cuh : cv_eigen_sym3), the last eigenvector rounded to float and the float viewpoint flip.
 #include <algorithm>
 
 #include "nn_graph.cuh"
@@ -99,24 +103,10 @@ __global__ void normals_fill_nan_kernel(float* __restrict__ out8, int n) {
   o[1] = make_float4(qnan, 0.0f, 0.0f, 0.0f);
 }
 
-// list == nullptr: every sorted point is a query; else the queries are list[0 .. *list_n)
-__global__ void normals_knn_kernel(const GridView g, int k, float vx, float vy, float vz, float* __restrict__ out8,
-                                   int32_t* __restrict__ out_nn, const int* __restrict__ list,
-                                   const int* __restrict__ list_n) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int T = blockDim.x;
-  unsigned long long* se = reinterpret_cast<unsigned long long*>(smem_raw);
-  int q = blockIdx.x * T + threadIdx.x;
-  if (list) {
-    if (q >= *list_n) return;
-    q = list[q];
-  }
-  if (q >= g.n) return;
-  const float4 p = g.pts[q];
-  const int orig = __float_as_int(p.w);
-  KnnList l;
+// the min(k, g.n) nearest points of p into this thread's column of the shared-memory list, ascending (distance, position)
+__device__ __forceinline__ void knn_list_search(const GridView& g, const float4& p, int k, unsigned long long* se, KnnList& l) {
   l.e = se + threadIdx.x;
-  l.stride = T;
+  l.stride = blockDim.x;
   l.k = min(k, g.n);
   l.count = 0;
   l.worst = ~0ull;
@@ -133,6 +123,25 @@ __global__ void normals_knn_kernel(const GridView g, int k, float vx, float vy, 
     ++r;
     full = false;
   }
+}
+
+// list == nullptr: every sorted point is a query; else the queries are list[0 .. *list_n)
+__global__ void normals_knn_kernel(const GridView g, int k, float vx, float vy, float vz, float* __restrict__ out8,
+                                   int32_t* __restrict__ out_nn, const int* __restrict__ list,
+                                   const int* __restrict__ list_n) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int T = blockDim.x;
+  unsigned long long* se = reinterpret_cast<unsigned long long*>(smem_raw);
+  int q = blockIdx.x * T + threadIdx.x;
+  if (list) {
+    if (q >= *list_n) return;
+    q = list[q];
+  }
+  if (q >= g.n) return;
+  const float4 p = g.pts[q];
+  const int orig = __float_as_int(p.w);
+  KnnList l;
+  knn_list_search(g, p, k, se, l);
   float* o = out8 + 8 * static_cast<size_t>(orig);
   if (out_nn) {
     for (int i = 0; i < k; ++i)
@@ -302,6 +311,86 @@ int launch_reglist(peb_ctx* ctx, const GridView& g, int k, const float vp[3], fl
   return PEB_OK;
 }
 
+// ---- cv::ppf_match_3d::computeNormalsPC3d (DESIGN.md §13): the same k-NN, OpenCV's tail -----------------------------
+// Every row gets the input's xyz; a non-finite point (not in the grid) also gets a NaN normal.  The normal kernels
+// below then write the normals of the finite points.
+__global__ void __launch_bounds__(256) cv_normals_fill_kernel(const float4* __restrict__ in, int n, float* __restrict__ out6) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float4 p = in[i];
+  float* o = out6 + 6 * static_cast<size_t>(i);
+  o[0] = p.x;
+  o[1] = p.y;
+  o[2] = p.z;
+  if (!finite3(p.x, p.y, p.z)) {
+    const float qnan = __int_as_float(0x7fc00000);
+    o[3] = o[4] = o[5] = qnan;
+  }
+}
+
+struct CvNormalArgs {
+  int k;      // neighbours; the launcher guarantees 1 <= k <= g.n
+  int flip;   // flipNormalViewpoint
+  float vx, vy, vz;
+  float* out6;      // rows of x y z nx ny nz, by original index
+  int32_t* out_nn;  // nullable, n x k original indices
+};
+
+__device__ __forceinline__ void cv_normal_store(const CvNormalArgs& a, const float4& p, int orig, const double (&acc)[9]) {
+  float nrm[3];
+  cv_normal_from_moments(acc, a.k, p.x, p.y, p.z, a.flip != 0, a.vx, a.vy, a.vz, nrm);
+  float* o = a.out6 + 6 * static_cast<size_t>(orig);
+  o[3] = nrm[0];
+  o[4] = nrm[1];
+  o[5] = nrm[2];
+}
+
+// k <= K <= 32: the register list of normals_reglist_kernel; the k neighbours are slots K - k .. K - 1, in list order
+template <int K>
+__global__ void __launch_bounds__(128, 4) cv_normals_reglist_kernel(const GridView g, const CvNormalArgs a) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= g.n) return;
+  const float4 p = g.pts[q];
+  const int orig = __float_as_int(p.w);
+  RegList<K> l;
+  reglist_knn<K>(g, p, a.k, l);
+  double acc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+  for (int s = 0; s < K; ++s) {
+    if (l.j[s] >= 0) {
+      const float4 c = g.pts[l.j[s]];
+      if (a.out_nn) a.out_nn[static_cast<size_t>(orig) * a.k + (s - (K - a.k))] = __float_as_int(c.w);
+      cv_moments_add(acc, c.x, c.y, c.z);
+    }
+  }
+  cv_normal_store(a, p, orig, acc);
+}
+
+// k > 32: the shared-memory list of normals_knn_kernel
+__global__ void cv_normals_knn_kernel(const GridView g, const CvNormalArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int T = blockDim.x;
+  const int q = blockIdx.x * T + threadIdx.x;
+  if (q >= g.n) return;
+  const float4 p = g.pts[q];
+  const int orig = __float_as_int(p.w);
+  KnnList l;
+  knn_list_search(g, p, a.k, reinterpret_cast<unsigned long long*>(smem_raw), l);
+  double acc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  for (int i = 0; i < l.count; ++i) {
+    const float4 c = g.pts[knn_key_pos(l.e[i * T])];
+    if (a.out_nn) a.out_nn[static_cast<size_t>(orig) * a.k + i] = __float_as_int(c.w);
+    cv_moments_add(acc, c.x, c.y, c.z);
+  }
+  cv_normal_store(a, p, orig, acc);
+}
+
+template <int K>
+int launch_cv_reglist(peb_ctx* ctx, const GridView& g, const CvNormalArgs& a) {
+  PEB_LAUNCH(ctx, cv_normals_reglist_kernel<K>, ceil_div(g.n, 128), 128, 0, g, a);
+  return PEB_OK;
+}
+
 // The k-nearest-neighbour graph of a grid's own points (nn_graph.cuh): row(q) = the kGraphK nearest OTHER points of
 // sorted position q, ascending (distance, position), in half rows of 12 with the distances from q to the neighbour
 // behind every chunk of four.
@@ -411,6 +500,30 @@ int normals_knn_device(peb_ctx* ctx, const float4* d_in, int n, int k, const flo
   const size_t smem = static_cast<size_t>(k) * T * 8;
   PEB_LAUNCH(ctx, normals_knn_kernel, ceil_div(g.n, T), T, smem, g, k, vp[0], vp[1], vp[2], d_out8, d_out_nn,
              static_cast<const int*>(nullptr), static_cast<const int*>(nullptr));
+  return PEB_OK;
+}
+
+int cv_normals_device(peb_ctx* ctx, const float4* d_in, int n, int k, bool flip, const float vp[3], float* d_out6,
+                      int32_t* d_out_nn) {
+  if (k < 1) return fail(ctx, PEB_E_INVALID_ARG, "cv_normals: k must be >= 1 (got %d)", k);
+  if (k > 192) return fail(ctx, PEB_E_UNSUPPORTED, "cv_normals: k = %d > 192 has no CUDA path (no CPU fallback)", k);
+  if (n == 0) return PEB_OK;
+  // the grid and the cell edge of normals_knn_device: the search is the same
+  const float occupancy = fmaxf(2.0f, static_cast<float>(k) / 2.4f);
+  PEB_TRY(grid_build(ctx, &ctx->aux_grid, d_in, nullptr, n, occupancy));
+  const GridView& g = ctx->aux_grid.view;
+  if (k > g.n)
+    return fail(ctx, PEB_E_INVALID_ARG, "cv_normals: k = %d exceeds the %d finite points of the cloud", k, g.n);
+  PEB_LAUNCH(ctx, cv_normals_fill_kernel, ceil_div(n, 256), 256, 0, d_in, n, d_out6);
+  if (d_out_nn) PEB_CUDA(ctx, cudaMemsetAsync(d_out_nn, 0xFF, static_cast<size_t>(n) * k * sizeof(int32_t), ctx->stream));
+  const CvNormalArgs a{k, flip ? 1 : 0, vp[0], vp[1], vp[2], d_out6, d_out_nn};
+  if (k <= 8) return launch_cv_reglist<8>(ctx, g, a);
+  if (k <= 16) return launch_cv_reglist<16>(ctx, g, a);
+  if (k <= 24) return launch_cv_reglist<24>(ctx, g, a);
+  if (k <= 32) return launch_cv_reglist<32>(ctx, g, a);
+  const int T = k <= 48 ? 128 : (k <= 96 ? 64 : 32);
+  const size_t smem = static_cast<size_t>(k) * T * 8;
+  PEB_LAUNCH(ctx, cv_normals_knn_kernel, ceil_div(g.n, T), T, smem, g, a);
   return PEB_OK;
 }
 

@@ -541,6 +541,22 @@ class NormalEstimation:
         return (out, nn) if return_neighbours else out
 
 
+def compute_normals_pc3d(pc, num_neighbors: int = 20, flip_viewpoint: bool = True, viewpoint=(0.0, 0.0, 0.0),
+                         ctx: Context | None = None, return_neighbours: bool = False):
+    """cv::ppf_match_3d::computeNormalsPC3d(pc, out, num_neighbors, flip_viewpoint, viewpoint), the reference's normals
+    slot (pose_estimation/src/opencv_surface_match.cpp:57-59), with OpenCV's arithmetic (peb_cv_normals, DESIGN.md §13).
+    pc: (N, >=3) float32 -> (N, 6) float32 rows x y z nx ny nz; with return_neighbours also the (N, k) int32 lists."""
+    ctx = ctx or default_context()
+    p = _cloud(pc)
+    k = int(num_neighbors)
+    vp = np.ascontiguousarray(np.asarray(viewpoint, np.float32).reshape(3))
+    out = np.empty((p.shape[0], 6), np.float32)
+    nn = np.empty((p.shape[0], max(k, 0)), np.int32) if return_neighbours else None
+    ctx.check(lib.peb_cv_normals(ctx.handle, p.ctypes.data, p.shape[0], _stride(p), k, int(bool(flip_viewpoint)),
+                                 vp.ctypes.data, out.ctypes.data, nn.ctypes.data if nn is not None else None))
+    return (out, nn) if return_neighbours else out
+
+
 class ConvergenceCriteria:
     """The part of pcl::registration::DefaultConvergenceCriteria<float> reachable through
     IterativeClosestPoint::getConvergeCriteria()."""
