@@ -8,6 +8,7 @@
 #include <string>
 #include <new>
 
+#include "block_select.cuh"
 #include "core_math.cuh"
 
 namespace peb {
@@ -122,6 +123,20 @@ int guarded(peb_ctx* ctx, const char* what, Fn fn) noexcept {
   return code;
 }
 
+// peb_debug_select_nth: one 1024-thread block per requested rank
+struct DebugLoad {
+  const float* v;
+  __device__ float operator()(int i) const { return v[i]; }
+};
+template <bool SKIP_NEG>
+__global__ void __launch_bounds__(1024) debug_select_nth_kernel(const float* __restrict__ v, int m, const int32_t* __restrict__ nths,
+                                                                float* __restrict__ out) {
+  __shared__ unsigned hist[2048];
+  __shared__ unsigned st[2];
+  __shared__ unsigned wsum[32];
+  const float r = block_select_nth<DebugLoad, SKIP_NEG>(DebugLoad{v}, m, nths[blockIdx.x], hist, st, wsum);
+  if (threadIdx.x == 0) out[blockIdx.x] = r;
+}
 }  // namespace
 }  // namespace peb
 
@@ -1020,6 +1035,43 @@ extern "C" PEB_API int peb_debug_exclusive_scan(peb_ctx* ctx, const uint32_t* in
     if (out_total) cudaMemcpyAsync(out_total, d + n, 4, cudaMemcpyDeviceToHost, ctx->stream);
     rc = sync(ctx);
   }
+  b.release();
+  return rc;
+}
+
+
+// development aid (not in the public header): block_select_nth over host values, one result per rank in nths, for
+// tests/test_gpu_block_select.py.  Every rank must be below the number of values taken (all m, or with skip_neg the
+// ones whose sign bit is clear); a rank outside is refused here, before any launch.
+extern "C" PEB_API int peb_debug_select_nth(peb_ctx* ctx, const float* values, size_t m, const int32_t* nths, size_t n_nth, int skip_neg,
+                                            float* out) {
+  if (!ctx || !values || !nths || !out || m == 0 || m > (1u << 30) || n_nth == 0 || n_nth > 65535) return PEB_E_INVALID_ARG;
+  size_t taken = m;
+  if (skip_neg) {
+    taken = 0;
+    for (size_t i = 0; i < m; ++i) taken += !std::signbit(values[i]);
+  }
+  for (size_t k = 0; k < n_nth; ++k)
+    if (nths[k] < 0 || static_cast<size_t>(nths[k]) >= taken)
+      return fail(ctx, PEB_E_INVALID_ARG, "debug_select_nth: rank %d outside the %zu values taken", nths[k], taken);
+  DeviceGuard guard(ctx->device);
+  DevBuf b;
+  const size_t o_nth = (m * 4 + 255) & ~static_cast<size_t>(255), o_out = o_nth + ((n_nth * 4 + 255) & ~static_cast<size_t>(255));
+  if (b.ensure(o_out + n_nth * 4) != cudaSuccess) return fail(ctx, PEB_E_OOM, "debug_select_nth: out of device memory");
+  char* base = b.as<char>();
+  float* d_v = reinterpret_cast<float*>(base);
+  int32_t* d_nth = reinterpret_cast<int32_t*>(base + o_nth);
+  float* d_out = reinterpret_cast<float*>(base + o_out);
+  const int rc = [&]() -> int {
+    PEB_CUDA(ctx, cudaMemcpyAsync(d_v, values, m * 4, cudaMemcpyHostToDevice, ctx->stream));
+    PEB_CUDA(ctx, cudaMemcpyAsync(d_nth, nths, n_nth * 4, cudaMemcpyHostToDevice, ctx->stream));
+    if (skip_neg)
+      PEB_LAUNCH(ctx, debug_select_nth_kernel<true>, static_cast<int>(n_nth), 1024, 0, d_v, static_cast<int>(m), d_nth, d_out);
+    else
+      PEB_LAUNCH(ctx, debug_select_nth_kernel<false>, static_cast<int>(n_nth), 1024, 0, d_v, static_cast<int>(m), d_nth, d_out);
+    PEB_CUDA(ctx, cudaMemcpyAsync(out, d_out, n_nth * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    return sync(ctx);
+  }();
   b.release();
   return rc;
 }

@@ -7,9 +7,12 @@
 namespace peb {
 
 // exact order statistic `nth` of m non-negative floats f(i), by three radix passes over the float bits (11 + 11 + 10);
-// one block of 1024 threads; returns the value to every thread.  nth < (number of values taken).
+// one block of 1024 threads; returns the value to every thread.  The result is the nth of the taken values ordered by
+// their bit patterns (for non-negative floats, +inf and denormals included, their numeric order).
+// Precondition: nth < (number of values taken).  Outside it no bin holds the rank and the bin state read after the
+// scan is whatever an earlier pass or call left in shared memory.
 // SKIP_NEG: values with the sign bit set are not taken (how a caller leaves entries out); the values of the others
-// and nth then refer to the taken ones only.
+// and nth then refer to the taken ones only.  -0.0f has the sign bit and is skipped as well.
 template <typename F, bool SKIP_NEG = false>
 __device__ float block_select_nth(F f, int m, int nth, unsigned* hist /* shared [2048] */, unsigned* s_state /* shared [2] */,
                                   unsigned* s_wsum /* shared [32] */) {

@@ -23,6 +23,7 @@
 //                      Frobenius error: one record per block, the host adds them in block order
 //     host             solve, PoseX = [Rx (Ry Rz) | t], fval / fval_old against the level's tolerance
 //     cv_move          Src_Moved = PoseX * srcPCT
+// Clouds are expected finite: a NaN row makes meanAvg NaN, here as in OpenCV.
 #include <algorithm>
 #include <cmath>
 #include <vector>

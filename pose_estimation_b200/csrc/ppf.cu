@@ -26,7 +26,8 @@
 //              poses (sorted by votes) — sequential by definition, microseconds of work.
 // Double precision throughout the feature / alpha / pose arithmetic like upstream (Vec3d); sin / cos / acos / atan2 are
 // CUDA's double functions (<= 2 ulp from glibc's): a feature within an ulp of a bin edge may quantise differently
-// than on the CPU (tests/test_ppf.py counts such cases; none in the committed cases).
+// than on the CPU (tests/test_ppf.py counts such cases; none in the committed cases; tests/test_gpu_ppf_edges.py fails on
+// any disagreement with the oracle that no quotient within 1e-12 of a bin edge explains).
 #include <algorithm>
 #include <cmath>
 #include <cstring>
