@@ -303,11 +303,11 @@ __device__ __forceinline__ bool graph_pays(const IcpLaunch& L, const IcpState* s
   return cnt > 0.0 && 4.0 * mse * static_cast<double>(L.knn_kappa) * cnt < __ldcg(L.knn_stat);
 }
 
-// adds one accepted correspondence (working point p, match best) to the estimator's moment sums
+// adds one accepted correspondence (working point p, match t = the target's point j, squared distance d2) to the
+// estimator's moment sums
 template <int EST, int NACC>
-__device__ __forceinline__ void accumulate_pair_impl(const GridView& g, const float4& p, const NnBest& best,
-                                                     double (&acc)[NACC]) {
-  const float4 t = g.pts[best.j];
+__device__ __forceinline__ void add_moments(const GridView& g, const float4& p, const float4& t, int j, float d2,
+                                            double (&acc)[NACC]) {
   if (EST == PEB_ESTIMATOR_SVD) {
     const double sx = p.x, sy = p.y, sz = p.z, tx = t.x, ty = t.y, tz = t.z;
     acc[0] += 1.0;
@@ -328,11 +328,11 @@ __device__ __forceinline__ void accumulate_pair_impl(const GridView& g, const fl
     acc[13] = fma(tz, sx, acc[13]);
     acc[14] = fma(tz, sy, acc[14]);
     acc[15] = fma(tz, sz, acc[15]);
-    acc[16] += static_cast<double>(best.d2);
+    acc[16] += static_cast<double>(d2);
   } else {
     acc[0] += 1.0;
-    acc[NACC - 1] += static_cast<double>(best.d2);
-    const float4 nr = g.normals[best.j];
+    acc[NACC - 1] += static_cast<double>(d2);
+    const float4 nr = g.normals[j];
     // [PCL] transformation_estimation_point_to_plane_lls.hpp: pairs with a non-finite
     // member are left out of the normal equations (they still count as correspondences)
     if (finite3(t.x, t.y, t.z) && finite3(nr.x, nr.y, nr.z)) {
@@ -372,11 +372,13 @@ __device__ __forceinline__ void accumulate_pair_impl(const GridView& g, const fl
     }
   }
 }
+// adds one accepted correspondence (working point p, match best) to the estimator's moment sums
 template <int EST, int NACC>
 __device__ __forceinline__ void accumulate_pair(const GridView& g, const float4& p, const NnBest& best,
                                                 double (&acc)[NACC]) {
   static_assert((EST == PEB_ESTIMATOR_SVD && NACC == kAccSvd) || (EST != PEB_ESTIMATOR_SVD && NACC == kAccLls), "layout");
-  accumulate_pair_impl<EST, NACC>(g, p, best, acc);
+  const float4 t = g.pts[best.j];
+  add_moments<EST, NACC>(g, p, t, best.j, best.d2, acc);
 }
 
 // First-iteration search of the 32 queries of a warp (one source patch), all lanes together.  A query
@@ -862,6 +864,60 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_search_kernel(const IcpLa
   }
 }
 
+// ---- the moment launch's copy pipeline ----
+// In pass k, block blk of a hypothesis reads queries blk * 128 + t + k * blocks_per_hyp * 128: one contiguous 2 KB chunk of
+// the working cloud per pass.  A per-thread load loop keeps one 512-byte load per warp in flight and then waits for the
+// dependent gather of the match, about 16 KB per SM: the launch was bound by that, at a third of HBM bandwidth.  Instead
+// thread 0 streams the chunks into a ring of kMomentRing slots in shared memory with 1-D bulk copies (one mbarrier per slot):
+// a slot is refilled once every thread has added its pass, kMomentRing - 2 passes before the threads read it.  The
+// accumulators keep their registers and every thread still adds its queries in increasing pass order, so every double is
+// summed as before.
+#ifndef PEB_MOMENT_RING
+#define PEB_MOMENT_RING 4
+#endif
+constexpr int kMomentRing = PEB_MOMENT_RING;  // (development: -DPEB_MOMENT_RING=n builds a variant library, PEB_LIB_VARIANT)
+static_assert(kMomentRing >= 2 && (kMomentRing & (kMomentRing - 1)) == 0, "ring depth: a power of two >= 2");
+#ifndef PEB_MOMENT_EVICT_FIRST
+#define PEB_MOMENT_EVICT_FIRST 0
+#endif
+
+__device__ __forceinline__ uint32_t smem_addr(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
+
+// thread 0: `bytes` (a multiple of 16) from global src into shared dst; completion is counted on the mbarrier bar
+__device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+#if PEB_MOMENT_EVICT_FIRST
+  // the working clouds are read once per iteration: let them leave L2 before the target's structures do
+  uint64_t policy;
+  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
+               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(policy) : "memory");
+#else
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+#endif
+}
+
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+  asm volatile(
+      "{\n"
+      ".reg .pred done;\n"
+      "WAIT:\n"
+      "mbarrier.try_wait.parity.shared::cta.b64 done, [%0], %1;\n"
+      "@!done bra WAIT;\n"
+      "}\n" ::"r"(bar), "r"(parity) : "memory");
+}
+
+// one query of a moment pass: its match j (-1: no pair) and the match t, read one pass before the query is added.  (The
+// working point is read from the ring again when it is added: 3 registers less in flight.  The point-to-plane sums hold
+// 58 of the 64 registers in doubles: there the match and its normal are read when added, as before, so as not to spill.)
+template <int EST>
+struct MomentGather {
+  static constexpr bool kAhead = EST == PEB_ESTIMATOR_SVD;
+  float4 t;
+  int j;
+};
+
 // CHAIN: the align has a rejector chain (icp_reject_kernel ran between the two launches): a pair is summed iff
 // kept[i] of its hypothesis is set, and the single align's correspondence outputs are written here.
 template <int EST, int MB, bool CHAIN>
@@ -877,47 +933,108 @@ __global__ void __launch_bounds__(kIcpThreads, MB) icp_moment_kernel(const IcpLa
   __shared__ double sm[kIcpThreads / 32][kAccMax];
   __shared__ double sm_tot[kAccMax];
   __shared__ int s_active;
+  __shared__ alignas(16) float4 s_ring[kMomentRing][kIcpThreads];
+  __shared__ alignas(8) unsigned long long s_full[kMomentRing];
   IcpState* st = L.states + h;
   if (threadIdx.x == 0) s_active = __ldcg(&st->active);
   __syncthreads();
-  if (!s_active) return;
+  if (!s_active) return;  // (before any copy: a block never leaves with one outstanding)
 
   double acc[NACC];
 #pragma unroll
   for (int i = 0; i < NACC; ++i) acc[i] = 0.0;
   const float4* work = L.work + static_cast<size_t>(h) * L.n_src;
-  for (int i = blk * kIcpThreads + threadIdx.x; i < L.n_src; i += L.blocks_per_hyp * kIcpThreads) {
-    const float4 p = __ldcg(work + i);
-    bool valid = finite3(p.x, p.y, p.z);
+  const int i0 = blk * kIcpThreads, stride = L.blocks_per_hyp * kIcpThreads;
+  const int n_pass = i0 < L.n_src ? (L.n_src - i0 + stride - 1) / stride : 0;  // (block-uniform)
+  // pass k into slot k % kMomentRing; the last chunk is clipped to n_src
+  auto issue = [&](int k) {
+    const int i = i0 + k * stride;
+    const int slot = k & (kMomentRing - 1);
+    bulk_copy_g2s(smem_addr(s_ring[slot]), work + i, static_cast<uint32_t>(min(kIcpThreads, L.n_src - i)) * sizeof(float4),
+                  smem_addr(&s_full[slot]));
+  };
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int s = 0; s < kMomentRing; ++s) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&s_full[s])) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    // The working points were written by the search grid through the generic proxy and acquired above (wait_for_search or
+    // griddepcontrol.wait); the bulk copies read them through the async proxy, which that acquire does not order.
+    asm volatile("fence.proxy.async.global;" ::: "memory");
+    for (int k = 0; k < min(kMomentRing, n_pass); ++k) issue(k);
+  }
+  __syncthreads();
+
+  // waits for pass k's chunk, reads this thread's query and starts the gathers of its match
+  using Gather = MomentGather<EST>;
+  auto fetch = [&](int k, Gather& q) {
+    const int slot = k & (kMomentRing - 1);
+    mbar_wait(smem_addr(&s_full[slot]), (k / kMomentRing) & 1);
+    const int i = i0 + k * stride + threadIdx.x;
+    q.j = -1;
+    if (i >= L.n_src) return;  // (past the clipped end: the slot holds an older chunk's bytes)
+    const float4 p = s_ring[slot][threadIdx.x];
     int j = __float_as_int(p.w);
-    if (j <= -2) {  // made non-finite by this launch's transform: searched all the same (see above)
-      valid = true;
-      j = -2 - j;
-    }
+    if (j <= -2) j = -2 - j;  // made non-finite by this launch's transform: searched all the same (see above)
+    else if (!finite3(p.x, p.y, p.z)) j = -1;
+    q.j = j;
+    if (Gather::kAhead && j >= 0) q.t = L.grid.pts[j];
+  };
+  auto add = [&](int k, const Gather& q) {
+    const float4 p = s_ring[k & (kMomentRing - 1)][threadIdx.x];
+    const int i = i0 + k * stride + threadIdx.x;
     if (CHAIN) {
       NnBest best;
-      const bool keep = valid && j >= 0 && kept[static_cast<size_t>(h) * L.n_src + i];
+      const bool keep = q.j >= 0 && kept[static_cast<size_t>(h) * L.n_src + i];
       if (keep) {
-        const float4 t = L.grid.pts[j];
+        const float4 t = Gather::kAhead ? q.t : L.grid.pts[q.j];
         best.d2 = l2_simple(p.x, p.y, p.z, t.x, t.y, t.z);
         best.idx = point_index(t);
-        best.j = j;
-        accumulate_pair<EST>(L.grid, p, best, acc);
+        add_moments<EST, NACC>(L.grid, p, t, q.j, best.d2, acc);
       }
-      if (L.corr_idx) {
+      if (L.corr_idx && i < L.n_src) {
         const int orig = __float_as_int(L.src[i].w);
         L.corr_idx[orig] = keep ? best.idx : -1;
         L.corr_d2[orig] = keep ? best.d2 : 0.0f;
       }
-      continue;
+      return;
     }
-    if (!valid || j < 0) continue;
-    const float4 t = L.grid.pts[j];
+    if (q.j < 0) return;
+    const float4 t = Gather::kAhead ? q.t : L.grid.pts[q.j];
     NnBest best;
     best.d2 = l2_simple(p.x, p.y, p.z, t.x, t.y, t.z);
     best.idx = point_index(t);
-    best.j = j;
-    if (keep_pair(L, valid, best)) accumulate_pair<EST>(L.grid, p, best, acc);
+    best.j = q.j;
+    if (keep_pair(L, true, best)) add_moments<EST, NACC>(L.grid, p, t, q.j, best.d2, acc);
+  };
+  // at pass k: every thread has added pass k - 1, whose slot takes pass k - 1 + kMomentRing
+  auto refill = [&](int k) {
+    __syncthreads();
+    if (threadIdx.x == 0 && k >= 1 && k - 1 + kMomentRing < n_pass) issue(k - 1 + kMomentRing);
+  };
+  // pass k: refill, start pass k + 1's gathers into `next`, add pass k (`cur`)
+  auto step = [&](int k, const Gather& cur, Gather& next) {
+    refill(k);
+    if (k + 1 < n_pass) fetch(k + 1, next);
+    add(k, cur);
+  };
+
+  if constexpr (Gather::kAhead) {
+    // (two records that swap roles: a copy from one to the other would wait for the gathers in flight)
+    Gather qa, qb;
+    if (n_pass > 0) fetch(0, qa);
+#pragma unroll 1
+    for (int k = 0; k < n_pass; k += 2) {
+      step(k, qa, qb);
+      if (k + 1 < n_pass) step(k + 1, qb, qa);
+    }
+  } else {
+#pragma unroll 1
+    for (int k = 0; k < n_pass; ++k) {
+      refill(k);
+      Gather q;
+      fetch(k, q);
+      add(k, q);
+    }
   }
 
   // ---- the block's record, the last block's solve: as in icp_iteration_body ----

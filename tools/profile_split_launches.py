@@ -124,7 +124,7 @@ def main():
             rows.append({"iteration": it, "search_ms": round(statistics.median(search), 4),
                          "moment_ms": round(statistics.median(moment), 4),
                          "moment_span_ms": round(statistics.median(span), 4), "search_kernel": sorted(names)})
-    out = {"card": info, "card_after": card(), "workload": "C4", "hypotheses": len(c4.guess),
+    out = {"card": info, "card_after": card(), "workload": "C4", "hypotheses": len(c4.guess), "n_src": len(c4.source),
            "iterations": bench.ITERATIONS, "steps": args.steps, "statistic": "median over steps",
            "profile_level": 2, "per_iteration": rows,
            "search_ms_total": round(sum(r["search_ms"] for r in rows), 3),
