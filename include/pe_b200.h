@@ -293,7 +293,8 @@ typedef struct peb_ppf_pose {
 } peb_ppf_pose;
 typedef struct peb_ppf_model peb_ppf_model;
 PEB_API void peb_ppf_params_default(peb_ppf_params* p); /* (0.03, 0.03, 40), thresholds -1, plain average */
-/* trainModel: the trained detector lives on ctx's device and belongs to ctx (destroy it before the context) */
+/* trainModel: the trained detector lives on ctx's device and belongs to ctx (destroy it before the context; destroying it
+ * after the context only frees its device memory, it never touches the destroyed context) */
 PEB_API int peb_ppf_train(peb_ctx* ctx, const float* model_xyzn, size_t n_model, const peb_ppf_params* params,
                           peb_ppf_model** out);
 PEB_API void peb_ppf_model_destroy(peb_ppf_model* m);
@@ -304,6 +305,51 @@ PEB_API int peb_ppf_model_sampled(const peb_ppf_model* m, float* out6, size_t ca
 PEB_API int peb_ppf_match(peb_ctx* ctx, const peb_ppf_model* m, const float* scene_xyzn, size_t n_scene,
                           double relative_scene_sample_step, double relative_scene_distance, peb_ppf_pose* results,
                           size_t cap, size_t* out_n, peb_ppf_pose* raw, size_t cap_raw, size_t* out_n_raw);
+
+/* ---- OpenCVSurfaceMatch::find_object_in_scene in one call ---------------------------------------------------------
+ * pose_estimation/src/opencv_surface_match.cpp:57-142 (with pose_estimation.cpp:211-345 in front of it): the cloud goes to
+ * the device once, every step runs there on a scene that stays resident, and the selected pose comes back.  The result is
+ * exactly what these calls give when made one after the other on the same context (same bytes):
+ *   1. peb_scene_prepare(pts, n, stride, filter, num_planes, sac, leaf) — skipped entirely when filter == NULL: pts is then
+ *      the N x 3 (or N x 6) cv::Mat find_object_in_scene receives, and num_planes, sac and leaf are ignored;
+ *   2. peb_cv_normals(normals_k, flip_viewpoint, viewpoint)                                         (:57-59)
+ *   3. peb_ppf_match(model, relative_scene_sample_step, relative_scene_distance)                    (:65)
+ *   4. peb_cvicp_register on the first max_icp_poses clustered poses, with the rows the model was trained on  (:85-94)
+ *   5. the selection rule of :100-124 (pe_b200::select_best_pose) over the refined poses;
+ *   6. the packing of :133-142 from refined[best].t and .q.
+ * refined[i] is the Pose3D registerModelToScene leaves behind: pose = the appended pose, q / t / angle recomputed from it
+ * (Pose3D::appendPose), residual filled, num_votes / model_index / alpha those of the cluster.
+ * refined must hold max_icp_poses records; out_scene_xyzn6 (nullable) n x 6 floats: the prepared scene with its normals
+ * (what the reference dumps as scene.ply at :127-132), *out_n_scene (nullable) its rows.
+ * Errors are those of the step entry points, same codes and messages; in addition a model trained on another context,
+ * max_icp_poses outside [1, 4096] and a NULL refined / out / params are PEB_E_INVALID_ARG.  An empty scene (from the input
+ * or after the preparation) is PEB_OK with n_results = 0 and best = -1; no ICP runs then. */
+typedef struct peb_surface_match_params {
+  int32_t normals_k;                  /* computeNormalsPC3d(.., 20, ..)                                        */
+  int32_t flip_viewpoint;             /* true                                                                  */
+  float viewpoint[3];                 /* (0, 0, 0)                                                             */
+  int32_t max_icp_poses;              /* 6: results_subset, opencv_surface_match.cpp:89-92                     */
+  double relative_scene_sample_step;  /* match(.., 1.0, ..)                                                    */
+  double relative_scene_distance;     /* match(.., .., 0.03)                                                   */
+  peb_cvicp_params icp;               /* ICP(250, 0.005f, 2.5f, 8)                                             */
+  int32_t reference_layout;           /* 1: pose7 exactly as :133-142 writes it (qz never written, left 0)     */
+  int32_t reserved;
+} peb_surface_match_params;
+/* the reference's values (listed above); reference_layout 0 */
+PEB_API void peb_surface_match_params_default(peb_surface_match_params* p);
+
+typedef struct peb_surface_match_result {
+  uint64_t n_results;  /* clustered PPF results (results.size()): the "> 5" of the selection rule */
+  int32_t n_refined;   /* min(n_results, max_icp_poses)                                            */
+  int32_t best;        /* index into the refined poses; -1 when n_results == 0                     */
+  float pose7[7];      /* {x y z qx qy qz qw} of refined[best]; zeros when best == -1               */
+  int32_t reserved;
+} peb_surface_match_result;
+
+PEB_API int peb_surface_match(peb_ctx* ctx, const peb_ppf_model* model, const void* pts, size_t n, size_t stride,
+                              const peb_prefilter_params* filter, int num_planes, const peb_sac_params* sac, float leaf,
+                              const peb_surface_match_params* params, peb_ppf_pose* refined, peb_surface_match_result* out,
+                              float* out_scene_xyzn6, size_t* out_n_scene);
 
 /* ---- pcl::NormalEstimation<PointXYZ,Normal>::compute  [PCL] features/.../impl/normal_3d.hpp */
 /* out_normal8: n x 8 floats = pcl::Normal memory image (nx ny nz 0 | curvature 0 0 0). */

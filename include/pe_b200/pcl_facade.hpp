@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "../pe_b200.h"
+#include "pose_select.hpp"
 
 namespace pe_b200 {
 
@@ -96,10 +97,9 @@ class ScenePrefilter {
 // PoseEstimation::create_surface_match_pc (pose_estimation/src/pose_estimation.cpp:246-261 + remove_planes :281-345) in ONE
 // library call: NaN removal, optional sphere filter, num_planes rounds of plane RANSAC + band removal, optional VoxelGrid.
 // The cloud crosses PCIe once in each direction.  planes (optional): num_planes x 4 coefficients.
-inline void create_surface_match_pc(Context& c, const void* pts, size_t n, size_t stride, const float* filter_pose,
-                                    float filter_radius, const std::string& filter_out, int num_planes, float leaf,
-                                    std::vector<float>& out_xyz4, std::vector<float>* planes = nullptr) {
-  peb_prefilter_params f;
+// the filter and RANSAC settings create_surface_match_pc applies (filter_pose == nullptr or radius <= 0: no sphere filter)
+inline void surface_match_pc_params(const float* filter_pose, float filter_radius, const std::string& filter_out,
+                                    peb_prefilter_params& f, peb_sac_params& sac) {
   std::memset(&f, 0, sizeof(f));
   f.plane_band = 0.005f;                                    // :320
   if (filter_pose && filter_radius > 0.0f) {                // :250-256
@@ -108,10 +108,17 @@ inline void create_surface_match_pc(Context& c, const void* pts, size_t n, size_
     for (int i = 0; i < 3; ++i) f.sphere_center[i] = filter_pose[i];
     f.sphere_radius = filter_radius;
   }
-  peb_sac_params sac;
   peb_sac_params_default(&sac);
   sac.distance_threshold = 0.0001;                          // :294
   sac.max_iterations = 100;                                 // :295
+}
+
+inline void create_surface_match_pc(Context& c, const void* pts, size_t n, size_t stride, const float* filter_pose,
+                                    float filter_radius, const std::string& filter_out, int num_planes, float leaf,
+                                    std::vector<float>& out_xyz4, std::vector<float>* planes = nullptr) {
+  peb_prefilter_params f;
+  peb_sac_params sac;
+  surface_match_pc_params(filter_pose, filter_radius, filter_out, f, sac);
   out_xyz4.resize(4 * (n ? n : 1));
   std::vector<float> pl(4 * static_cast<size_t>(num_planes > 0 ? num_planes : 1), 0.0f);
   size_t m = 0;
@@ -338,28 +345,7 @@ class IterativeClosestPoint {
 };
 
 // ---- the step right after the path (SURVEY.md 8f rank 3): host-side, no device work ----------------
-// Which refined hypothesis the node returns: pose_estimation/src/opencv_surface_match.cpp:100-124.
-// Most votes wins; but if the matcher produced more than 5 results in total, the lowest residual among
-// the refined poses with more than 400 votes overrides it (the loop keeps the LAST assignment, so a later
-// pose with more votes still takes over — reproduced as written).
-inline size_t select_best_pose(const int* num_votes, const double* residual, size_t n_subset, size_t n_results_total) {
-  int max_votes = 0;
-  float min_res = 10000.0f;
-  size_t best_idx = 0;
-  for (size_t i = 0; i < n_subset; ++i) {
-    if (num_votes[i] > max_votes) {
-      max_votes = num_votes[i];
-      best_idx = i;
-    }
-    if (n_results_total > 5) {
-      if (residual[i] < min_res && num_votes[i] > 400) {
-        min_res = static_cast<float>(residual[i]);
-        best_idx = i;
-      }
-    }
-  }
-  return best_idx;
-}
+// select_best_pose and pack_pose3d are in pose_select.hpp (the library runs them too, in peb_surface_match).
 
 // rotation part of a column-major 4x4 -> unit quaternion (w, x, y, z), w >= 0
 inline void rotation_to_quat(const float* T16, double q[4]) {
@@ -440,6 +426,7 @@ class PPF3DDetector {
     p_.num_angles = numAngles;
   }
   ~PPF3DDetector() { peb_ppf_model_destroy(m_); }
+  const peb_ppf_model* model() const { return m_; }  // the trained detector (nullptr before trainModel)
   PPF3DDetector(const PPF3DDetector&) = delete;
   PPF3DDetector& operator=(const PPF3DDetector&) = delete;
   void setSearchParams(double positionThreshold = -1, double rotationThreshold = -1, bool useWeightedClustering = false) {
@@ -472,6 +459,49 @@ class PPF3DDetector {
   peb_ppf_params p_;
   peb_ppf_model* m_ = nullptr;
 };
+
+// OpenCVSurfaceMatch::find_object_in_scene (pose_estimation/src/opencv_surface_match.cpp:57-142) in ONE library call
+// (peb_surface_match): computeNormalsPC3d, detector.match, cv ICP of the first params.max_icp_poses results against the rows
+// the detector was trained on, the selection rule and the packing.  pts: the N x 3 (or N x 6) CV_32F cloud the function
+// receives (ptr<float>(0), step).  refined: the refined Pose3D records; pose7: {x y z qx qy qz qw} of refined[best] (zeros
+// when nothing was found: result.best == -1).  Same bytes as the step-by-step calls above.
+inline peb_surface_match_result find_object_in_scene(Context& c, const PPF3DDetector& detector, const void* pts, size_t n,
+                                                     size_t stride, const peb_surface_match_params& params,
+                                                     std::vector<peb_ppf_pose>& refined, float pose7[7],
+                                                     std::vector<float>* scene_xyzn6 = nullptr) {
+  refined.resize(params.max_icp_poses > 0 ? static_cast<size_t>(params.max_icp_poses) : 1);
+  if (scene_xyzn6) scene_xyzn6->resize(6 * (n ? n : 1));
+  peb_surface_match_result r;
+  size_t m = 0;
+  c.check(peb_surface_match(c.get(), detector.model(), pts, n, stride, nullptr, 0, nullptr, 0.0f, &params, refined.data(), &r,
+                            scene_xyzn6 ? scene_xyzn6->data() : nullptr, &m));
+  refined.resize(static_cast<size_t>(r.n_refined));
+  if (scene_xyzn6) scene_xyzn6->resize(6 * m);
+  std::memcpy(pose7, r.pose7, sizeof(r.pose7));
+  return r;
+}
+
+// The same from the organised cloud on: PoseEstimation::create_surface_match_pc's preparation (arguments as in
+// create_surface_match_pc above; leaf 0 = no VoxelGrid, as the reference) in front, the cloud crossing PCIe once.
+inline peb_surface_match_result find_object_in_scene(Context& c, const PPF3DDetector& detector, const void* pts, size_t n,
+                                                     size_t stride, const float* filter_pose, float filter_radius,
+                                                     const std::string& filter_out, int num_planes, float leaf,
+                                                     const peb_surface_match_params& params, std::vector<peb_ppf_pose>& refined,
+                                                     float pose7[7], std::vector<float>* scene_xyzn6 = nullptr) {
+  peb_prefilter_params f;
+  peb_sac_params sac;
+  surface_match_pc_params(filter_pose, filter_radius, filter_out, f, sac);
+  refined.resize(params.max_icp_poses > 0 ? static_cast<size_t>(params.max_icp_poses) : 1);
+  if (scene_xyzn6) scene_xyzn6->resize(6 * (n ? n : 1));
+  peb_surface_match_result r;
+  size_t m = 0;
+  c.check(peb_surface_match(c.get(), detector.model(), pts, n, stride, &f, num_planes, &sac, leaf, &params, refined.data(), &r,
+                            scene_xyzn6 ? scene_xyzn6->data() : nullptr, &m));
+  refined.resize(static_cast<size_t>(r.n_refined));
+  if (scene_xyzn6) scene_xyzn6->resize(6 * m);
+  std::memcpy(pose7, r.pose7, sizeof(r.pose7));
+  return r;
+}
 
 // The manager's side of the pose (pose_estimation_manager/src/pose_transformer.cpp:78-121, PoseTransformer::obj_in_base_frame):
 // the published {x, y, z, qx, qy, qz, qw} (camera frame) -> hand-eye calibration (row-major 4x4, he_calibration_mat_) -> the

@@ -151,6 +151,21 @@ class PpfPose(C.Structure):
         return np.array(self.pose, np.float64).reshape(4, 4)
 
 
+class SurfaceMatchParams(C.Structure):
+    """peb_surface_match_params (64 bytes)."""
+
+    _fields_ = [("normals_k", C.c_int32), ("flip_viewpoint", C.c_int32), ("viewpoint", C.c_float * 3), ("max_icp_poses", C.c_int32),
+                ("relative_scene_sample_step", C.c_double), ("relative_scene_distance", C.c_double), ("icp", CvIcpParams),
+                ("reference_layout", C.c_int32), ("reserved", C.c_int32)]
+
+
+class SurfaceMatchResult(C.Structure):
+    """peb_surface_match_result (48 bytes)."""
+
+    _fields_ = [("n_results", C.c_uint64), ("n_refined", C.c_int32), ("best", C.c_int32), ("pose7", C.c_float * 7),
+                ("reserved", C.c_int32)]
+
+
 class GridInfo(C.Structure):
     _fields_ = [
         ("origin", C.c_float * 3),
@@ -186,6 +201,9 @@ SYMBOLS = {
     "peb_ppf_model_destroy": (None, [_vp]),
     "peb_ppf_model_sampled": (_i, [_vp, _vp, _sz, _pp(_sz)]),
     "peb_ppf_match": (_i, [_vp, _vp, _vp, _sz, _d, _d, _vp, _sz, _pp(_sz), _vp, _sz, _pp(_sz)]),
+    "peb_surface_match_params_default": (None, [_pp(SurfaceMatchParams)]),
+    "peb_surface_match": (_i, [_vp, _vp, _vp, _sz, _sz, _pp(PrefilterParams), _i, _pp(SacParams), _f, _pp(SurfaceMatchParams), _vp,
+                               _pp(SurfaceMatchResult), _vp, _pp(_sz)]),
     "peb_normals_knn": (_i, [_vp, _vp, _sz, _sz, _i, _vp, _vp]),
     "peb_normals_knn_ex": (_i, [_vp, _vp, _sz, _sz, _i, _vp, _vp, _vp]),
     "peb_cv_normals": (_i, [_vp, _vp, _sz, _sz, _i, _i, _vp, _vp, _vp]),

@@ -10,6 +10,7 @@
 
 #include "block_select.cuh"
 #include "core_math.cuh"
+#include "../../include/pe_b200/pose_select.hpp"  // select_best_pose / pack_pose3d: the same definitions as the facade's
 
 namespace peb {
 
@@ -161,6 +162,21 @@ PEB_API void peb_icp_params_default(peb_icp_params* p) {
   p->fitness_max_range = DBL_MAX;
 }
 
+PEB_API void peb_surface_match_params_default(peb_surface_match_params* p) {
+  if (!p) return;
+  std::memset(p, 0, sizeof(*p));
+  // opencv_surface_match.cpp:57-59, :65, :85, :89-92
+  p->normals_k = 20;
+  p->flip_viewpoint = 1;
+  p->max_icp_poses = 6;
+  p->relative_scene_sample_step = 1.0;
+  p->relative_scene_distance = 0.03;
+  p->icp.iterations = 250;
+  p->icp.num_levels = 8;
+  p->icp.tolerance = 0.005f;
+  p->icp.rejection_scale = 2.5f;
+}
+
 PEB_API int peb_ctx_create(int device, peb_ctx** out) {
   if (!out) return PEB_E_INVALID_ARG;
   *out = nullptr;
@@ -207,7 +223,8 @@ PEB_API void peb_ctx_destroy(peb_ctx* ctx) {
   DevBuf* bufs[] = {&ctx->d_small, &ctx->d_scratch, &ctx->d_stage, &ctx->tgt_raw, &ctx->tgt_nrm_raw, &ctx->src, &ctx->work, &ctx->slack, &ctx->anchors, &ctx->nn_cache, &ctx->dbg,
                     &ctx->corr_idx, &ctx->corr_d2, &ctx->partials, &ctx->state, &ctx->trace, &ctx->d_guesses,
                     &ctx->d_results, &ctx->d_aligned, &ctx->vg_in, &ctx->vg_out, &ctx->vg_flags, &ctx->vg_scan,
-                    &ctx->vg_starts, &ctx->nrm_in, &ctx->nrm_out, &ctx->brute_keys, &ctx->nn_q, &ctx->nn_idx, &ctx->nn_d2, &ctx->epochs, &ctx->cv_arena};
+                    &ctx->vg_starts, &ctx->nrm_in, &ctx->nrm_out, &ctx->brute_keys, &ctx->nn_q, &ctx->nn_idx, &ctx->nn_d2, &ctx->epochs, &ctx->cv_arena,
+                    &ctx->cv_in, &ctx->sm_scene};
   for (DevBuf* b : bufs) b->release();
   ctx->sort_scratch.release();
   for (DevBuf& b : ctx->scan_scratch) b.release();
@@ -515,18 +532,19 @@ static int sac_plane_impl(peb_ctx* ctx, const void* pts, size_t n, size_t stride
 }
 
 // ---- create_surface_match_pc in one call ---------------------------------------------------------------
-static int scene_prepare_impl(peb_ctx* ctx, const void* pts, size_t n, size_t stride, const peb_prefilter_params* filter,
-                              int num_planes, const peb_sac_params* sac, float leaf, float* out_xyz4, size_t* out_n,
-                              float* out_planes) {
-  if (!ctx || !filter || !out_n) return PEB_E_INVALID_ARG;
-  DeviceGuard guard(ctx->device);
-  *out_n = 0;
+static int scene_prepare_check(peb_ctx* ctx, const void* pts, size_t n, size_t stride, int num_planes, const peb_sac_params* sac) {
   PEB_TRY(check_cloud(ctx, "scene_prepare", pts, n, stride));
   if (num_planes < 0 || num_planes > PEB_PREFILTER_MAX_PLANES)
     return fail(ctx, PEB_E_INVALID_ARG, "scene_prepare: num_planes %d out of [0, %d]", num_planes, PEB_PREFILTER_MAX_PLANES);
   if (num_planes > 0 && !sac) return fail(ctx, PEB_E_INVALID_ARG, "scene_prepare: plane removal needs RANSAC parameters");
-  if (n > 0 && !out_xyz4) return fail(ctx, PEB_E_INVALID_ARG, "scene_prepare: null output");
-  if (n == 0) return PEB_OK;
+  return PEB_OK;
+}
+
+// the device part of peb_scene_prepare (n > 0, arguments checked): the prepared cloud, float4 x y z 1, is left in
+// ctx->vg_in or ctx->vg_out (*d_out, *out_m points)
+static int scene_prepare_device(peb_ctx* ctx, const void* pts, size_t n, size_t stride, const peb_prefilter_params* filter,
+                                int num_planes, const peb_sac_params* sac, float leaf, const float4** d_out, size_t* out_m,
+                                float* out_planes) {
   PEB_CUDA(ctx, ctx->vg_in.ensure(n * sizeof(float4)));
   PEB_CUDA(ctx, ctx->vg_out.ensure(n * sizeof(float4)));
   float4* cur = ctx->vg_in.as<float4>();
@@ -558,9 +576,100 @@ static int scene_prepare_impl(peb_ctx* ctx, const void* pts, size_t n, size_t st
     std::swap(cur, other);
     m = v;
   }
+  *d_out = cur;
+  *out_m = m;
+  return PEB_OK;
+}
+
+static int scene_prepare_impl(peb_ctx* ctx, const void* pts, size_t n, size_t stride, const peb_prefilter_params* filter,
+                              int num_planes, const peb_sac_params* sac, float leaf, float* out_xyz4, size_t* out_n,
+                              float* out_planes) {
+  if (!ctx || !filter || !out_n) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  *out_n = 0;
+  PEB_TRY(scene_prepare_check(ctx, pts, n, stride, num_planes, sac));
+  if (n > 0 && !out_xyz4) return fail(ctx, PEB_E_INVALID_ARG, "scene_prepare: null output");
+  if (n == 0) return PEB_OK;
+  const float4* cur = nullptr;
+  size_t m = 0;
+  PEB_TRY(scene_prepare_device(ctx, pts, n, stride, filter, num_planes, sac, leaf, &cur, &m, out_planes));
   if (m > 0) PEB_CUDA(ctx, cudaMemcpyAsync(out_xyz4, cur, m * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
   PEB_TRY(sync(ctx));
   *out_n = m;
+  return PEB_OK;
+}
+
+// ---- OpenCVSurfaceMatch::find_object_in_scene in one call ------------------------------------------------
+// Buffer ownership along the chain (DESIGN.md section 14): the preparation ping-pongs between vg_in / vg_out (the
+// input upload goes through d_stage), the normals build their grid in aux_grid and write the scene rows into sm_scene,
+// which no later stage touches; the PPF match samples sm_scene into nrm_in (its frames in nrm_out, its sort in aux_grid's
+// key buffers, votes in cv_arena); the cv ICP reads the model's resident rows and sm_scene and works in cv_arena,
+// aux_grid and h_cv.
+static int surface_match_impl(peb_ctx* ctx, const peb_ppf_model* model, const void* pts, size_t n, size_t stride,
+                              const peb_prefilter_params* filter, int num_planes, const peb_sac_params* sac, float leaf,
+                              const peb_surface_match_params* prm, peb_ppf_pose* refined, peb_surface_match_result* out,
+                              float* out_scene_xyzn6, size_t* out_n_scene) {
+  if (!ctx) return PEB_E_INVALID_ARG;
+  if (out) {
+    std::memset(out, 0, sizeof(*out));
+    out->best = -1;
+  }
+  if (out_n_scene) *out_n_scene = 0;
+  if (!prm || !refined || !out) return fail(ctx, PEB_E_INVALID_ARG, "surface_match: null params / refined / out");
+  if (!model) return fail(ctx, PEB_E_INVALID_ARG, "surface_match: null model");
+  if (ppf_model_ctx(model) != ctx) return fail(ctx, PEB_E_INVALID_ARG, "surface_match: the model was trained on another context");
+  if (prm->max_icp_poses < 1 || prm->max_icp_poses > 4096)
+    return fail(ctx, PEB_E_INVALID_ARG, "surface_match: max_icp_poses %d out of [1, 4096]", prm->max_icp_poses);
+  DeviceGuard guard(ctx->device);
+  // 1. create_surface_match_pc, or the caller's cloud as it is
+  const float4* d_xyz4 = nullptr;
+  size_t m = 0;
+  if (filter) {
+    PEB_TRY(scene_prepare_check(ctx, pts, n, stride, num_planes, sac));
+    if (n > 0) PEB_TRY(scene_prepare_device(ctx, pts, n, stride, filter, num_planes, sac, leaf, &d_xyz4, &m, nullptr));
+  } else {
+    PEB_TRY(check_cloud(ctx, "cv_normals", pts, n, stride));
+    m = n;
+    if (n > 0) {
+      PEB_CUDA(ctx, ctx->vg_in.ensure(n * sizeof(float4)));
+      PEB_TRY(upload_cloud(ctx, pts, n, stride, 1.0f, ctx->vg_in.as<float4>()));
+      d_xyz4 = ctx->vg_in.as<float4>();
+    }
+  }
+  // 2. computeNormalsPC3d into the chain's own buffer (:57-59)
+  PEB_CUDA(ctx, ctx->sm_scene.ensure(std::max<size_t>(m, 1) * 6 * sizeof(float)));
+  float* d_scene6 = ctx->sm_scene.as<float>();
+  PEB_TRY(cv_normals_device(ctx, d_xyz4, static_cast<int>(m), prm->normals_k, prm->flip_viewpoint != 0, prm->viewpoint, d_scene6,
+                            nullptr));
+  if (out_scene_xyzn6 && m > 0)
+    PEB_CUDA(ctx, cudaMemcpyAsync(out_scene_xyzn6, d_scene6, m * 6 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  // 3. PPF3DDetector::match on the resident scene (:65)
+  std::vector<peb_ppf_pose> clustered;
+  PEB_TRY(ppf_match_device(ctx, model, d_scene6, m, prm->relative_scene_sample_step, prm->relative_scene_distance, clustered));
+  out->n_results = clustered.size();
+  const size_t n_ref = std::min(clustered.size(), static_cast<size_t>(prm->max_icp_poses));
+  out->n_refined = static_cast<int32_t>(n_ref);
+  if (n_ref > 0) {
+    // 4. ICP(..).registerModelToScene(model rows, scene, first n_ref poses) (:85-94)
+    std::vector<double> poses(16 * n_ref), residuals(n_ref);
+    for (size_t i = 0; i < n_ref; ++i) std::copy(clustered[i].pose, clustered[i].pose + 16, &poses[16 * i]);
+    size_t n_rows = 0;
+    const float* d_rows = ppf_model_rows(model, &n_rows);
+    PEB_TRY(cvicp_register_core(ctx, d_rows, n_rows, d_scene6, m, &prm->icp, poses.data(), n_ref, residuals.data()));
+    std::vector<int> votes(n_ref);
+    for (size_t i = 0; i < n_ref; ++i) {
+      refined[i] = clustered[i];
+      ppf_set_appended_pose(refined[i], &poses[16 * i]);
+      refined[i].residual = residuals[i];
+      votes[i] = static_cast<int>(refined[i].num_votes);
+    }
+    // 5. / 6. the selection rule (:100-124) and the packing (:133-142)
+    const size_t best = pe_b200::select_best_pose(votes.data(), residuals.data(), n_ref, clustered.size());
+    out->best = static_cast<int32_t>(best);
+    pe_b200::pack_pose3d(refined[best], out->pose7, prm->reference_layout != 0);
+  }
+  PEB_TRY(sync(ctx));
+  if (out_n_scene) *out_n_scene = m;
   return PEB_OK;
 }
 
@@ -1101,6 +1210,16 @@ PEB_API int peb_sac_plane(peb_ctx* ctx, const void* pts, size_t n, size_t stride
 
 PEB_API int peb_scene_prepare(peb_ctx* ctx, const void* pts, size_t n, size_t stride, const peb_prefilter_params* filter, int num_planes, const peb_sac_params* sac, float leaf, float* out_xyz4, size_t* out_n, float* out_planes) {
   return guarded(ctx, "peb_scene_prepare", [&]() { return scene_prepare_impl(ctx, pts, n, stride, filter, num_planes, sac, leaf, out_xyz4, out_n, out_planes); });
+}
+
+PEB_API int peb_surface_match(peb_ctx* ctx, const peb_ppf_model* model, const void* pts, size_t n, size_t stride,
+                              const peb_prefilter_params* filter, int num_planes, const peb_sac_params* sac, float leaf,
+                              const peb_surface_match_params* params, peb_ppf_pose* refined, peb_surface_match_result* out,
+                              float* out_scene_xyzn6, size_t* out_n_scene) {
+  return guarded(ctx, "peb_surface_match", [&]() {
+    return surface_match_impl(ctx, model, pts, n, stride, filter, num_planes, sac, leaf, params, refined, out, out_scene_xyzn6,
+                              out_n_scene);
+  });
 }
 
 PEB_API int peb_cvicp_register(peb_ctx* ctx, const float* model_xyzn, size_t n_model, const float* scene_xyzn, size_t n_scene, const peb_cvicp_params* params, double* poses, size_t n_poses, double* out_residuals) {

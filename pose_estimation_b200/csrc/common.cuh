@@ -211,7 +211,9 @@ struct peb_ctx {
   peb::DevBuf vg_in, vg_out, vg_flags, vg_scan, vg_starts;
   peb::DevBuf nrm_in, nrm_out;
   peb::DevBuf brute_keys;    // brute-force validator: one 64-bit (distance, index) key per query, merged over the target segments with atomicMin
-  peb::DevBuf cv_arena;      // cv::ppf_match_3d::ICP mode: all device buffers of a call
+  peb::DevBuf cv_arena;      // cv::ppf_match_3d::ICP mode: the working buffers of a call (also the PPF match's vote scratch)
+  peb::DevBuf cv_in;         // peb_cvicp_register: the uploaded model and scene rows
+  peb::DevBuf sm_scene;      // peb_surface_match: the prepared scene with its normals (n x 6 floats); no other stage touches it
   peb::PinnedBuf h_cv;       // cv ICP mode: pose tables (two, alternating) + accumulator read-back
   peb::PinnedBuf h_sac;      // plane RANSAC: sample indices / coordinates, candidate planes, counts, moment records
 };
@@ -298,9 +300,21 @@ int scene_prefilter_device(peb_ctx* ctx, const float4* d_in, int n, const peb_pr
 // sac.cu
 int sac_plane_device(peb_ctx* ctx, const float4* d_pts, int n, const peb_sac_params* prm, float out_coeff[4],
                      int32_t* d_out_inliers, size_t* out_n_inliers, int32_t* out_iterations);
-// cvicp.cu (host pointers in, results on the host)
+// cvicp.cu (host pointers in, results on the host): the two uploads into ctx->cv_in, then the core
 int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, const float* h_scene, size_t n_scene,
                           const peb_cvicp_params* prm, double* poses, size_t n_poses, double* residuals);
+// the core over DEVICE model / scene rows (read only; they must not lie in ctx->cv_arena or ctx->aux_grid)
+int cvicp_register_core(peb_ctx* ctx, const float* d_model, size_t n_model, const float* d_scene, size_t n_scene,
+                        const peb_cvicp_params* prm, double* poses, size_t n_poses, double* residuals);
+// ppf.cu: peb_ppf_match over a DEVICE scene of n x 6 floats (it must not lie in ctx->nrm_in / nrm_out / cv_arena / d_stage
+// / aux_grid): the clustered poses, same checks after the null ones and same bytes as the host entry point
+int ppf_match_device(peb_ctx* ctx, const peb_ppf_model* m, const float* d_scene6, size_t n_scene, double rel_sample_step,
+                     double rel_distance, std::vector<peb_ppf_pose>& clustered);
+peb_ctx* ppf_model_ctx(const peb_ppf_model* m);
+// the rows the model was trained on (n x 6 floats, resident on the model's device)
+const float* ppf_model_rows(const peb_ppf_model* m, size_t* n_rows);
+// Pose3D::appendPose once the appended pose is known: pose, then q / angle / t recomputed from it
+void ppf_set_appended_pose(peb_ppf_pose& p, const double* pose16);
 // normals.cu
 int target_graph_ensure(peb_ctx* ctx);  // builds ctx->tgt_knn for the current target grid if it is not there yet
 int normals_knn_device(peb_ctx* ctx, const float4* d_in, int n, int k, const float vp[3], float* d_out8,

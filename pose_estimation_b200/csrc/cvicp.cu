@@ -437,14 +437,35 @@ void identity44(double* P) {
 
 }  // namespace
 
-int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, const float* h_scene, size_t n_scene,
-                          const peb_cvicp_params* prm, double* poses, size_t n_poses, double* residuals) {
+// the argument checks, before anything is uploaded
+static int cvicp_check(peb_ctx* ctx, size_t n_model, size_t n_scene, const peb_cvicp_params* prm, size_t n_poses) {
   if (prm->iterations < 0 || prm->num_levels < 1 || prm->num_levels > 16)
     return fail(ctx, PEB_E_INVALID_ARG, "cvicp: iterations >= 0 and 1 <= num_levels <= 16 expected");
   if (n_poses == 0) return PEB_OK;
   if (n_model == 0 || n_scene == 0) return fail(ctx, PEB_E_INVALID_ARG, "cvicp: empty model or scene");
   if (n_poses > 4096) return fail(ctx, PEB_E_UNSUPPORTED, "cvicp: at most 4096 poses per call");
   if (n_model > (1u << 26) || n_scene > (1u << 26)) return fail(ctx, PEB_E_INVALID_ARG, "cvicp: cloud too large");
+  return PEB_OK;
+}
+
+int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, const float* h_scene, size_t n_scene,
+                          const peb_cvicp_params* prm, double* poses, size_t n_poses, double* residuals) {
+  PEB_TRY(cvicp_check(ctx, n_model, n_scene, prm, n_poses));
+  if (n_poses == 0) return PEB_OK;
+  // the two uploads: model and scene one after the other in ctx->cv_in
+  const size_t model_bytes = (sizeof(float) * 6 * n_model + 255) & ~static_cast<size_t>(255);
+  PEB_CUDA(ctx, ctx->cv_in.ensure(model_bytes + sizeof(float) * 6 * n_scene));
+  float* d_model = ctx->cv_in.as<float>();
+  float* d_scene = reinterpret_cast<float*>(ctx->cv_in.as<char>() + model_bytes);
+  PEB_CUDA(ctx, cudaMemcpyAsync(d_model, h_model, sizeof(float) * 6 * n_model, cudaMemcpyHostToDevice, ctx->stream));
+  PEB_CUDA(ctx, cudaMemcpyAsync(d_scene, h_scene, sizeof(float) * 6 * n_scene, cudaMemcpyHostToDevice, ctx->stream));
+  return cvicp_register_core(ctx, d_model, n_model, d_scene, n_scene, prm, poses, n_poses, residuals);
+}
+
+int cvicp_register_core(peb_ctx* ctx, const float* d_model, size_t n_model, const float* d_scene, size_t n_scene,
+                        const peb_cvicp_params* prm, double* poses, size_t n_poses, double* residuals) {
+  PEB_TRY(cvicp_check(ctx, n_model, n_scene, prm, n_poses));
+  if (n_poses == 0) return PEB_OK;
   const int n = static_cast<int>(n_model), ns = static_cast<int>(n_scene), H = static_cast<int>(n_poses);
   cudaStream_t st = ctx->stream;
   const bool robust = prm->rejection_scale > 0.0f;
@@ -457,7 +478,6 @@ int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, co
     off += (bytes + 255) & ~static_cast<size_t>(255);
     return o;
   };
-  const size_t o_model = carve(sizeof(float) * 6 * n), o_scene = carve(sizeof(float) * 6 * ns);
   const size_t o_src0 = carve(sizeof(float) * 6 * n * static_cast<size_t>(H));
   const size_t o_pct = carve(sizeof(float) * 6 * n * static_cast<size_t>(H)), o_moved = carve(sizeof(float) * 6 * n * static_cast<size_t>(H));
   const size_t o_idx = carve(sizeof(int) * n * static_cast<size_t>(H)), o_dist = carve(sizeof(float) * n * static_cast<size_t>(H));
@@ -468,8 +488,6 @@ int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, co
   const size_t o_acc = carve(sizeof(double) * kCvAcc * kCvAccBlocks * H), o_thr = carve(sizeof(float) * H);
   PEB_CUDA(ctx, ctx->cv_arena.ensure(off));
   char* base = ctx->cv_arena.as<char>();
-  float* d_model = reinterpret_cast<float*>(base + o_model);
-  float* d_scene = reinterpret_cast<float*>(base + o_scene);
   float* d_src0 = reinterpret_cast<float*>(base + o_src0);
   float* d_pct = reinterpret_cast<float*>(base + o_pct);
   float* d_moved = reinterpret_cast<float*>(base + o_moved);
@@ -497,9 +515,6 @@ int cvicp_register_device(peb_ctx* ctx, const float* h_model, size_t n_model, co
     stage_k ^= 1;
     return PEB_OK;
   };
-
-  PEB_CUDA(ctx, cudaMemcpyAsync(d_model, h_model, sizeof(float) * 6 * n, cudaMemcpyHostToDevice, st));
-  PEB_CUDA(ctx, cudaMemcpyAsync(d_scene, h_scene, sizeof(float) * 6 * ns, cudaMemcpyHostToDevice, st));
 
   // ---- the model through every input pose, meanAvg ----
   for (int h = 0; h < H; ++h) {

@@ -38,6 +38,7 @@
 
 struct peb_ppf_model {
   peb_ctx* ctx = nullptr;
+  int device = 0;              // ctx's device, kept here: destroying the model never reads ctx (it may be gone already)
   peb_ppf_params prm{};
   double angle_step = 0.0;     // radians
   float distance_step = 0.0f;  // float like upstream
@@ -50,6 +51,8 @@ struct peb_ppf_model {
   peb::DevBuf frames;          // n x 12 double (R row-major, t)
   peb::DevBuf bucket_start;    // (na^3 * nd) * ranges + 1: the pairs of a feature bin, by range of the model reference point
   peb::DevBuf nodes;           // uint2 (model reference, alpha bits) per stored pair
+  peb::DevBuf rows;            // n_rows x 6 float: the rows trained on, resident for the cv ICP of peb_surface_match
+  size_t n_rows = 0;
   std::vector<float> h_sampled;
 };
 
@@ -519,19 +522,26 @@ struct Sampled {
   float lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0};
 };
 
-// samplePCByQuantization of a host cloud (n x 6 floats): the sampled rows land in `out` (device), lattice order
-int ppf_sample(peb_ctx* ctx, const float* h_pc6, size_t n_in, float sample_step, DevBuf* out, Sampled* info) {
-  info->n = 0;
+// the argument checks of ppf_sample, before anything is uploaded
+int ppf_sample_check(peb_ctx* ctx, size_t n_in, float sample_step) {
   if (n_in == 0) return PEB_OK;
   if (n_in > static_cast<size_t>(INT32_MAX) / 8) return fail(ctx, PEB_E_INVALID_ARG, "ppf: too many points");
-  const int n = static_cast<int>(n_in);
   if (!(sample_step > 0.0f) || !(sample_step <= 1.0f)) return fail(ctx, PEB_E_INVALID_ARG, "ppf: sampling step must be in (0, 1] (got %g)", sample_step);
   const int nsd = static_cast<int>(1.0 / sample_step);
   const long long cells = static_cast<long long>(nsd + 1) * (nsd + 1) * (nsd + 1);
   if (cells >= (1ll << 31)) return fail(ctx, PEB_E_UNSUPPORTED, "ppf: sampling step %g gives %lld lattice cells", sample_step, cells);
-  PEB_CUDA(ctx, ctx->d_stage.ensure(static_cast<size_t>(n) * 24));
-  float* d_in = ctx->d_stage.as<float>();
-  PEB_CUDA(ctx, cudaMemcpyAsync(d_in, h_pc6, static_cast<size_t>(n) * 24, cudaMemcpyHostToDevice, ctx->stream));
+  return PEB_OK;
+}
+
+// samplePCByQuantization of a DEVICE cloud (n x 6 floats, read only): the sampled rows land in `out` (device), lattice
+// order.  `out` must not alias d_in.
+int ppf_sample_device(peb_ctx* ctx, const float* d_in, size_t n_in, float sample_step, DevBuf* out, Sampled* info) {
+  info->n = 0;
+  PEB_TRY(ppf_sample_check(ctx, n_in, sample_step));
+  if (n_in == 0) return PEB_OK;
+  const int n = static_cast<int>(n_in);
+  const int nsd = static_cast<int>(1.0 / sample_step);
+  const long long cells = static_cast<long long>(nsd + 1) * (nsd + 1) * (nsd + 1);
   PEB_CUDA(ctx, ctx->d_small.ensure(256));
   PEB_CUDA(ctx, ctx->h_small.ensure(256));
   unsigned* d_box = ctx->d_small.as<unsigned>();
@@ -582,6 +592,16 @@ int ppf_sample(peb_ctx* ctx, const float* h_pc6, size_t n_in, float sample_step,
   PEB_LAUNCH(ctx, ppf_cell_mean_kernel, ceil_div(static_cast<long long>(n_runs) * 32, 128), 128, 0, d_in, sk, sv, n,
              ctx->vg_starts.as<uint32_t>(), n_runs, out->as<float>());
   return PEB_OK;
+}
+
+// the same for a host cloud: uploaded to `staging` (ctx->d_stage for a scene, the model's own rows for training) first
+int ppf_sample(peb_ctx* ctx, const float* h_pc6, size_t n_in, float sample_step, DevBuf* staging, DevBuf* out, Sampled* info) {
+  info->n = 0;
+  PEB_TRY(ppf_sample_check(ctx, n_in, sample_step));
+  if (n_in == 0) return PEB_OK;
+  PEB_CUDA(ctx, staging->ensure(n_in * 24));
+  PEB_CUDA(ctx, cudaMemcpyAsync(staging->p, h_pc6, n_in * 24, cudaMemcpyHostToDevice, ctx->stream));
+  return ppf_sample_device(ctx, staging->as<float>(), n_in, sample_step, out, info);
 }
 
 // [CV] Pose3D::updatePoseQuat
@@ -692,6 +712,7 @@ int train_impl(peb_ctx* ctx, const float* model6, size_t n_model, const peb_ppf_
     }
   } drop{m};
   m->ctx = ctx;
+  m->device = ctx->device;
   m->prm = *prm;
   // [CV] PPF3DDetector::PPF3DDetector / setSearchParams
   m->angle_step = (360.0 / prm->num_angles) * kPi / 180.0;
@@ -699,7 +720,9 @@ int train_impl(peb_ctx* ctx, const float* model6, size_t n_model, const peb_ppf_
   m->rotation_threshold = prm->rotation_threshold < 0 ? ((360 / m->angle_step) / 180.0 * kPi) : prm->rotation_threshold;
   m->num_angles = static_cast<int>(std::floor(2 * kPi / m->angle_step));
   Sampled info;
-  PEB_TRY(ppf_sample(ctx, model6, n_model, static_cast<float>(prm->relative_sampling_step), &m->sampled, &info));
+  // the rows stay on the device with the model: peb_surface_match refines against them without another upload
+  PEB_TRY(ppf_sample(ctx, model6, n_model, static_cast<float>(prm->relative_sampling_step), &m->rows, &m->sampled, &info));
+  m->n_rows = n_model;
   if (info.n < 2) return fail(ctx, PEB_E_INVALID_ARG, "ppf_train: the model samples to %d points", info.n);
   // (a voting tile flattens the buckets of 256 scene pairs into one 32-bit item range: 256 n^2 must stay below 2^32)
   if (info.n > 4095) return fail(ctx, PEB_E_UNSUPPORTED, "ppf_train: %d sampled model points (at most 4095)", info.n);
@@ -746,22 +769,23 @@ int train_impl(peb_ctx* ctx, const float* model6, size_t n_model, const peb_ppf_
   return PEB_OK;
 }
 
-int match_impl(peb_ctx* ctx, const peb_ppf_model* m, const float* scene6, size_t n_scene, double rel_sample_step,
-               double rel_distance, peb_ppf_pose* results, size_t cap, size_t* out_n, peb_ppf_pose* raw, size_t cap_raw,
-               size_t* out_n_raw) {
-  if (!ctx) return PEB_E_INVALID_ARG;
-  if (out_n) *out_n = 0;
-  if (out_n_raw) *out_n_raw = 0;
-  if (!m || !scene6) return fail(ctx, PEB_E_INVALID_ARG, "ppf_match: null model / scene");
+// the checks of peb_ppf_match that do not depend on where the scene is
+int match_check(peb_ctx* ctx, const peb_ppf_model* m, double rel_sample_step) {
   if (m->ctx != ctx) return fail(ctx, PEB_E_INVALID_ARG, "ppf_match: the model was trained on another context");
   if (!(rel_sample_step > 0.0) || !(rel_sample_step <= 1.0))
     return fail(ctx, PEB_E_INVALID_ARG, "ppf_match: relative scene sample step must be in (0, 1] (got %g)", rel_sample_step);
-  DeviceScope scope(ctx->device);
+  return PEB_OK;
+}
+
+// match over a scene that is already sampled into ctx->nrm_in (info from ppf_sample*): raw poses in reference order, then
+// clustered.  Uses nrm_out (scene frames) and cv_arena.
+int match_sampled(peb_ctx* ctx, const peb_ppf_model* m, const Sampled& info, double rel_sample_step,
+                  std::vector<peb_ppf_pose>& h_raw, std::vector<peb_ppf_pose>& clustered) {
+  h_raw.clear();
+  clustered.clear();
   const int step = static_cast<int>(1.0 / rel_sample_step);
   DevBuf& scene = ctx->nrm_in;       // sampled scene rows
   DevBuf& frames = ctx->nrm_out;     // their frames
-  Sampled info;
-  PEB_TRY(ppf_sample(ctx, scene6, n_scene, static_cast<float>(rel_distance), &scene, &info));
   const int ms = info.n;
   if (ms == 0) return PEB_OK;
   const int n_ref = (ms + step - 1) / step;
@@ -783,13 +807,28 @@ int match_impl(peb_ctx* ctx, const peb_ppf_model* m, const float* scene6, size_t
              m->bucket_start.as<uint32_t>(), m->nodes.as<uint2>(), m->n, m->num_angles, m->chunk, m->ranges, pair_scratch, refs);
   PEB_LAUNCH(ctx, ppf_pose_kernel, ceil_div(n_ref, 128), 128, 0, refs, n_ref, step, frames.as<double>(), m->frames.as<double>(),
              m->num_angles, d_poses);
-  std::vector<peb_ppf_pose> h_raw(static_cast<size_t>(n_ref));
+  h_raw.resize(static_cast<size_t>(n_ref));
   PEB_CUDA(ctx, cudaMemcpyAsync(h_raw.data(), d_poses, pose_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   PEB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  cluster_poses(*m, h_raw, clustered);
+  return PEB_OK;
+}
+
+int match_impl(peb_ctx* ctx, const peb_ppf_model* m, const float* scene6, size_t n_scene, double rel_sample_step,
+               double rel_distance, peb_ppf_pose* results, size_t cap, size_t* out_n, peb_ppf_pose* raw, size_t cap_raw,
+               size_t* out_n_raw) {
+  if (!ctx) return PEB_E_INVALID_ARG;
+  if (out_n) *out_n = 0;
+  if (out_n_raw) *out_n_raw = 0;
+  if (!m || !scene6) return fail(ctx, PEB_E_INVALID_ARG, "ppf_match: null model / scene");
+  PEB_TRY(match_check(ctx, m, rel_sample_step));
+  DeviceScope scope(ctx->device);
+  Sampled info;
+  PEB_TRY(ppf_sample(ctx, scene6, n_scene, static_cast<float>(rel_distance), &ctx->d_stage, &ctx->nrm_in, &info));
+  std::vector<peb_ppf_pose> h_raw, clustered;
+  PEB_TRY(match_sampled(ctx, m, info, rel_sample_step, h_raw, clustered));
   if (out_n_raw) *out_n_raw = h_raw.size();
   if (raw) std::memcpy(raw, h_raw.data(), std::min(cap_raw, h_raw.size()) * sizeof(peb_ppf_pose));
-  std::vector<peb_ppf_pose> clustered;
-  cluster_poses(*m, h_raw, clustered);
   if (out_n) *out_n = clustered.size();
   if (results) std::memcpy(results, clustered.data(), std::min(cap, clustered.size()) * sizeof(peb_ppf_pose));
   return PEB_OK;
@@ -814,6 +853,40 @@ int guarded(peb_ctx* ctx, const char* what, Fn fn) noexcept {
 }
 
 }  // namespace
+
+// peb_ppf_match over a DEVICE scene (n x 6 floats, not written; must not be ctx->nrm_in / nrm_out / cv_arena / d_stage):
+// the clustered poses, most votes first.  Same checks (after the null ones) and bytes as the host entry point.
+int ppf_match_device(peb_ctx* ctx, const peb_ppf_model* m, const float* d_scene6, size_t n_scene, double rel_sample_step,
+                     double rel_distance, std::vector<peb_ppf_pose>& clustered) {
+  clustered.clear();
+  PEB_TRY(match_check(ctx, m, rel_sample_step));
+  DeviceScope scope(ctx->device);
+  Sampled info;
+  PEB_TRY(ppf_sample_device(ctx, d_scene6, n_scene, static_cast<float>(rel_distance), &ctx->nrm_in, &info));
+  std::vector<peb_ppf_pose> h_raw;
+  return match_sampled(ctx, m, info, rel_sample_step, h_raw, clustered);
+}
+
+peb_ctx* ppf_model_ctx(const peb_ppf_model* m) { return m->ctx; }
+
+const float* ppf_model_rows(const peb_ppf_model* m, size_t* n_rows) {
+  *n_rows = m->n_rows;
+  return m->rows.as<float>();
+}
+
+// [CV] Pose3D::appendPose, given the appended pose (icp_pose * pose): pose, then q, angle and t recomputed from it
+void ppf_set_appended_pose(peb_ppf_pose& p, const double* pose16) {
+  for (int a = 0; a < 16; ++a) p.pose[a] = pose16[a];
+  double R[9];
+  for (int a = 0; a < 3; ++a)
+    for (int b = 0; b < 3; ++b) R[3 * a + b] = pose16[4 * a + b];
+  dcm_to_quat(R, p.q);
+  p.angle = pose_angle(R);
+  p.t[0] = pose16[3];
+  p.t[1] = pose16[7];
+  p.t[2] = pose16[11];
+}
+
 }  // namespace peb
 
 extern "C" {
@@ -836,11 +909,12 @@ PEB_API int peb_ppf_train(peb_ctx* ctx, const float* model_xyzn, size_t n_model,
 PEB_API void peb_ppf_model_destroy(peb_ppf_model* m) {
   if (!m) return;
   {
-    peb::DeviceScope scope(m->ctx ? m->ctx->device : 0);
+    peb::DeviceScope scope(m->device);
     m->sampled.release();
     m->frames.release();
     m->bucket_start.release();
     m->nodes.release();
+    m->rows.release();
   }
   delete m;
 }

@@ -17,7 +17,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import CvIcpParams, IcpParams, IcpResult, GridInfo, PpfParams, PpfPose, PrefilterParams, SacParams, lib
+from ._lib import (CvIcpParams, IcpParams, IcpResult, GridInfo, PpfParams, PpfPose, PrefilterParams, SacParams, SurfaceMatchParams,
+                   SurfaceMatchResult, lib)
 
 DBL_MAX = float(np.finfo(np.float64).max)
 
@@ -280,15 +281,9 @@ class ScenePrefilter:
         return out[: m.value].copy()
 
 
-def create_surface_match_pc(cloud, ctx: Context | None = None, filter_pose=None, filter_radius: float = 0.0,
-                            filter_out: str = "outliers", num_planes: int = 0, leaf: float = 0.0, plane_band: float = 0.005,
-                            distance_threshold: float = 0.0001, max_iterations: int = 100):
-    """PoseEstimation::create_surface_match_pc (pose_estimation/src/pose_estimation.cpp:211-279) from the organized cloud
-    on: NaN removal, the optional sphere filter around the last pose, num_planes rounds of plane RANSAC + 5 mm band
-    removal (remove_planes, :281-345, with the reference's RANSAC settings as defaults) and — leaf > 0 — the VoxelGrid,
-    in ONE library call (peb_scene_prepare).  -> (points (M, 4) float32, plane coefficients (num_planes, 4))."""
-    ctx = ctx or default_context()
-    p = _cloud(cloud)
+def _surface_match_pc_params(filter_pose, filter_radius, filter_out, plane_band=0.005, distance_threshold=0.0001,
+                             max_iterations=100):
+    """The filter and RANSAC settings of create_surface_match_pc -> (PrefilterParams, SacParams)."""
     f = PrefilterParams()
     f.plane_band = float(plane_band)
     if filter_pose is not None and filter_radius > 0:
@@ -300,6 +295,19 @@ def create_surface_match_pc(cloud, ctx: Context | None = None, filter_pose=None,
     lib.peb_sac_params_default(C.byref(sp))
     sp.distance_threshold = float(distance_threshold)
     sp.max_iterations = int(max_iterations)
+    return f, sp
+
+
+def create_surface_match_pc(cloud, ctx: Context | None = None, filter_pose=None, filter_radius: float = 0.0,
+                            filter_out: str = "outliers", num_planes: int = 0, leaf: float = 0.0, plane_band: float = 0.005,
+                            distance_threshold: float = 0.0001, max_iterations: int = 100):
+    """PoseEstimation::create_surface_match_pc (pose_estimation/src/pose_estimation.cpp:211-279) from the organized cloud
+    on: NaN removal, the optional sphere filter around the last pose, num_planes rounds of plane RANSAC + 5 mm band
+    removal (remove_planes, :281-345, with the reference's RANSAC settings as defaults) and — leaf > 0 — the VoxelGrid,
+    in ONE library call (peb_scene_prepare).  -> (points (M, 4) float32, plane coefficients (num_planes, 4))."""
+    ctx = ctx or default_context()
+    p = _cloud(cloud)
+    f, sp = _surface_match_pc_params(filter_pose, filter_radius, filter_out, plane_band, distance_threshold, max_iterations)
     out = np.empty((max(p.shape[0], 1), 4), np.float32)
     planes = np.zeros((max(num_planes, 1), 4), np.float32)
     m = C.c_size_t(0)
@@ -460,6 +468,52 @@ class PPF3DDetector:
             self.close()
         except Exception:
             pass
+
+
+def surface_match_params(**overrides) -> SurfaceMatchParams:
+    """peb_surface_match_params with the reference's values (peb_surface_match_params_default: k = 20 normals flipped
+    towards (0, 0, 0), match(.., 1.0, 0.03), the first 6 results refined by ICP(250, 0.005f, 2.5f, 8), corrected pose7
+    layout); keyword arguments override fields (icp=(iterations, tolerance, rejection_scale, num_levels))."""
+    p = SurfaceMatchParams()
+    lib.peb_surface_match_params_default(C.byref(p))
+    for k, v in overrides.items():
+        if k == "icp":
+            it, tol, rej, lev = v
+            p.icp = CvIcpParams(int(it), int(lev), float(tol), float(rej))
+        elif k == "viewpoint":
+            p.viewpoint[:] = [float(x) for x in v]
+        else:
+            setattr(p, k, type(getattr(p, k))(v))
+    return p
+
+
+def find_object_in_scene(detector: "PPF3DDetector", cloud, params: SurfaceMatchParams | None = None, prepare: bool = False,
+                         filter_pose=None, filter_radius: float = 0.0, filter_out: str = "outliers", num_planes: int = 0,
+                         leaf: float = 0.0, return_scene: bool = False):
+    """OpenCVSurfaceMatch::find_object_in_scene (pose_estimation/src/opencv_surface_match.cpp:57-142) in ONE library call
+    (peb_surface_match) on the detector's context: computeNormalsPC3d, detector.match, cv ICP of the first
+    params.max_icp_poses results against the rows the detector was trained on, the selection rule and the packing.
+    cloud: the (N, >=3) float cloud the function receives; prepare=True runs create_surface_match_pc's preparation in front
+    of it (NaN removal, sphere filter, num_planes plane removals, leaf > 0: VoxelGrid) with its arguments.
+    -> (refined PpfPose list, best (-1: nothing found), pose7 float32[7], n_results) [+ scene (M, 6) float32 with
+    return_scene]; the same bytes as the step-by-step calls."""
+    ctx = detector.ctx
+    p = _cloud(cloud)
+    params = params if params is not None else surface_match_params()
+    f = sp = None
+    if prepare:
+        f, sp = _surface_match_pc_params(filter_pose, filter_radius, filter_out)
+    refined = (PpfPose * max(int(params.max_icp_poses), 1))()
+    res = SurfaceMatchResult()
+    scene = np.empty((max(p.shape[0], 1), 6), np.float32) if return_scene else None
+    m = C.c_size_t(0)
+    ctx.check(lib.peb_surface_match(ctx.handle, detector._model, p.ctypes.data, p.shape[0], _stride(p),
+                                    C.byref(f) if f is not None else None, int(num_planes), C.byref(sp) if sp is not None else None,
+                                    float(leaf), C.byref(params), refined, C.byref(res),
+                                    scene.ctypes.data if scene is not None else None, C.byref(m)))
+    out = ([PpfPose.from_buffer_copy(r) for r in refined[: res.n_refined]], int(res.best), np.array(res.pose7, np.float32),
+           int(res.n_results))
+    return out + (scene[: m.value].copy(),) if return_scene else out
 
 
 class VoxelGrid:

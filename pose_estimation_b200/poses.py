@@ -59,6 +59,51 @@ def pack_pose(T, reference_layout: bool = False) -> np.ndarray:
     return pose
 
 
+def pack_pose3d(t, q, reference_layout: bool = False) -> np.ndarray:
+    """{x, y, z, qx, qy, qz, qw} float32 from a Pose3D's t and q (w, x, y, z), as opencv_surface_match.cpp:133-142 builds
+    it (pe_b200::pack_pose3d).  reference_layout=True: qz is never written, pose[6] gets q[3] and then q[0]."""
+    t = np.asarray(t, np.float64)
+    q = np.asarray(q, np.float64)
+    pose = np.zeros(7, np.float32)
+    pose[:3] = t[:3]
+    pose[3], pose[4] = q[1], q[2]
+    if reference_layout:
+        pose[6] = q[3]
+        pose[6] = q[0]
+    else:
+        pose[5], pose[6] = q[3], q[0]
+    return pose
+
+
+def pose3d_from_matrix(P):
+    """Pose3D::appendPose's bookkeeping once the appended pose P (4 x 4, float64) is known: (q (w, x, y, z), t, angle) with
+    OpenCV's dcmToQuat and the angle from the trace (the same operations as ppf.cu, so the same bits)."""
+    import math
+
+    P = np.asarray(P, np.float64).reshape(4, 4)
+    R = [float(v) for v in P[:3, :3].ravel()]
+    tr = R[0] + R[4] + R[8]
+    q = [0.0] * 4
+    if tr > 0:
+        q[0], q[1], q[2], q[3] = tr + 1.0, R[5] - R[7], R[6] - R[2], R[1] - R[3]
+    else:
+        i = 0
+        if R[4] > R[0]:
+            i = 1
+        if R[8] > R[3 * i + i]:
+            i = 2
+        j, k = (i + 1) % 3, (i + 2) % 3
+        q[i + 1] = R[3 * i + i] - R[3 * j + j] - R[3 * k + k] + 1.0
+        q[j + 1] = R[3 * i + j] + R[3 * j + i]
+        q[k + 1] = R[3 * i + k] + R[3 * k + i]
+        q[0] = R[3 * j + k] - R[3 * k + j]
+    s = 1.0 / math.sqrt(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3])
+    q = [v * s for v in q]
+    eps = 1.192092896e-07
+    angle = 0.0 if abs(tr - 3) <= eps else (math.pi if abs(tr + 1) <= eps else math.acos((tr - 1) / 2))
+    return np.array(q), P[:3, 3].copy(), angle
+
+
 def _eigen_quat_from_matrix(m: np.ndarray) -> np.ndarray:
     """Eigen::Quaternionf(Matrix3f) (Eigen/src/Geometry/Quaternion.h : quaternionbase_assign_impl), float32,
     -> (x, y, z, w), no sign normalisation."""
