@@ -460,6 +460,56 @@ PEB_API int peb_icp_align_ex(peb_ctx* ctx, const float guess[16], const peb_icp_
 PEB_API int peb_icp_align_batch_ex(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_icp_params* params,
                                    const peb_rejector* chain, size_t n_chain, peb_icp_result* results);
 
+/* ---- pcl::GeneralizedIterativeClosestPoint<PointXYZ, PointXYZ>::align ----------------------------------------
+ * Plane-to-plane ICP for clouds without normals (DESIGN.md section 15).  [PCL] registration/include/pcl/registration/gicp.h,
+ * impl/gicp.hpp, bfgs.h (restated from recollection, unverified against PCL, like sections 2, 9 and 11):
+ *   covariances  per point of each cloud, its k nearest neighbours (the point itself included) in its own cloud; float
+ *                products summed in double in list order; mean / k, cov / k - mean mean^T; JacobiSVD; U diag(1, 1, 0.001) U^T.
+ *                Computed once per cloud and k, kept until the next peb_source_set* / peb_target_set* (peb_gicp_covariances
+ *                returns them: n x 9 doubles, row-major, original order, NaN rows for non-finite points).
+ *   outer loop   output = transformPointCloud(input, guess); transformation_ = I; per iteration: every finite source point's
+ *                exact nearest target point of transformation_ * output[i] is a pair iff d2 < max_corr_dist^2 (STRICT <;
+ *                ICP keeps d2 <= max^2), M_i = (R C_src R^T + C_tgt)^-1 with R = top-left of transformation_ * guess in
+ *                double; then the BFGS below; delta = max |previous - transformation_| over the 16 entries, scaled by
+ *                1 / rotation_epsilon in the rotation block and 1 / transformation_epsilon elsewhere; stop when
+ *                iterations >= max_iterations or delta < 1 (converged = 1 in both cases, as in PCL); T = previous * guess.
+ *   BFGS         x = (t, atan2(T21, T22), asin(-T20), atan2(T10, T00)) of the float transformation_, f = (1/m) sum res^T M res,
+ *                res = (Rz Ry Rx (float quaternions) * output[i] + t) - target (float, widened); GSL's vector_bfgs2 with
+ *                Fletcher's line search (rho = sigma = 0.01, tau 9 / 0.05 / 0.5, cubic interpolation), at most
+ *                max_inner_iterations steps or until |g| < 0.01.  The quadratic of the cubic's derivative is solved in closed
+ *                form (PCL: Eigen's PolynomialSolver).
+ * Where PCL is undefined, this library defines:
+ *   - non-finite points are neither queries nor neighbours;
+ *   - k < 1, or k above the number of finite points of either cloud, is PEB_E_INVALID_ARG (PCL prints an error and runs
+ *     on with empty covariances); k > 192 is PEB_E_UNSUPPORTED (the bound of peb_normals_knn);
+ *   - an iteration with fewer than 4 pairs ends the align (PCL: NotEnoughPointsException; with none it would divide by
+ *     zero): state PEB_NO_CORRESPONDENCES, converged 0, T = previous * guess;
+ *   - PCL's GICP never consults its convergence criteria, so state is this library's record: PEB_TRANSFORM when delta < 1,
+ *     PEB_ITERATIONS at the cap;
+ *   - last_mse = mean d2 of the last iteration's pairs, n_correspondences = their number, fitness = getFitnessScore.
+ * The device keeps H x n_src x 72 bytes of Mahalanobis matrices; PEB_E_OOM if they cannot be allocated.  Every record of
+ * a batch is byte-identical to the single align of the same guess.  max_iterations and max_inner_iterations must be >= 1,
+ * max_corr_dist >= 0 and both epsilons > 0 (PEB_E_INVALID_ARG); a batch holds at most 65535 guesses. */
+typedef struct peb_gicp_params {
+  int32_t max_iterations;        /* setMaximumIterations              (200)     */
+  int32_t k_correspondences;     /* setCorrespondenceRandomness       (20)      */
+  int32_t max_inner_iterations;  /* setMaximumOptimizerIterations     (20)      */
+  int32_t reserved;
+  double max_corr_dist;          /* setMaxCorrespondenceDistance      (5)       */
+  double transformation_epsilon; /* setTransformationEpsilon          (5e-4)    */
+  double rotation_epsilon;       /* setRotationEpsilon                (2e-3)    */
+  double fitness_max_range;      /* getFitnessScore(max_range)        (DBL_MAX) */
+} peb_gicp_params;
+PEB_API void peb_gicp_params_default(peb_gicp_params* p);
+/* guess: column-major 4x4 (NULL = identity); the outputs as peb_icp_align's (corr of the last iteration, -1 = no pair) */
+PEB_API int peb_gicp_align(peb_ctx* ctx, const float guess[16], const peb_gicp_params* params, peb_icp_result* result,
+                           float* out_aligned_xyz4, int32_t* out_corr_idx, float* out_corr_d2);
+/* H guesses (H x 16 floats, column-major each), H records */
+PEB_API int peb_gicp_align_batch(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_gicp_params* params,
+                                 peb_icp_result* results);
+/* the covariances GICP uses for k neighbours: which 0 = source, 1 = target; out9 holds n x 9 doubles */
+PEB_API int peb_gicp_covariances(peb_ctx* ctx, int which, int k, double* out9);
+
 /* pcl::Registration::getFitnessScore(max_range) for an arbitrary transform */
 PEB_API int peb_fitness_score(peb_ctx* ctx, const float T[16], double max_range, double* out_fitness,
                               int32_t* out_n_inliers);

@@ -10,6 +10,7 @@
 //        normals slot      pose_estimation/src/opencv_surface_match.cpp:57-59
 //   pe_b200::IterativeClosestPoint             pcl::IterativeClosestPoint<PointXYZ, PointXYZ>
 //   pe_b200::IterativeClosestPointWithNormals  pcl::IterativeClosestPointWithNormals<PointNormal, PointNormal>
+//   pe_b200::GeneralizedIterativeClosestPoint  pcl::GeneralizedIterativeClosestPoint<PointXYZ, PointXYZ>
 //        refinement slot   pose_estimation/src/opencv_surface_match.cpp:85-94
 //
 // Clouds are passed as (pointer, count, stride in bytes): pcl::PointCloud<PointXYZ>::points.data()
@@ -341,6 +342,60 @@ class IterativeClosestPoint {
   peb_icp_params params_;
   peb_icp_result result_;
   ConvergenceCriteria criteria_;
+  size_t n_src_ = 0;
+};
+
+// pcl::GeneralizedIterativeClosestPoint<PointXYZ, PointXYZ> (peb_gicp_align, DESIGN.md section 15): plane-to-plane ICP
+// whose per-point covariances come from k neighbours of each cloud, so neither cloud needs normals
+class GeneralizedIterativeClosestPoint {
+ public:
+  explicit GeneralizedIterativeClosestPoint(Context& c) : c_(c) {
+    peb_gicp_params_default(&params_);
+    std::memset(&result_, 0, sizeof(result_));
+    for (int i = 0; i < 4; ++i) result_.T[5 * i] = 1.0f;
+  }
+
+  void setInputSource(const void* pts, size_t n, size_t stride = 16) {
+    c_.check(peb_source_set(c_.get(), pts, n, stride));
+    n_src_ = n;
+  }
+  void setInputTarget(const void* pts, size_t n, size_t stride = 16) {
+    c_.check(peb_target_set(c_.get(), pts, n, stride, nullptr, 0));
+  }
+  void setMaximumIterations(int n) { params_.max_iterations = n; }
+  void setCorrespondenceRandomness(int k) { params_.k_correspondences = k; }
+  void setMaximumOptimizerIterations(int n) { params_.max_inner_iterations = n; }
+  void setRotationEpsilon(double e) { params_.rotation_epsilon = e; }
+  void setMaxCorrespondenceDistance(double d) { params_.max_corr_dist = d; }
+  void setTransformationEpsilon(double e) { params_.transformation_epsilon = e; }
+
+  // align(output, guess): out_xyz4 (nullable) receives final * input as x y z 1 records
+  void align(std::vector<float>* out_xyz4 = nullptr, const float* guess16 = nullptr) {
+    if (out_xyz4) out_xyz4->resize(4 * n_src_);
+    float* out = out_xyz4 && n_src_ ? out_xyz4->data() : nullptr;
+    c_.check(peb_gicp_align(c_.get(), guess16, &params_, &result_, out, nullptr, nullptr));
+  }
+  // H initial poses (column-major 4 x 4 each) against one source / one target; results[h] is the align of guess h
+  void alignBatch(const float* guesses16, size_t n_guesses, std::vector<peb_icp_result>& results) {
+    results.resize(n_guesses);
+    c_.check(peb_gicp_align_batch(c_.get(), guesses16, n_guesses, &params_, results.data()));
+  }
+  bool hasConverged() const { return result_.converged != 0; }
+  const float* getFinalTransformation() const { return result_.T; }  // column-major 4x4
+  double getFitnessScore(double max_range = DBL_MAX) {
+    if (max_range == params_.fitness_max_range) return result_.fitness;
+    double f = 0;
+    c_.check(peb_fitness_score(c_.get(), result_.T, max_range, &f, nullptr));
+    return f;
+  }
+  int nr_iterations() const { return result_.iterations; }
+  const peb_icp_result& result() const { return result_; }
+  const peb_gicp_params& params() const { return params_; }
+
+ private:
+  Context& c_;
+  peb_gicp_params params_;
+  peb_icp_result result_;
   size_t n_src_ = 0;
 };
 

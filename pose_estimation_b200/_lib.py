@@ -97,6 +97,21 @@ class IcpResult(C.Structure):
     ]
 
 
+class GicpParams(C.Structure):
+    """peb_gicp_params."""
+
+    _fields_ = [
+        ("max_iterations", C.c_int32),
+        ("k_correspondences", C.c_int32),
+        ("max_inner_iterations", C.c_int32),
+        ("reserved", C.c_int32),
+        ("max_corr_dist", C.c_double),
+        ("transformation_epsilon", C.c_double),
+        ("rotation_epsilon", C.c_double),
+        ("fitness_max_range", C.c_double),
+    ]
+
+
 class PrefilterParams(C.Structure):
     """peb_prefilter_params."""
 
@@ -222,6 +237,10 @@ SYMBOLS = {
     "peb_icp_align_batch": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp]),
     "peb_icp_align_ex": (_i, [_vp, _vp, _pp(IcpParams), _vp, _sz, _pp(IcpResult), _vp, _vp, _vp]),
     "peb_icp_align_batch_ex": (_i, [_vp, _vp, _sz, _pp(IcpParams), _vp, _sz, _vp]),
+    "peb_gicp_params_default": (None, [_pp(GicpParams)]),
+    "peb_gicp_align": (_i, [_vp, _vp, _pp(GicpParams), _pp(IcpResult), _vp, _vp, _vp]),
+    "peb_gicp_align_batch": (_i, [_vp, _vp, _sz, _pp(GicpParams), _vp]),
+    "peb_gicp_covariances": (_i, [_vp, _i, _i, _vp]),
     "peb_fitness_score": (_i, [_vp, _vp, _d, _pp(_d), _pp(C.c_int32)]),
     "peb_target_set_dev": (_i, [_vp, _vp, _sz, _vp]),
     "peb_source_set_dev": (_i, [_vp, _vp, _sz]),

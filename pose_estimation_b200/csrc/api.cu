@@ -3,6 +3,7 @@
 // file and there is no CPU implementation behind any entry point: if the device path cannot run,
 // the call fails with a peb_status and a message.
 #include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -74,6 +75,7 @@ struct DeviceGuard {
 
 int target_finish(peb_ctx* ctx, size_t n, bool has_normals) {
   ctx->tgt_knn_valid = false;
+  ctx->gicp_tgt_k = 0;
   ctx->n_tgt = n;
   ctx->tgt_has_normals = has_normals;
   return grid_build(ctx, &ctx->tgt_grid, ctx->tgt_raw.as<float4>(), has_normals ? ctx->tgt_nrm_raw.as<float4>() : nullptr,
@@ -82,6 +84,7 @@ int target_finish(peb_ctx* ctx, size_t n, bool has_normals) {
 
 int source_finish(peb_ctx* ctx, size_t n) {
   ctx->n_src = n;
+  ctx->gicp_src_k = 0;
   PEB_TRY(grid_build(ctx, &ctx->src_grid, ctx->src.as<float4>(), nullptr, static_cast<int>(n), ctx->src_sort_occupancy));
   ctx->n_src_sorted = ctx->src_grid.view.n;
   ctx->src_set = true;
@@ -224,7 +227,8 @@ PEB_API void peb_ctx_destroy(peb_ctx* ctx) {
                     &ctx->corr_idx, &ctx->corr_d2, &ctx->partials, &ctx->state, &ctx->trace, &ctx->d_guesses,
                     &ctx->d_results, &ctx->d_aligned, &ctx->vg_in, &ctx->vg_out, &ctx->vg_flags, &ctx->vg_scan,
                     &ctx->vg_starts, &ctx->nrm_in, &ctx->nrm_out, &ctx->brute_keys, &ctx->nn_q, &ctx->nn_idx, &ctx->nn_d2, &ctx->epochs, &ctx->cv_arena,
-                    &ctx->cv_in, &ctx->sm_scene};
+                    &ctx->cv_in, &ctx->sm_scene, &ctx->gicp_src_cov, &ctx->gicp_tgt_cov, &ctx->gicp_state, &ctx->gicp_prev,
+                    &ctx->gicp_tq, &ctx->gicp_d2, &ctx->gicp_M, &ctx->gicp_alive, &ctx->gicp_final, &ctx->gicp_fit};
   for (DevBuf* b : bufs) b->release();
   ctx->sort_scratch.release();
   for (DevBuf& b : ctx->scan_scratch) b.release();
@@ -1037,6 +1041,93 @@ static int icp_align_batch_impl(peb_ctx* ctx, const float* guesses, size_t n_gue
     return fail(ctx, PEB_E_CUDA, "align_batch: a per-hypothesis dependency wait ran into its bound (internal error; "
                                  "peb_ctx_set_int(ctx, \"flag_deps\", 0) restores whole-grid dependencies)");
   return PEB_OK;
+}
+
+// ---- GeneralizedIterativeClosestPoint -------------------------------------------------------------------------------
+static int gicp_check_params(peb_ctx* ctx, const peb_gicp_params* p) {
+  if (p->max_iterations < 1) return fail(ctx, PEB_E_INVALID_ARG, "gicp: max_iterations must be >= 1 (got %d)", p->max_iterations);
+  if (p->max_inner_iterations < 1)
+    return fail(ctx, PEB_E_INVALID_ARG, "gicp: max_inner_iterations must be >= 1 (got %d)", p->max_inner_iterations);
+  if (!(p->max_corr_dist >= 0.0) || !(p->transformation_epsilon > 0.0) || !(p->rotation_epsilon > 0.0))
+    return fail(ctx, PEB_E_INVALID_ARG, "gicp: max_corr_dist must be >= 0 and both epsilons > 0");
+  return PEB_OK;
+}
+
+PEB_API void peb_gicp_params_default(peb_gicp_params* p) {
+  if (!p) return;
+  p->max_iterations = 200;
+  p->k_correspondences = 20;
+  p->max_inner_iterations = 20;
+  p->reserved = 0;
+  p->max_corr_dist = 5.0;
+  p->transformation_epsilon = 5e-4;
+  p->rotation_epsilon = 2e-3;
+  p->fitness_max_range = DBL_MAX;
+}
+
+static int gicp_align_impl(peb_ctx* ctx, const float guess[16], const peb_gicp_params* params, peb_icp_result* result,
+                           float* out_aligned_xyz4, int32_t* out_corr_idx, float* out_corr_d2) {
+  if (!ctx || !params || !result) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  PEB_TRY(gicp_check_params(ctx, params));
+  const float* d_g = nullptr;
+  PEB_TRY(upload_guesses(ctx, guess, 1, &d_g));
+  const size_t n = ctx->n_src;
+  PEB_CUDA(ctx, ctx->d_results.ensure(sizeof(peb_icp_result)));
+  PEB_CUDA(ctx, ctx->d_aligned.ensure(std::max<size_t>(n, 1) * sizeof(float4)));
+  PEB_CUDA(ctx, ctx->corr_idx.ensure(std::max<size_t>(n, 1) * sizeof(int32_t)));
+  PEB_CUDA(ctx, ctx->corr_d2.ensure(std::max<size_t>(n, 1) * sizeof(float)));
+  PEB_TRY(gicp_align_device(ctx, d_g, 1, params, ctx->d_results.as<peb_icp_result>(), out_aligned_xyz4 ? ctx->d_aligned.as<float4>() : nullptr,
+                            out_corr_idx ? ctx->corr_idx.as<int32_t>() : nullptr, out_corr_d2 ? ctx->corr_d2.as<float>() : nullptr));
+  PEB_CUDA(ctx, cudaMemcpyAsync(result, ctx->d_results.p, sizeof(peb_icp_result), cudaMemcpyDeviceToHost, ctx->stream));
+  if (out_aligned_xyz4 && n)
+    PEB_CUDA(ctx, cudaMemcpyAsync(out_aligned_xyz4, ctx->d_aligned.p, n * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
+  if (out_corr_idx && n)
+    PEB_CUDA(ctx, cudaMemcpyAsync(out_corr_idx, ctx->corr_idx.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (out_corr_d2 && n)
+    PEB_CUDA(ctx, cudaMemcpyAsync(out_corr_d2, ctx->corr_d2.p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  return sync(ctx);
+}
+
+static int gicp_align_batch_impl(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_gicp_params* params,
+                                 peb_icp_result* results) {
+  if (!ctx || !params) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  PEB_TRY(gicp_check_params(ctx, params));
+  if (n_guesses == 0) return PEB_OK;
+  if (!guesses || !results) return fail(ctx, PEB_E_INVALID_ARG, "gicp_align_batch: null guesses / results");
+  if (n_guesses > 65535) return fail(ctx, PEB_E_INVALID_ARG, "gicp_align_batch: %zu guesses (at most 65535)", n_guesses);
+  const float* d_g = nullptr;
+  PEB_TRY(upload_guesses(ctx, guesses, n_guesses, &d_g));
+  PEB_CUDA(ctx, ctx->d_results.ensure(n_guesses * sizeof(peb_icp_result)));
+  PEB_TRY(gicp_align_device(ctx, d_g, n_guesses, params, ctx->d_results.as<peb_icp_result>(), nullptr, nullptr, nullptr));
+  PEB_CUDA(ctx, cudaMemcpyAsync(results, ctx->d_results.p, n_guesses * sizeof(peb_icp_result), cudaMemcpyDeviceToHost, ctx->stream));
+  return sync(ctx);
+}
+
+static int gicp_covariances_impl(peb_ctx* ctx, int which, int k, double* out9) {
+  if (!ctx) return PEB_E_INVALID_ARG;
+  DeviceGuard guard(ctx->device);
+  if (which != 0 && which != 1) return fail(ctx, PEB_E_INVALID_ARG, "gicp_covariances: which must be 0 (source) or 1 (target)");
+  PEB_TRY(gicp_check_k(ctx, k));
+  const size_t n = which == 0 ? ctx->n_src : ctx->n_tgt;
+  if (n > 0 && !out9) return fail(ctx, PEB_E_INVALID_ARG, "gicp_covariances: null output");
+  PEB_CUDA(ctx, ctx->d_stage.ensure(std::max<size_t>(n, 1) * 9 * sizeof(double)));
+  PEB_TRY(gicp_covariances_device(ctx, which, k, ctx->d_stage.as<double>()));
+  if (n) PEB_CUDA(ctx, cudaMemcpyAsync(out9, ctx->d_stage.p, n * 9 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  return sync(ctx);
+}
+
+PEB_API int peb_gicp_align(peb_ctx* ctx, const float guess[16], const peb_gicp_params* params, peb_icp_result* result,
+                           float* out_aligned_xyz4, int32_t* out_corr_idx, float* out_corr_d2) {
+  return guarded(ctx, "peb_gicp_align", [&] { return gicp_align_impl(ctx, guess, params, result, out_aligned_xyz4, out_corr_idx, out_corr_d2); });
+}
+PEB_API int peb_gicp_align_batch(peb_ctx* ctx, const float* guesses, size_t n_guesses, const peb_gicp_params* params,
+                                 peb_icp_result* results) {
+  return guarded(ctx, "peb_gicp_align_batch", [&] { return gicp_align_batch_impl(ctx, guesses, n_guesses, params, results); });
+}
+PEB_API int peb_gicp_covariances(peb_ctx* ctx, int which, int k, double* out9) {
+  return guarded(ctx, "peb_gicp_covariances", [&] { return gicp_covariances_impl(ctx, which, k, out9); });
 }
 
 PEB_API int peb_fitness_score(peb_ctx* ctx, const float T[16], double max_range, double* out_fitness, int32_t* out_n_inliers) {

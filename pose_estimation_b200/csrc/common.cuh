@@ -216,6 +216,13 @@ struct peb_ctx {
   peb::DevBuf sm_scene;      // peb_surface_match: the prepared scene with its normals (n x 6 floats); no other stage touches it
   peb::PinnedBuf h_cv;       // cv ICP mode: pose tables (two, alternating) + accumulator read-back
   peb::PinnedBuf h_sac;      // plane RANSAC: sample indices / coordinates, candidate planes, counts, moment records
+
+  // GeneralizedIterativeClosestPoint (gicp.cu)
+  peb::DevBuf gicp_src_cov;  // (finite source points) x 9 doubles, sorted grid position
+  peb::DevBuf gicp_tgt_cov;  // (finite target points) x 9 doubles, sorted grid position
+  int gicp_src_k = 0;        // k of the cached covariances, 0: none (peb_source_set* / peb_target_set* clear them)
+  int gicp_tgt_k = 0;
+  peb::DevBuf gicp_state, gicp_prev, gicp_tq, gicp_d2, gicp_M, gicp_alive, gicp_final, gicp_fit;
 };
 
 namespace peb {
@@ -289,6 +296,9 @@ int icp_output_device(peb_ctx* ctx, float4* d_out);
 int nn_search_device(peb_ctx* ctx, const float4* d_q, int nq, int32_t* d_idx, float* d_d2);
 // fitness of one transform (device, 16 floats); the record's n_correspondences carries the inlier count
 int fitness_device(peb_ctx* ctx, const float* d_T, double max_range, peb_icp_result* d_result);
+// the same for H transforms (H x 16 floats); every hypothesis is summed with the blocks of a single one, so a record does
+// not depend on the batch around it
+int fitness_batch_device(peb_ctx* ctx, const float* d_T, size_t H, double max_range, peb_icp_result* d_results);
 // brute.cu
 int nn_bruteforce_device(peb_ctx* ctx, const float4* d_q, int nq, int32_t* d_idx, float* d_d2);
 // voxel.cu
@@ -322,5 +332,12 @@ int normals_knn_device(peb_ctx* ctx, const float4* d_in, int n, int k, const flo
 // cv::ppf_match_3d::computeNormalsPC3d: d_out6 = n rows of x y z nx ny nz (DESIGN.md §13)
 int cv_normals_device(peb_ctx* ctx, const float4* d_in, int n, int k, bool flip, const float vp[3], float* d_out6,
                       int32_t* d_out_nn /*nullable, n x k original indices*/);
+
+// gicp.cu: the checks of k against the resident clouds, the covariances (which 0: source, 1: target; n x 9 doubles in
+// original order, NaN rows for non-finite points) and the align of H guesses (nullable: identity) into d_results
+int gicp_check_k(peb_ctx* ctx, int k);
+int gicp_covariances_device(peb_ctx* ctx, int which, int k, double* d_out9);
+int gicp_align_device(peb_ctx* ctx, const float* d_guesses, size_t H, const peb_gicp_params* prm, peb_icp_result* d_results,
+                      float4* d_aligned, int32_t* d_corr_idx, float* d_corr_d2);
 
 }  // namespace peb

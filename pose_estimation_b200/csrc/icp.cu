@@ -2460,6 +2460,25 @@ int fitness_device(peb_ctx* ctx, const float* d_T, double max_range, peb_icp_res
   return launch_fitness_g(ctx, ctx->nn_group, L, 1);
 }
 
+int fitness_batch_device(peb_ctx* ctx, const float* d_T, size_t H, double max_range, peb_icp_result* d_results) {
+  if (H == 0) return PEB_OK;
+  peb_icp_params prm;
+  peb_icp_params_default(&prm);
+  prm.fitness_max_range = max_range;
+  IcpLaunch L{};
+  PEB_TRY(prepare_launch(ctx, H, &prm, L));
+  L.results = d_results;
+  L.fitness_only = 1;
+  L.warm = 0;
+  L.blocks_per_hyp = blocks_for(ctx->n_src_sorted, 1, ctx->nn_group, ctx->blocks_factor);
+  L.part_stride = std::max(L.part_stride, L.blocks_per_hyp);
+  PEB_CUDA(ctx, ctx->partials.ensure(H * static_cast<size_t>(L.part_stride) * kAccMax * sizeof(double)));
+  L.partials = ctx->partials.as<double>();
+  PEB_LAUNCH(ctx, icp_init_kernel, ceil_div(static_cast<long long>(H), 128), 128, 0, L.states, d_T, static_cast<int>(H),
+             static_cast<int*>(nullptr));
+  return launch_fitness_g(ctx, ctx->nn_group, L, H);
+}
+
 int icp_output_device(peb_ctx* ctx, float4* d_out) {
   const int n = static_cast<int>(ctx->n_src);
   if (n == 0) return PEB_OK;

@@ -17,7 +17,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import (CvIcpParams, IcpParams, IcpResult, GridInfo, PpfParams, PpfPose, PrefilterParams, SacParams, SurfaceMatchParams,
+from ._lib import (CvIcpParams, GicpParams, IcpParams, IcpResult, GridInfo, PpfParams, PpfPose, PrefilterParams, SacParams, SurfaceMatchParams,
                    SurfaceMatchResult, lib)
 
 DBL_MAX = float(np.finfo(np.float64).max)
@@ -809,6 +809,98 @@ class IterativeClosestPoint:
         n = C.c_size_t(0)
         self._sctx.check(lib.peb_icp_trace(self._sctx.handle, buf.ctypes.data, cap, C.byref(n)))
         return buf[: n.value].reshape(-1, 4, 4).transpose(0, 2, 1).copy()
+
+
+class GeneralizedIterativeClosestPoint:
+    """pcl::GeneralizedIterativeClosestPoint<PointXYZ, PointXYZ> ([PCL] registration/gicp.h): plane-to-plane ICP that
+    builds its own per-point covariances from k neighbours, so it needs no normals (peb_gicp_align, DESIGN.md §15)."""
+
+    def __init__(self, ctx: Context | None = None):
+        self.ctx = ctx or default_context()
+        self.params = GicpParams()
+        lib.peb_gicp_params_default(C.byref(self.params))
+        self._result: IcpResult | None = None
+        self._n_src = 0
+        self.correspondences = None
+
+    def setInputSource(self, cloud):
+        self.ctx.source_set(cloud)
+        self._n_src = _cloud(cloud).shape[0]
+
+    def setInputTarget(self, cloud):
+        self.ctx.target_set(_cloud(cloud))
+
+    def setMaximumIterations(self, n: int):
+        self.params.max_iterations = int(n)
+
+    def setCorrespondenceRandomness(self, k: int):
+        self.params.k_correspondences = int(k)
+
+    def setMaximumOptimizerIterations(self, n: int):
+        self.params.max_inner_iterations = int(n)
+
+    def setRotationEpsilon(self, e: float):
+        self.params.rotation_epsilon = float(e)
+
+    def setMaxCorrespondenceDistance(self, d: float):
+        self.params.max_corr_dist = float(d)
+
+    def setTransformationEpsilon(self, e: float):
+        self.params.transformation_epsilon = float(e)
+
+    def align(self, guess=None, want_output: bool = True, want_correspondences: bool = False) -> np.ndarray | None:
+        """align(output, guess): returns the (N, 4) transformed source (or None)."""
+        g = _col_major(guess) if guess is not None else None
+        res = IcpResult()
+        n = self._n_src
+        out = np.empty((n, 4), np.float32) if (want_output and n) else None
+        idx = np.empty(n, np.int32) if (want_correspondences and n) else None
+        d2 = np.empty(n, np.float32) if (want_correspondences and n) else None
+        self.ctx.check(lib.peb_gicp_align(self.ctx.handle, g.ctypes.data if g is not None else None, C.byref(self.params),
+                                          C.byref(res), out.ctypes.data if out is not None else None,
+                                          idx.ctypes.data if idx is not None else None, d2.ctypes.data if d2 is not None else None))
+        self._result = res
+        self.correspondences = (idx, d2) if want_correspondences else None
+        return out
+
+    def alignBatch(self, guesses) -> list[IcpResult]:
+        """H initial poses (H, 4, 4) -> H records, each the single align of its guess."""
+        g = np.ascontiguousarray(np.asarray(guesses, np.float32).reshape(-1, 4, 4).transpose(0, 2, 1)).reshape(-1, 16)
+        H = g.shape[0]
+        res = (IcpResult * max(H, 1))()
+        self.ctx.check(lib.peb_gicp_align_batch(self.ctx.handle, g.ctypes.data, H, C.byref(self.params), res))
+        return list(res)[:H]
+
+    def covariances(self, which: str = "source") -> np.ndarray:
+        """The (N, 3, 3) covariances of the source or the target for the current k (NaN for non-finite points)."""
+        w = 0 if which == "source" else 1
+        n = self._n_src if w == 0 else self.ctx._keep_t.shape[0]
+        out = np.empty((max(n, 1), 9), np.float64)
+        self.ctx.check(lib.peb_gicp_covariances(self.ctx.handle, w, self.params.k_correspondences, out.ctypes.data))
+        return out[:n].reshape(n, 3, 3)
+
+    def hasConverged(self) -> bool:
+        return bool(self._result and self._result.converged)
+
+    def getFinalTransformation(self) -> np.ndarray:
+        if self._result is None:
+            return np.eye(4, dtype=np.float32)
+        return result_matrix(self._result)
+
+    def getFitnessScore(self, max_range: float = DBL_MAX) -> float:
+        if self._result is None:
+            raise ValueError("getFitnessScore before align")
+        if max_range == self.params.fitness_max_range:
+            return self._result.fitness
+        return self.ctx.fitness_score(self.getFinalTransformation(), max_range)[0]
+
+    @property
+    def nr_iterations_(self) -> int:
+        return self._result.iterations if self._result else 0
+
+    @property
+    def result(self) -> IcpResult | None:
+        return self._result
 
 
 class IterativeClosestPointWithNormals(IterativeClosestPoint):
